@@ -2,22 +2,26 @@
 """bench.py -- env-steps/sec of the fused env.step() hot path (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
-                    [--env PointTSP-v0] [--envs 65536]
+                    [--env PointTSP-v0] [--envs 65536] [--dump-outputs DIR]
 
 One "step" = one crl_step() launch over one batch of `--envs` envs (10 MuJoCo substeps + task logic +
 full observation write per env, auto-reset on, iid U(-1,1)^2 actions drawn IN the kernel per (env, step):
 SURVEY 8d).  Default workload = BASELINE.json configs[1]: PointTSP, 65,536 batched envs, 1 x B200.
 
-Timing.  K (= --steps) is the granule: after W warm-up steps the bench times a whole number of K-step
-blocks, back to back, for at least --min-seconds of device time (CUDA events on the launching stream, a
-barrier + synchronize on both sides), in segments of >= 50 ms; `ms_per_step` is the MEDIAN segment's time
-per step (the best segment is reported beside it), so `--steps 20` and `--steps 64000` measure the same
-steady state.  A 65,536-env batch is 39 MB of state + observation and would sit in the 126 MB L2, so the
-steps cycle a RING of independent replicas of the batch (each its own state, layouts and counters;
-together > 2 x L2): every launch finds its inputs in HBM.  `value` = steps x envs / device time, max over
-ranks.  `e2e` = the same metric through ZoneVecEnv.step_host(): HOST numpy actions in, HOST obs / reward /
-done out, copies inside every call.  The same line also carries BASELINE.json configs[2] and [3]
-(`configs`), and under --gpus N > 1 configs[4] (all three tasks at 1,048,576 envs per GPU).
+Timing.  After W warm-up steps the bench times exactly K (= --steps) steps, back to back (CUDA events on the
+launching stream, a barrier + synchronize on both sides).  The K steps are queued behind a device-side spin,
+so the window holds device work only, not the host's launch of the first step.  `ms_per_step` = window / K
+(the fastest and slowest graph replay inside the window are reported beside it).  A 65,536-env batch is
+39 MB of state + observation and would sit in the 126 MB L2, so the steps cycle a RING of independent
+replicas of the batch (each its own state, layouts and counters; together > 2 x L2): every launch finds its
+inputs in HBM.  `value` = steps x envs / device time, max over ranks.  `e2e` = the same metric through
+ZoneVecEnv.step_host(): HOST numpy actions in, HOST obs / reward / done out, copies inside every call.  The
+same line also carries BASELINE.json configs[2] and [3] (`configs`), and under --gpus N > 1 configs[4] (all
+three tasks at 1,048,576 envs per GPU).
+
+Outputs.  Seeds and the in-kernel action draws are fixed, so the same arguments step the same envs with the
+same actions in every run.  `--dump-outputs DIR` writes what the timed path's last step returned to its caller
+(see dump_outputs()), so that two builds of the project can be compared output for output.
 
 `--impl reference` times the reference's CPU path: mujoco-py / Safety Gym cannot be installed here, so that
 is the oracle's port of it (oracle/), in three topologies -- see cpu_baselines().
@@ -260,6 +264,7 @@ class Ring:
                 took = n // self.R + (1 if r < n % self.R else 0)
                 if took and e.tick(took):
                     self.prefetch_launches += 3 if self.task == 0 else 4
+            self.last_env = self.envs[(n - 1) % self.R]                # every graph starts at replica 0
 
     def counters(self):
         c = self.torch.zeros(8, dtype=self.torch.float64, device=self.dev)
@@ -268,48 +273,53 @@ class Ring:
         return c
 
 
-def measure(ring, K, W, min_seconds, world, dist, seg_ms=50.0, max_segments=400):
-    """Time whole K-step blocks for >= min_seconds.  Returns dict(ms_per_step median/best/mean, ...)."""
+def measure(ring, K, W, world, dist, spin_cycles=20_000_000):
+    """Time exactly K steps after W warm-up steps.  The K steps' graphs are captured first and queued behind a
+    spin of `spin_cycles` SM clocks (~10 ms), so the events around them hold device work only, not the host's
+    launch of the first graph (slow: a graph's first launch also uploads it).  Returns dict(ms_per_step, ...)."""
     torch = ring.torch
-    dev = ring.dev
     ring.run(ring.prepare(W))
-    torch.cuda.synchronize()
-    # calibration: one block
-    plan_k = ring.prepare(K)
-    t0, t1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    t0.record()
-    ring.run(plan_k)
-    t1.record()
-    torch.cuda.synchronize()
-    block_ms = max(t0.elapsed_time(t1), 1e-3)
-    blocks_per_seg = max(1, int(round(seg_ms / block_ms)))
-    seg_steps = blocks_per_seg * K
-    n_seg = int(min(max_segments, max(3, -(-min_seconds * 1e3 // (blocks_per_seg * block_ms)))))
-    if world > 1:                                                      # every rank times the same number of steps
-        t = torch.tensor([seg_steps, n_seg], device=dev, dtype=torch.int64)
-        dist.all_reduce(t, op=dist.ReduceOp.MAX)
-        seg_steps, n_seg = int(t[0]) // K * K, int(t[1])
-    plan = ring.prepare(seg_steps)
+    plan = ring.prepare(K)
     ring.prefetch_launches = 0
-    ev = [torch.cuda.Event(enable_timing=True) for _ in range(n_seg + 1)]
+    ev = [torch.cuda.Event(enable_timing=True) for _ in range(len(plan) + 1)]
     torch.cuda.synchronize()
     if world > 1:
         dist.barrier()
-    wall0 = time.perf_counter()
+    torch.cuda._sleep(spin_cycles)
     ev[0].record()
-    for i in range(n_seg):
-        ring.run(plan)
+    for i, n in enumerate(plan):
+        ring.run([n])
         ev[i + 1].record()
     torch.cuda.synchronize()
-    wall = time.perf_counter() - wall0
     if world > 1:
         dist.barrier()
-    seg = sorted(ev[i].elapsed_time(ev[i + 1]) / seg_steps for i in range(n_seg))
-    total_ms = ev[0].elapsed_time(ev[n_seg])
-    return {'ms_per_step': seg[len(seg) // 2], 'ms_per_step_best': seg[0], 'ms_per_step_worst': seg[-1],
-            'ms_per_step_mean': total_ms / (n_seg * seg_steps), 'timed_steps': n_seg * seg_steps,
-            'blocks': n_seg * seg_steps // K, 'segments': n_seg, 'steps_per_segment': seg_steps,
-            'timed_region_s': total_ms * 1e-3, 'wall_s': wall, 'calibration_block_ms': block_ms}
+    seg = sorted(ev[i].elapsed_time(ev[i + 1]) / n for i, n in enumerate(plan))
+    total_ms = ev[0].elapsed_time(ev[-1])
+    return {'ms_per_step': total_ms / K, 'ms_per_step_best': seg[0], 'ms_per_step_worst': seg[-1],
+            'ms_per_step_mean': total_ms / K, 'timed_steps': K, 'segments': len(plan),
+            'timed_region_s': total_ms * 1e-3}
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(env, out_dir, seed=0):
+    """What the timed path's last step handed its caller (ZoneVecEnv.step_random: obs, zone_obs, reward, done and the
+    info arrays) as out_dir/<name>.npy, float32.  When they exceed DUMP_BYTES in all, every array keeps the rows of
+    the same fixed, seeded sample of envs, listed in env_index.npy."""
+    import numpy as np
+    got = dict(env._obs_dict(), reward=env.reward, done=env.done, **{'info_' + k: v for k, v in env._info().items()})
+    got = {k: v.float().cpu().numpy() for k, v in got.items()}
+    B = env.num_envs
+    room = DUMP_BYTES - 4096 * (len(got) + 1)                          # less a generous .npy header per file
+    if sum(a.nbytes for a in got.values()) > room:
+        row = sum(a.nbytes for a in got.values()) // B
+        keep = np.sort(np.random.RandomState(seed).choice(B, room // (row + 8), replace=False))
+        got = {k: a[keep] for k, a in got.items()}
+        got['env_index'] = keep.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in got.items():
+        np.save(os.path.join(out_dir, k + '.npy'), a)
 
 
 def device_line(ring, m, world, peak):
@@ -383,8 +393,10 @@ def run_ours(args):
     time.sleep(0.5)                                                    # nvidia-smi start-up
     ring = Ring(crl, _lib, args, args.env, B, dev, rank, chained=chained, streams=args.streams)
     sampler.mark()
-    m = measure(ring, K, W, args.min_seconds, world, dist)
+    m = measure(ring, K, W, world, dist)
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(ring.last_env, args.dump_outputs)
     for k in ('ms_per_step', 'ms_per_step_best', 'ms_per_step_mean'):
         m[k] = rank_max(m[k])
     head = device_line(ring, m, world, peak)
@@ -521,7 +533,7 @@ def run_ours(args):
             if (env_id, b) == (args.env, B):
                 continue
             r2 = Ring(crl, _lib, args, env_id, b, dev, rank, chained=chained, streams=args.streams)
-            m2 = measure(r2, K, W, args.extra_seconds, world, dist)
+            m2 = measure(r2, K, W, world, dist)
             for k in ('ms_per_step', 'ms_per_step_best', 'ms_per_step_mean'):
                 m2[k] = rank_max(m2[k])
             d = device_line(r2, m2, world, peak)
@@ -558,11 +570,11 @@ def run_ours(args):
                    'ring_replicas': head_R, 'streams': head_S, 'chained_steps': head_chained,
                    'concurrency': 'the ring\'s replicas are independent env batches, each stepped on its own CUDA stream (launches of '
                                   'different replicas overlap; steps of one replica are ordered by its stream)', 'prefetch_every': args.prefetch_every, 'layout_bank': args.bank or None,
-                   'timing': f'{m["blocks"]} blocks of K={K} steps back to back ({m["timed_region_s"]:.2f} s of device time, CUDA events, '
-                             f'barrier + synchronize on both sides), {m["segments"]} segments of {m["steps_per_segment"]} steps; '
-                             f'ms_per_step / value = the MEDIAN segment, max over ranks'},
+                   'timing': f'K={K} steps after W={W} warm-up steps, back to back ({m["timed_region_s"] * 1e3:.2f} ms of device '
+                             f'time, CUDA events queued behind a device spin, barrier + synchronize on both sides), '
+                             f'{m["segments"]} graph replays; ms_per_step / value = the whole window, max over ranks'},
         'timing': {k: m[k] for k in ('ms_per_step', 'ms_per_step_best', 'ms_per_step_worst', 'ms_per_step_mean', 'timed_steps',
-                                     'blocks', 'segments', 'steps_per_segment', 'timed_region_s', 'wall_s', 'calibration_block_ms')},
+                                     'segments', 'timed_region_s')},
         'roofline': {'bound': 'hbm', 'achieved': head['achieved_gbs'], 'peak': peak, 'unit': 'GB/s', 'frac': head['frac'],
                      'traffic': traffic, 'traffic_note': traffic_note if traffic is not None else None,
                      'algorithmic_bytes_per_launch': sb * B, 'peak_source': peak_src, 'kernel': 'step_kernel',
@@ -669,13 +681,13 @@ def head_ring_desc(step_bytes, B):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument('--gpus', type=int, default=1)
-    ap.add_argument('--steps', type=int, default=2000)
+    ap.add_argument('--steps', type=int, default=100000, help='timed steps of the headline workload and of each extra config')
     ap.add_argument('--warmup', type=int, default=200)
     ap.add_argument('--impl', default='ours', choices=['ours', 'reference'])
     ap.add_argument('--env', default='PointTSP-v0')
     ap.add_argument('--envs', type=int, default=65536)
-    ap.add_argument('--min-seconds', type=float, default=1.5, help='device time of the headline timed region')
-    ap.add_argument('--extra-seconds', type=float, default=0.6, help='device time of each extra config')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='write the outputs of the last timed step (rank 0\'s envs) to DIR/<name>.npy, <= 64 MB in all')
     ap.add_argument('--e2e-seconds', type=float, default=1.0)
     ap.add_argument('--e2e-max-calls', type=int, default=20000)
     ap.add_argument('--cpu-seconds', type=float, default=9.0)

@@ -309,10 +309,10 @@ def test_philox_reset_twin_layouts_are_valid():
 
 
 def test_timeout_wrapper_matches_the_reference_class():
-    """compat.TimeoutWrapper against the REAL main/envs/wrappers.py:161-194 (imported over the gym / mujoco_py / glfw stubs
-    when /root/reference is present; the recorded expectations below otherwise) on a scripted inner env."""
-    import importlib
-    import sys
+    """compat.TimeoutWrapper against the REAL main/envs/wrappers.py:161-194 on a scripted inner env: the reference class's
+    trace (imported over the gym / mujoco_py / glfw stubs of tests/golden/stubs, which it matched when compat.TimeoutWrapper
+    was written) is stored in tests/golden/timeout_wrapper_trace.json, as JSON (tuples read back as lists)."""
+    import json
     from combinatorial_rl_tasks_b200.compat import TimeoutWrapper
 
     class Inner:
@@ -343,17 +343,7 @@ def test_timeout_wrapper_matches_the_reference_class():
     assert ours[1] == (('obs', 1), 1.5, False, {'timer': 1}) and ours[4] == (('obs', 4), 6.0, False, {'timer': 4})
     assert ours[5] == (('obs', 4), 0, False, {'timer': 5}) and ours[7] == (('obs', 4), 0, True, {'timer': 7})
     assert ours[8] == (('obs', 4), 0, False, {'timer': 8}) and ours[10] == ('obs', 0) and ours[11][3] == {'timer': 1}
-    ref_dir = '/root/reference/main'
-    if os.path.isdir(ref_dir):
-        stubs = os.path.join(ROOT, 'tests', 'golden', 'stubs')
-        saved = list(sys.path)
-        sys.path[:0] = [stubs, ref_dir]
-        try:
-            ref_mod = importlib.import_module('envs.wrappers')
-            real = ref_mod.TimeoutWrapper.__new__(ref_mod.TimeoutWrapper)     # gym.Wrapper.__init__ of the stub needs a gym.Env
-            real.env, real.max_timeout, real.timer, real.inner_done, real.last_obs = Inner(), 7, 0, False, None
-            assert trace(real) == ours
-        finally:
-            sys.path[:] = saved
-            for m in [m for m in sys.modules if m == 'envs' or m.startswith('envs.')]:
-                del sys.modules[m]
+    with open(os.path.join(ROOT, 'tests', 'golden', 'timeout_wrapper_trace.json')) as f:
+        real = json.load(f)
+    assert len(real) == len(ours) == 12
+    assert json.loads(json.dumps(ours)) == real

@@ -2,7 +2,7 @@
 """Device-timed sweep of the step kernel over (env, envs, chained, streams, ...) in ONE process (bench.py's
 Ring / measure, no e2e, no CPU baseline): one JSON line per case.  Tuning tool; bench.py is the record.
 
-    python tools/sweep.py PointTSP-v0:65536:c1:s1 PointTTSP-v0:262144:c0:s2 ... [--seconds 1.0] [--steps 200]
+    python tools/sweep.py PointTSP-v0:65536:c1:s1 PointTTSP-v0:262144:c0:s2 ... [--steps 20000] [--warmup 50]
     case = env:envs[:cX][:sY][:pZ][:bK][:wW][:rR]   c = chained (0/1, default auto), s = streams, p = prefetch_every, b = layout bank size,
            w = sampler warps per SM, r = minimum number of ring replicas
 """
@@ -19,8 +19,7 @@ import bench  # noqa: E402
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument('cases', nargs='+')
-    ap.add_argument('--seconds', type=float, default=1.0)
-    ap.add_argument('--steps', type=int, default=200)
+    ap.add_argument('--steps', type=int, default=20000, help='timed steps per case')
     ap.add_argument('--warmup', type=int, default=50)
     ap.add_argument('--cfg', action='append', default=[])
     ap.add_argument('--no-auto-reset', action='store_true')
@@ -39,7 +38,7 @@ def main():
                                   cfg=a.cfg, no_auto_reset=a.no_auto_reset, env=env_id, min_replicas=opt.get('r', 0))
         ring = bench.Ring(crl, _lib, args, env_id, B, dev, 0, chained=(None if 'c' not in opt else bool(opt['c'])),
                           streams=opt.get('s', 0))
-        m = bench.measure(ring, a.steps, a.warmup, a.seconds, 1, None)
+        m = bench.measure(ring, a.steps, a.warmup, 1, None)
         d = bench.device_line(ring, m, 1, peak)
         c = ring.counters().cpu().numpy()
         print(json.dumps({'case': case, 'lib': os.environ.get('CRL_B200_LIB', 'default'), 'frac': round(d['frac'], 4),
