@@ -14,6 +14,7 @@ TASK_TSP, TASK_TTSP, TASK_CM = 0, 1, 2
 SEED_INCREMENT, SEED_FIXED_RANGE = 0, 1
 STEP_AUTO_RESET, STEP_PHYSICS_ONLY, STEP_CHAINED, STEP_CHAIN_START, STEP_TRACK_ROWS = 1, 2, 4, 8, 16
 STEP_GOALS, STEP_WAIT, STEP_ACTION_COUNTER, STEP_HOST_ZERO_COPY, STEP_NO_ZONE_OBS, STEP_HOST_PLANES = 32, 64, 128, 256, 512, 1024
+STEP_ZONE_OBS_DELTA = 2048
 ABI_VERSION = 8
 NUM_PLANES = 23
 

@@ -13,7 +13,8 @@
 //      background sampler parked it in (prefetch_*_kernel); only if the slot is empty does
 //      its warp build the layout cooperatively (32 rejection-sampling candidates per round),
 //   5. stages its zone_obs row in shared memory, from where each warp's 32 rows (one
-//      contiguous span of B x N x Z) leave with a single cp.async.bulk shared->global copy,
+//      contiguous span of B x N x Z) leave with a single cp.async.bulk shared->global copy
+//      (CRL_STEP_ZONE_OBS_DELTA: only the rows that change are built and written),
 //   6. integrates all frameskip substeps in registers (crl_core.cuh) while that copy drains,
 //   7. writes state and the 8-float obs row.
 // Episode statistics go through warp ballots and one atomic per warp.  Also here: the
@@ -835,27 +836,28 @@ __device__ __forceinline__ void zone_obs_send(const KParams& p, const Env<N>& en
   zone_obs_issue<TASK, N>(p, stage, lane, warp_env0, 32);
 }
 
-// CRL_STEP_HOST_ZERO_COPY: the rows of `mask`'s lanes (the envs whose zone_obs row this step changed) from the
-// warp's stage straight into the caller's host mirror of zone_obs (pinned, device-mapped), each row by the whole
-// warp with coalesced stores.  A handful of rows per launch: the host buffer stays a byte-exact copy of the device
-// one with no list, no gather kernel and no host-side scatter.
-// CRL_STEP_HOST_PLANES (TimedTSP): the host mirror is PLANE-major, float[Z][B][N] (the caller views it as (B, N, Z)
-// through strides), so that the one column that moves every step -- time left, plane 6 -- is a contiguous
-// [B][N] array: the warp writes its 32 x N values of it with fully coalesced stores, every step; a changed row
-// (a visit, a reset) is N values in each of the other planes.
+// The rows of `mask`'s lanes (the envs whose zone_obs row this step changed) from the warp's stage into `out`, each
+// row by the whole warp with coalesced stores.  A handful of rows per launch.  CRL_STEP_HOST_ZERO_COPY: `out` is the
+// caller's host mirror of zone_obs (pinned, device-mapped), which so stays a byte-exact copy of the device one with no
+// list, no gather kernel and no host-side scatter.  CRL_STEP_ZONE_OBS_DELTA: `out` is the device zone_obs itself.
+// CRL_STEP_HOST_PLANES (TimedTSP, host mirror only): the host mirror is PLANE-major, float[Z][B][N] (the caller views
+// it as (B, N, Z) through strides), so that the one column that moves every step -- time left, plane 6 -- is a
+// contiguous [B][N] array: the warp writes its 32 x N values of it with fully coalesced stores, every step; a changed
+// row (a visit, a reset) is N values in each of the other planes.
 template <int TASK, int N>
-__device__ __noinline__ void rows_to_host(const KParams& p, const float* stage, unsigned mask, int lane, int warp_env0) {
+__device__ __noinline__ void send_rows(const KParams& p, float* out, const float* stage, unsigned mask, int lane,
+                                       int warp_env0) {
   constexpr int Z = ZoneDim<TASK>::Z, ROW = N * Z;
   if (TASK == CRL_TASK_TTSP && (p.flags & CRL_STEP_HOST_PLANES)) {
     const size_t plane = (size_t)p.B * N;
     const int n_valid = max(0, min(32, p.B - warp_env0));
-    float* tl = p.zone_obs_host + 6 * plane + (size_t)warp_env0 * N;
+    float* tl = out + 6 * plane + (size_t)warp_env0 * N;
     for (int i = lane; i < n_valid * N; i += 32) tl[i] = stage[(i / N) * ROW + (i % N) * Z + 6];
     while (mask) {
       const int src = __ffs(mask) - 1;
       mask &= mask - 1u;
       const float* row = stage + src * ROW;
-      float* dst = p.zone_obs_host + (size_t)(warp_env0 + src) * N;
+      float* dst = out + (size_t)(warp_env0 + src) * N;
       for (int i = lane; i < 6 * N; i += 32) dst[(size_t)(i / N) * plane + (i % N)] = row[(i % N) * Z + (i / N)];
     }
     return;
@@ -863,10 +865,28 @@ __device__ __noinline__ void rows_to_host(const KParams& p, const float* stage, 
   while (mask) {
     const int src = __ffs(mask) - 1;
     mask &= mask - 1u;
-    float* dst = p.zone_obs_host + (size_t)(warp_env0 + src) * ROW;
+    float* dst = out + (size_t)(warp_env0 + src) * ROW;
     const float* row = stage + src * ROW;
     for (int i = lane; i < ROW; i += 32) dst[i] = row[i];
   }
+}
+
+// zone_obs of the plain step: the warp's rows are staged and leave with one bulk copy.  CRL_STEP_ZONE_OBS_DELTA: only
+// the lanes in `changed` (the warp's mask of rows this step changes) build their row; every other row of p.zone_obs
+// already holds what this step would write, and a warp whose valid rows all change (every TimedTSP step) still sends
+// its span with the one bulk copy.  Returns true when the bulk copy went out; otherwise the staged rows are left for
+// send_rows.  One zone_row for both ways: a second inlined copy reloads the spilled parts of `env` a second time.
+template <int TASK, int N>
+__device__ __forceinline__ bool zone_obs_step(const KParams& p, const Env<N>& env, float* stage, int lane, int warp_env0,
+                                              unsigned changed) {
+  constexpr int ROW = N * ZoneDim<TASK>::Z;
+  const int n_valid = max(0, min(32, p.B - warp_env0));
+  const unsigned all = n_valid >= 32 ? kFull : (1u << n_valid) - 1u;
+  const unsigned m = (p.flags & CRL_STEP_ZONE_OBS_DELTA) ? changed : all;
+  if ((m >> lane) & 1u) zone_row<TASK, N>(p, env, stage + lane * ROW);
+  if (m != all) return false;
+  zone_obs_issue<TASK, N>(p, stage, lane, warp_env0, 32);
+  return true;
 }
 
 __device__ __forceinline__ void zone_obs_wait(int lane) {
@@ -1101,13 +1121,15 @@ __global__ void __maxnreg__(MaxRegs<N>::v) step_kernel(const __grid_constant__ K
     }
   }
   int fired_out = -1;
-  // lanes whose zone_obs row changed, when the rows go straight to the host (zone_obs_host): parked in shared
-  // memory, not in a register that would be live across the whole task logic of the ordinary step
+  // lanes whose zone_obs row changed, when only those rows are written (zone_obs_host, CRL_STEP_ZONE_OBS_DELTA):
+  // parked in shared memory, not in a register that would be live across the whole task logic of the ordinary step.
+  // A physics-only step changes no row.
   __shared__ unsigned s_rows_mask[kThreads / 32];
-  if (p.zone_obs_host && lane == 0) s_rows_mask[warp] = 0u;
+  const bool some_rows = p.zone_obs_host || (p.flags & CRL_STEP_ZONE_OBS_DELTA);
+  if (some_rows && lane == 0) s_rows_mask[warp] = 0u;
   bool fresh = false;   // true: this env was rebuilt by the auto-reset, no physics this call
   if (!(p.flags & CRL_STEP_PHYSICS_ONLY)) {
-    // does this step rewrite the env's zone_obs row with different bytes? (CRL_STEP_TRACK_ROWS)
+    // does this step rewrite the env's zone_obs row with different bytes? (CRL_STEP_TRACK_ROWS, CRL_STEP_ZONE_OBS_DELTA)
     // TimedTSP's time-left column moves every step: the whole row counts as changed -- unless the host mirror is
     // plane-major (CRL_STEP_HOST_PLANES), where that column is shipped as its own contiguous plane every step
     bool row_changed = TASK == CRL_TASK_TTSP && !(p.flags & CRL_STEP_HOST_PLANES);
@@ -1191,16 +1213,16 @@ __global__ void __maxnreg__(MaxRegs<N>::v) step_kernel(const __grid_constant__ K
       park_now = (p.flags & CRL_STEP_WAIT) && done && !(p.flags & CRL_STEP_AUTO_RESET);
       if (parked) { reward = 0.f; event = 0; }
     }
-    if (p.flags & CRL_STEP_TRACK_ROWS) {
+    if (p.flags & (CRL_STEP_TRACK_ROWS | CRL_STEP_ZONE_OBS_DELTA)) {
       // a finished env's row changes too, if it is rebuilt below
       const bool ch = (live && (row_changed || fired >= 0 || (done && (p.flags & CRL_STEP_AUTO_RESET)))) || parked;
       const unsigned cm = __ballot_sync(kFull, ch);
-      if (cm) {
+      // the rows themselves are written below: to the host mirror, or only these rows of the device zone_obs
+      if (some_rows && lane == 0) s_rows_mask[warp] = cm;
+      if ((p.flags & CRL_STEP_TRACK_ROWS) && cm) {
         uint32_t base = 0u;
         if (lane == 0) base = atomicAdd(p.row_list, (uint32_t)__popc(cm));
-        if (p.zone_obs_host) {
-          if (lane == 0) s_rows_mask[warp] = cm;   // the rows themselves go straight to the host mirror, below
-        } else {
+        if (!p.zone_obs_host) {
           base = __shfl_sync(kFull, base, 0);
           if (ch) p.row_list[4u + base + (uint32_t)__popc(cm & ((1u << lane) - 1u))] = (uint32_t)e;
         }
@@ -1274,8 +1296,20 @@ __global__ void __maxnreg__(MaxRegs<N>::v) step_kernel(const __grid_constant__ K
     // (6) zone_obs leaves now and drains under the physics
     // (CRL_STEP_NO_ZONE_OBS: a consumer that builds the zone rows from the state planes itself --
     // crl_zone_encode_state -- needs neither the rows nor their 360 / 420 / 168 bytes per env-step)
-    if (!(p.flags & CRL_STEP_NO_ZONE_OBS)) zone_obs_send<TASK, N>(p, env, live, stage, lane, warp_env0, false);
-    if (p.zone_obs_host) rows_to_host<TASK, N>(p, stage, s_rows_mask[warp], lane, warp_env0);
+    // Staged rows that still go out one by one, through ONE call site of send_rows (each costs spill reloads): the
+    // changed rows of a CRL_STEP_ZONE_OBS_DELTA step into zone_obs, or those of a host-direct step into the host
+    // mirror (never both, see step_launch)
+    unsigned rows = 0u;
+    if (some_rows) {
+      __syncwarp();
+      rows = s_rows_mask[warp];
+    }
+    if (!(p.flags & CRL_STEP_NO_ZONE_OBS) && zone_obs_step<TASK, N>(p, env, stage, lane, warp_env0, rows) && !p.zone_obs_host)
+      rows = 0u;
+    if (rows || p.zone_obs_host) {
+      __syncwarp();
+      send_rows<TASK, N>(p, p.zone_obs_host ? p.zone_obs_host : p.zone_obs, stage, rows, lane, warp_env0);
+    }
     // (7) physics: all frameskip substeps in registers
     if (fresh) {
       sincosf(env.b.phi, &s, &c);
@@ -1292,7 +1326,7 @@ __global__ void __maxnreg__(MaxRegs<N>::v) step_kernel(const __grid_constant__ K
   } else {
     if (!(p.flags & CRL_STEP_NO_ZONE_OBS))
       zone_obs_send<TASK, N>(p, env, live || revive, stage, lane, warp_env0, parked && !revive);
-    if (p.zone_obs_host) rows_to_host<TASK, N>(p, stage, s_rows_mask[warp], lane, warp_env0);
+    if (p.zone_obs_host) send_rows<TASK, N>(p, p.zone_obs_host, stage, s_rows_mask[warp], lane, warp_env0);
     // an env rebuilt by the auto-reset still integrates its OLD body: the shaped reward of the
     // episode's last step is measured at the post-physics position (TSP_next_city_env.py:57-67)
     Body pb = fresh ? old_b : env.b;
@@ -1814,6 +1848,9 @@ static int step_launch(const CrlConfig* c, const CrlState* st, const float* acti
   if ((flags & CRL_STEP_HOST_PLANES) && (!zone_obs_host || c->task != CRL_TASK_TTSP)) return CRL_ERR_CONFIG;
   // the walls live in the EXT kernels only (the plain rollout kernels keep their register allocation)
   const bool ext = (flags & (CRL_STEP_GOALS | CRL_STEP_WAIT)) != 0u || c->walled != 0u;
+  if ((flags & CRL_STEP_ZONE_OBS_DELTA) && (ext || zone_obs_host || (flags & CRL_STEP_NO_ZONE_OBS))) return CRL_ERR_CONFIG;
+  // every TimedTSP row changes every step (time left): the flag would only add the per-row predicate to the step
+  if (c->task == CRL_TASK_TTSP) p.flags &= ~CRL_STEP_ZONE_OBS_DELTA;
   // Programmatic launch (this grid may start while its predecessor drains) is safe when the
   // kernel then waits for the whole predecessor (plain, chain start) or for its own previous
   // step (chained).  After a CHAINED launch, though, "the predecessor is complete" no longer

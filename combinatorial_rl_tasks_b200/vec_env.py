@@ -10,7 +10,8 @@ reference (main/src/torch_ac/torch_utils/penv.py:23-69 over main/envs/make_env.p
   main/src/utils/format.py:27-28 builds), ``reward`` (B,) f32, ``done`` (B,) bool,
   ``info`` = dict of tensors {'goal_met' (B,) bool, 'cost' zeros, 'event' (B,) int8};
 * the returned tensors are persistent buffers owned by the env and overwritten by the
-  next call (clone what must outlive a step);
+  next call (clone what must outlive a step).  They are READ-ONLY for the caller: a step
+  rewrites only the ``zone_obs`` rows that change, so an in-place edit would survive it;
 * calls are asynchronous on the current CUDA stream.
 
 All arithmetic happens in libcrl_b200.so (include/crl_b200.h); torch only owns the
@@ -137,6 +138,9 @@ class ZoneVecEnv:
         # envs whose zone_obs row changed in the last step (CRL_STEP_TRACK_ROWS, step_host)
         self._row_list = z(4 + B, dtype=torch.int32)
         self._mirror_ok = False                   # True: the host zone_obs buffer equals the device one
+        # True: the bound zone_obs tensor holds the rows of the current state, so a step may write only the rows that
+        # change (CRL_STEP_ZONE_OBS_DELTA).  Set by a full reset and by every step that writes zone_obs
+        self._zone_obs_ok = False
         self.delta_rows = 0                       # rows the last step_host moved (B = all)
         # outputs
         self._cost = z(B)
@@ -235,6 +239,7 @@ class ZoneVecEnv:
         (self.obs, self.zone_obs, self.result, self.shaped_reward, self.reward, self.done, self.goal_met, self.event,
          self.need_next_goal, self.out) = binding
         self._mirror_ok = False
+        self._zone_obs_ok = False
         self._chain_ok = False
 
     @property
@@ -249,6 +254,7 @@ class ZoneVecEnv:
     def write_zone_obs(self, on):
         self._write_zone_obs = bool(on)
         self._mirror_ok = False
+        self._zone_obs_ok = False
 
     def _guard(self):
         """Make this env's device current for the call; free when it already is (the usual case)."""
@@ -286,6 +292,7 @@ class ZoneVecEnv:
         self._pf_interval = self._pf_due = max(self.prefetch_every, 1)
         self._chain_ok = False
         self._mirror_ok = False
+        self._zone_obs_ok = False
 
     def prefetch(self, stream=None, warps_per_sm=0):
         """One sampler round (crl_prefetch_layouts): fill the empty next-layout slots.
@@ -381,6 +388,9 @@ class ZoneVecEnv:
             self.gpu_launches += 1
             self._chain_ok = False
             self._mirror_ok = False
+            # a reset of every env writes every row; after a masked reset or host-supplied layouts the next step
+            # writes them all
+            self._zone_obs_ok = layout is None and mask is None
             if self.prefetch_every and not torch.cuda.is_current_stream_capturing():
                 # the reset above must be visible to the prefetcher: same-stream launch
                 self.prefetch(torch.cuda.current_stream(self.device))
@@ -396,6 +406,9 @@ class ZoneVecEnv:
             flags |= self._mode_flags
         if not self._write_zone_obs:
             flags |= _lib.STEP_NO_ZONE_OBS
+        elif self._zone_obs_ok and not flags & (_lib.STEP_GOALS | _lib.STEP_WAIT) and not self.spec.walled:
+            # only the rows that change are written (the goal-conditioned, WaitWrapper and walled kernels write all)
+            flags |= _lib.STEP_ZONE_OBS_DELTA
         with self._guard():
             if actions is None:
                 aptr = None
@@ -412,13 +425,16 @@ class ZoneVecEnv:
         self.gpu_launches += 1
         self._chain_ok = bool(chained)
         self._mirror_ok = False
+        self._zone_obs_ok = self._write_zone_obs
         if self.prefetch_every and not torch.cuda.is_current_stream_capturing():
             self.tick()
         return self._obs_dict(), self.reward, self.done, self._info()
 
     def step(self, actions):
         """ParallelEnv.step (penv.py:52-59): finished envs restart inside the call; their
-        returned observation is the new episode's first one, reward/done/info the old one's."""
+        returned observation is the new episode's first one, reward/done/info the old one's.
+        The returned tensors are the env's own buffers and READ-ONLY for the caller: once ``zone_obs``
+        holds the current rows, a step rewrites only the rows that change, so an in-place edit would stay."""
         # with wait=True a parked env (finished under step_no_reset) is WaitWrapper's no-op followed by
         # the worker's reset: (first obs of the new episode, 0, True, {}) -- wrappers.py:36-44, penv.py:7-10
         return self._step(actions, (_lib.STEP_AUTO_RESET if self.auto_reset else 0) | (_lib.STEP_WAIT if self.wait else 0))
@@ -426,7 +442,8 @@ class ZoneVecEnv:
     def step_no_reset(self, actions):
         """ParallelEnv.step_no_reset (penv.py:61-66).  With ``wait=True`` (the reference wraps each
         env in WaitWrapper for the hierarchical collectors) an env that finished earlier is a
-        no-op: zero observation, reward 0, done True, until reset()."""
+        no-op: zero observation, reward 0, done True, until reset().  The returned tensors are
+        read-only for the caller, as with step()."""
         return self._step(actions, _lib.STEP_WAIT if self.wait else 0)
 
     # -- goal RPCs of the goal-conditioned variants (zone-goals penv.py:75-99), batched ------
@@ -480,7 +497,11 @@ class ZoneVecEnv:
         """A step with U(-1,1)^2 actions drawn in-kernel (Philox): action_space.sample().
         ``chained=True`` for back-to-back rollout steps with nothing else enqueued in between.
         ``replayable=True`` (CRL_STEP_ACTION_COUNTER): the draw's step index advances on the device, so a
-        CUDA graph that captured this call draws fresh iid actions at every replay."""
+        CUDA graph that captured this call draws fresh iid actions at every replay.  The returned tensors
+        are read-only for the caller, as with step().  A captured step keeps the zone_obs mode it was
+        captured with: captured while ``zone_obs`` held the current rows, every replay writes only the rows
+        that change, so the graph must not be replayed after anything that leaves stale rows there
+        (bind_outputs, a step with ``write_zone_obs = False``, load_state_dict, a masked reset)."""
         flags = (_lib.STEP_AUTO_RESET if auto_reset else 0) | (_lib.STEP_ACTION_COUNTER if replayable else 0)
         return self._step(None, flags, action_seed, chained=chained)
 
@@ -527,6 +548,7 @@ class ZoneVecEnv:
             self._step_index += 1
             self.gpu_launches += 1
             self._chain_ok = False
+            self._zone_obs_ok = True              # the kernel writes all of the device zone_obs as well
             if self.prefetch_every:
                 self.tick()
             return h['ret']
@@ -585,6 +607,7 @@ class ZoneVecEnv:
         self.gpu_launches += 1
         self._chain_ok = False                    # memcpys follow the step kernel on the stream
         self._mirror_ok = True
+        self._zone_obs_ok = True                  # every path above writes all of the device zone_obs
         if self.prefetch_every:
             self.tick()                           # the background sampler's cadence, as in _step
         return h['ret']
@@ -734,6 +757,7 @@ class ZoneVecEnv:
             self.stamp[2].copy_(d['action_count'])
         self._chain_ok = False
         self._mirror_ok = False
+        self._zone_obs_ok = False
         if self.prefetch_every and self.state.bank_zone_xy is None:
             self.prefetch(torch.cuda.current_stream(self.device))
 
@@ -747,6 +771,7 @@ class ZoneVecEnv:
                                                   self._stream()))
         self._chain_ok = False
         self._mirror_ok = False
+        self._zone_obs_ok = False
 
     def get_qpos_qvel(self, env_ids=None):
         n = self.num_envs if env_ids is None else len(env_ids)

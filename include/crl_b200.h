@@ -147,6 +147,14 @@ enum CrlError {
  * would cross PCIe every step (420 B per env); plane-major, that column is one contiguous [B][N] plane the step
  * writes with coalesced stores (60 B per env), and only the rows of visits and resets touch the other six planes. */
 #define CRL_STEP_HOST_PLANES 1024u
+/* The step writes only the zone_obs rows whose bytes change -- the rows CRL_STEP_TRACK_ROWS lists: a zone fired, the env
+ * was rebuilt by the auto-reset, a ColourMatch cooldown ticked, every TimedTSP row -- and leaves every other row of
+ * CrlOut.zone_obs untouched.  PRECONDITION: out->zone_obs holds the rows of the state the step starts from, as a crl_reset
+ * of all envs or a step that wrote zone_obs left them.  PointTSP then moves 224 instead of 584 bytes per env-step, plus a
+ * row for each zone event and reset.  TimedTSP ignores the flag (its time-left column moves every step).  Not with CRL_STEP_NO_ZONE_OBS, the host-direct steps (crl_step_host_delta with
+ * CRL_STEP_HOST_ZERO_COPY, crl_host_call_step) or the goal-conditioned / WaitWrapper / walled kernels (CRL_STEP_GOALS,
+ * CRL_STEP_WAIT, CrlConfig.walled): CRL_ERR_CONFIG.  A library that ignores the bit writes every row: the same bytes. */
+#define CRL_STEP_ZONE_OBS_DELTA 2048u
 
 /* how a reset chooses the episode's seed; wrappers.py:10-23 and Engine.seed/reset */
 enum CrlSeedMode {
@@ -269,7 +277,8 @@ const char* crl_strerror(int code);
 #define CRL_NUM_PLANES 23
 int crl_plane_bytes(const CrlConfig* cfg, int64_t* out_bytes, int32_t n);
 
-/* Algorithmic HBM bytes one env-step moves in this layout: read, written. */
+/* Algorithmic HBM bytes one env-step moves in this layout: read, written.  The written figure counts the whole zone_obs
+ * row; a CRL_STEP_ZONE_OBS_DELTA step writes that row only when it changes. */
 int crl_step_bytes(const CrlConfig* cfg, int64_t* bytes_read, int64_t* bytes_written);
 
 /* Engine.reset() for the envs with mask[e] != 0 (all envs if mask == NULL): choose the
