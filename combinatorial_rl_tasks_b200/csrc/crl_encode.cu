@@ -28,7 +28,7 @@
 //    of W1) that multiply the bias split into a bf16 high and low part;
 //  * epilogue 1 = one cvt.rn.relu.bf16x2.f32 per pair of values + 16-byte stores: 8 consecutive rows m of
 //    one hidden unit j are exactly one 16-byte unit of the layer-2 B operand in MN-major layout;
-//  * epilogue 2 = one max per value + the register adds + two coalesced stores per 32 values.
+//  * epilogue 2 = one max per value (NaN-propagating) + the register adds + two coalesced stores per 32 values.
 // A padding row is all zeros including its ones, hence stays exactly zero through both layers and
 // drops out of the mean by itself.
 //
@@ -291,6 +291,14 @@ __device__ __forceinline__ void load_half_row(const EncArgs& a, int tile, int m,
   }
 }
 
+// max(v, 0) that passes a NaN on, as epilogue 1's cvt.rn.relu does (fmaxf would turn it into 0): a non-finite input row
+// must give a non-finite `pooled` for its env, not a finite wrong one.  Same bits as fmaxf for every other v.
+__device__ __forceinline__ float relu_nan(float v) {
+  float r;
+  asm("max.NaN.f32 %0, %1, 0f00000000;" : "=f"(r) : "f"(v));
+  return r;
+}
+
 // relu of 32 consecutive rows m of this thread's hidden unit -> bf16 -> four 16-byte units of H1
 __device__ __forceinline__ void relu_to_h1(const uint32_t (&v)[32], uint8_t* h1_row, int c, bool in_range) {
 #ifdef CRL_ENC_DIAG_NO_H1_STORE                                 // timing diagnostic (wrong results): epilogue 1 without its shared-memory stores
@@ -316,7 +324,7 @@ __device__ __forceinline__ void relu_pool16(const uint32_t (&v)[32], float inv_n
     float s[4];
 #pragma unroll
     for (int i = 0; i < 4; ++i)
-      s[i] = fmaxf(__uint_as_float(v[8 * g + 2 * i]), 0.f) + fmaxf(__uint_as_float(v[8 * g + 2 * i + 1]), 0.f);
+      s[i] = relu_nan(__uint_as_float(v[8 * g + 2 * i])) + relu_nan(__uint_as_float(v[8 * g + 2 * i + 1]));
     q[g] = (s[0] + s[1]) + (s[2] + s[3]);
   }
   r0 = (q[0] + q[1]) * inv_n;
@@ -347,7 +355,7 @@ __device__ __forceinline__ void relu_pool_store(const uint32_t (&v)[32], float* 
     float s[4];
 #pragma unroll
     for (int i = 0; i < 4; ++i)
-      s[i] = fmaxf(__uint_as_float(v[8 * g + 2 * i]), 0.f) + fmaxf(__uint_as_float(v[8 * g + 2 * i + 1]), 0.f);
+      s[i] = relu_nan(__uint_as_float(v[8 * g + 2 * i])) + relu_nan(__uint_as_float(v[8 * g + 2 * i + 1]));
     q[g] = (s[0] + s[1]) + (s[2] + s[3]);
   }
   if (XHEAD) {                                               // crl_encoder_forward: bf16 into the head's operand image
@@ -1237,7 +1245,7 @@ __global__ void __launch_bounds__(kGroupThreads, 1) zone_encode_precise_kernel(c
           for (int u = 0; u < 4; ++u) {
             float hi[8], lo[8];
 #pragma unroll
-            for (int i = 0; i < 8; ++i) split_bf16(fmaxf(__uint_as_float(v[u * 8 + i]) + b1v, 0.f), hi[i], lo[i]);
+            for (int i = 0; i < 8; ++i) split_bf16(relu_nan(__uint_as_float(v[u * 8 + i]) + b1v), hi[i], lo[i]);
             const uint32_t at = h1_off + (uint32_t)((c * 4 + u) * 128);
             *reinterpret_cast<uint4*>(smem + o.s_h1hi + at) =
                 make_uint4(pack_bf16(hi[0], hi[1]), pack_bf16(hi[2], hi[3]), pack_bf16(hi[4], hi[5]), pack_bf16(hi[6], hi[7]));
@@ -1283,7 +1291,7 @@ __global__ void __launch_bounds__(kGroupThreads, 1) zone_encode_precise_kernel(c
 #pragma unroll
           for (int i = 0; i < 32; ++i) {
             const int slot = (row0 + i) & (a.S - 1);
-            if (slot < a.N) sum += fmaxf(__uint_as_float(v[i]) + b2v, 0.f);
+            if (slot < a.N) sum += relu_nan(__uint_as_float(v[i]) + b2v);
             if (slot == a.S - 1) {
               const int e = (tile << (7 - log2_s)) + ((row0 + i) >> log2_s);
               if (e < a.B) a.out[(size_t)e * a.h + j2] = sum * inv_n;
