@@ -27,7 +27,8 @@ SYMBOLS = ['crl_abi_version', 'crl_strerror', 'crl_plane_bytes', 'crl_step_bytes
            'crl_encoder_packed_bytes', 'crl_encoder_pack', 'crl_zone_encode', 'crl_zone_encode_state',
            'crl_encoder_head_packed_bytes', 'crl_encoder_pack_head', 'crl_encoder_head',
            'crl_encoder_workspace_bytes', 'crl_encoder_forward',
-           'crl_encoder_precise_packed_bytes', 'crl_encoder_pack_precise', 'crl_zone_encode_precise']
+           'crl_encoder_precise_packed_bytes', 'crl_encoder_pack_precise', 'crl_zone_encode_precise',
+           'crl_encoder_backward_workspace_bytes', 'crl_zone_encode_backward']
 
 
 class CrlConfig(ctypes.Structure):
@@ -117,6 +118,8 @@ def load():
     lib.crl_encoder_pack_precise.argtypes = [P(CrlEncoderShape)] + [c_void_p] * 6
     lib.crl_zone_encode_precise.argtypes = [P(CrlEncoderShape), c_int32] + [c_void_p] * 6
     lib.crl_encoder_forward.argtypes = [P(CrlEncoderShape), P(CrlConfig), P(CrlState), c_int32] + [c_void_p] * 8
+    lib.crl_encoder_backward_workspace_bytes.argtypes = [P(CrlEncoderShape), c_int32, P(c_int64)]
+    lib.crl_zone_encode_backward.argtypes = [P(CrlEncoderShape), c_int32] + [c_void_p] * 11
     for name in SYMBOLS:
         getattr(lib, name)
     if lib.crl_abi_version() != ABI_VERSION:

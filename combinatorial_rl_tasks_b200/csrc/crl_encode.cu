@@ -1309,6 +1309,303 @@ __global__ void __launch_bounds__(kGroupThreads, 1) zone_encode_precise_kernel(c
   if (t < 32) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" :: "r"(tmem_base), "r"(kTmemCols) : "memory");
 }
 
+// ---- backward: dL/d(W1, b1, W2, b2) of pooled, given g = dL/dpooled (crl_zone_encode_backward) ------------------
+// One persistent CTA per SM walks tiles of kBwdRows = 64 (env, zone-slot) rows (4 envs x 16 slots or 8 x 8; padding slots
+// are all-zero rows as in the forward, so they contribute exact zeros) and, per tile, on the tensor cores:
+//   L1   H1^T  = W1 X^T                 (recomputed exactly as the forward: same image, folded biases)  -> bf16 relu H1
+//   L2   A2^T  = W2 H1^T                                                                                   -> dH2
+//        dH2[m][i] = acc2 > 0 ? bf16(g[e(m)][i] * fp32(1/N)) : 0        (select: a masked NaN g gives 0)
+//   dH1  D^T   = W2^T dH2^T             (the W2 image read through an MN-major descriptor)
+//        dH1[m][j] = H1[m][j] > 0 ? bf16(D[m][j]) : 0                   (written over H1 in place)
+//   dW2 += dH2^T H1   (M = W2 image row, N = H1 row incl. the ones row h: column h is db2)
+//   dW1 += dH1^T X    (M = hidden unit, N = input column incl. the ones column in_dim: column in_dim is db1)
+// dW2 / dW1 stay in TMEM for the CTA's whole life (2 x 192 + 2 x 32 columns); the per-tile accumulators take the last
+// 64 columns, one M-block at a time.  At the end every CTA writes its fp32 partial to the workspace and
+// encoder_bwd_reduce_kernel sums the partials in a fixed order in fp64: no float atomics, bit-identical from run to run.
+// Operand images (no swizzle, kBwdRows = R = 64): H1 / dH1 element (m, j) at (j % 8) 16 + (j / 8) 16 R + (m / 8) 128 +
+// (m % 8) 2 -- MN-major B of L2 (LBO 16 R, SBO 128) and K-major A / B of the weight gradients (LBO 128, SBO 16 R);
+// dH2 the same keyed by the W2 image row r; X as in the forward, which read along m is the MN-major B of dW1.
+constexpr int kBwdRows = 64;
+constexpr int kBwdThreads = 256;                    // 8 warps: (TMEM lane quadrant, half of the 64 row columns)
+constexpr uint32_t kBwdW2Col = 0, kBwdW2Stride = 192, kBwdW1Col = 384, kBwdScratchCol = 448;
+
+struct BwdOffsets { uint32_t h1, dh2, x, x_bytes, bar, tmem_slot, smem_end; };
+__host__ __device__ inline BwdOffsets bwd_offsets(int h, int in_dim) {
+  const Offsets f = offsets(h, in_dim);             // the resident weight image is the forward's, at the same place
+  BwdOffsets o;
+  o.h1 = (f.packed_end + 127u) & ~127u;
+  o.dh2 = o.h1 + (uint32_t)padded_k(h) * kBwdRows * 2;
+  o.x = o.dh2 + (uint32_t)padded_m(h) * kBwdRows * 2;
+  o.x_bytes = (uint32_t)kBwdRows * padded_k1(in_dim) * 2;
+  o.bar = o.x + 2 * o.x_bytes;                        // two X buffers: the next tile is staged while dW1 reads this one
+  o.tmem_slot = o.bar + 16;                           // mbarriers: MMA completion, weights' bulk copy
+  o.smem_end = o.tmem_slot + 16;
+  return o;
+}
+// floats of one CTA's partial: dW2 | db2 as [h + 1][h] (column j of the torch layout is row j here), then dW1 | db1 as
+// [in_dim + 1][h]
+__host__ __device__ inline int64_t bwd_partial_floats(int h, int in_dim) { return (int64_t)(h + 1 + in_dim + 1) * h; }
+
+struct BwdArgs {
+  const float *obs, *zone_obs, *g;
+  const uint8_t* packed;
+  float* part;
+  int* status;
+  int B, N, Z, obs_dim, h, n_tiles, S;
+};
+
+// eight consecutive values (k = 8 kc ..) of row m of a backward tile; zeros for padding rows and rows beyond the batch
+__device__ __forceinline__ void bwd_load_chunk(const BwdArgs& a, int tile, int m, int kc, float (&x)[8]) {
+#pragma unroll
+  for (int j = 0; j < 8; ++j) x[j] = 0.f;
+  const int sh = a.S == 16 ? 4 : 3;
+  const int e = tile * (kBwdRows >> sh) + (m >> sh), slot = m & (a.S - 1);
+  const int in_dim = a.obs_dim + a.Z;
+  if (tile < a.n_tiles && e < a.B && slot < a.N && 8 * kc < padded_k1(in_dim)) {
+    const float* ob = a.obs + (size_t)e * a.obs_dim;
+    const float* zo = a.zone_obs + ((size_t)e * a.N + slot) * a.Z;
+#pragma unroll
+    for (int j = 0; j < 8; ++j) {
+      const int k = 8 * kc + j;
+      if (k < a.obs_dim) x[j] = __ldg(ob + k);
+      else if (k < in_dim) x[j] = __ldg(zo + (k - a.obs_dim));
+      else if (k <= in_dim + 1) x[j] = 1.f;
+    }
+  }
+}
+
+__device__ __forceinline__ float bf16_bits_to_float(uint32_t b) { return __uint_as_float(b << 16); }
+
+__global__ void __launch_bounds__(kBwdThreads, 1) zone_encode_backward_kernel(const BwdArgs a) {
+  extern __shared__ __align__(128) uint8_t smem[];
+  const int in_dim = a.obs_dim + a.Z;
+  const Offsets fo = offsets(a.h, in_dim);
+  const BwdOffsets o = bwd_offsets(a.h, in_dim);
+  const int KP = padded_k(a.h), MP = padded_m(a.h), kK1 = padded_k1(in_dim), n_mb = MP / 128;
+  const int t = threadIdx.x, lane = t & 31;
+  const int warp = __shfl_sync(0xffffffffu, t >> 5, 0);
+  const int q = warp & 3, ch = warp >> 2;                     // lane quadrant, rows m = 32 ch .. 32 ch + 31
+  const bool leader = elect_one();
+  const uint32_t bar = smem_u32(smem + o.bar), wbar = bar + 8u;
+  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(smem + o.tmem_slot);
+  if (t == 0) {
+    mbar_init(bar, 1);
+    mbar_init(wbar, 1);
+    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    bulk_load_weights(wbar, smem_u32(smem), a.packed, fo.packed_end);
+  }
+  if (t < 32) {
+    __syncwarp();
+    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" :: "r"(smem_u32(tmem_slot)), "r"(kTmemCols) : "memory");
+    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+  }
+  tc_fence_before();
+  __syncthreads();
+  tc_fence_after();
+  const uint32_t tmem_base = *tmem_slot;
+  const uint32_t lane_addr = (uint32_t)(q * 32) << 16;
+  const uint32_t scratch = tmem_base + kBwdScratchCol;
+  // instruction descriptors (D fp32, A / B bf16, M = 128): bit 15 = A MN-major, bit 16 = B MN-major
+  const uint32_t id_base = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(128 >> 4) << 24);
+  const uint32_t id_rows = id_base | ((uint32_t)(kBwdRows >> 3) << 17);               // N = 64 rows
+  const uint32_t id_l2 = id_rows | (1u << 16), id_dh1 = id_rows | (1u << 15) | (1u << 16);
+  const uint32_t id_dw2 = id_base | ((uint32_t)(KP >> 3) << 17);                       // N = H1 rows
+  const uint32_t id_dw1 = id_base | ((uint32_t)(kK1 >> 3) << 17) | (1u << 16);          // N = input columns
+  const uint32_t w1_addr = smem_u32(smem + fo.w1), w2_addr = smem_u32(smem + fo.w2);
+  const uint32_t h1_addr = smem_u32(smem + o.h1), dh2_addr = smem_u32(smem + o.dh2);
+  uint8_t* h1buf = smem + o.h1;
+  uint8_t* dh2buf = smem + o.dh2;
+  const float inv_n = 1.0f / (float)a.N;
+  const int sh = a.S == 16 ? 4 : 3;
+  uint32_t parity = 0u;
+  bool healthy = true;
+  // issue (warp 0, converged; one elected lane executes) + commit, then everyone waits for completion
+  auto mma_phase = [&](auto&& issue) {
+    if (warp == 0) {
+      tc_fence_after();
+      issue();
+      if (leader) mma_commit(bar);
+      __syncwarp();
+    }
+    healthy = mbar_wait(bar, parity) && healthy;
+    parity ^= 1u;
+    tc_fence_after();
+  };
+  auto phase_end = [&]() {                                    // smem written for the tensor pipe / TMEM read: next phase may go
+    fence_async_smem();
+    tc_fence_before();
+    __syncthreads();
+  };
+  // hidden unit of W2 / W1 image row r (pack_kernel's row map: M-block 1 keeps units 128 .. 191 in its upper 64 rows)
+  auto unit_of_row = [](int r) { return r < 128 ? r : (r >= 192 ? r - 64 : -1); };
+
+  const int m_st = t & (kBwdRows - 1), kc_st = t >> 6;        // the 16-byte unit of X this thread stages
+  const uint32_t x_off = (uint32_t)((m_st & 7) * 16 + (m_st >> 3) * (16 * kK1) + kc_st * 128);
+  float x[8];
+  int tile = (int)blockIdx.x;
+  bwd_load_chunk(a, tile, m_st, kc_st, x);
+  for (int k = 0; tile < a.n_tiles; tile += (int)gridDim.x, ++k) {
+    const uint32_t xb = o.x + (uint32_t)(k & 1) * o.x_bytes;
+    if (kc_st < kK1 / 8)
+      *reinterpret_cast<uint4*>(smem + xb + x_off) =
+          make_uint4(pack_bf16(x[0], x[1]), pack_bf16(x[2], x[3]), pack_bf16(x[4], x[5]), pack_bf16(x[6], x[7]));
+    phase_end();
+    bwd_load_chunk(a, tile + (int)gridDim.x, m_st, kc_st, x);  // the next tile's rows travel under this one
+    const uint32_t x_addr = smem_u32(smem + xb);
+    if (k == 0 && warp == 0) { healthy = mbar_wait(wbar, 0u) && healthy; __syncwarp(); }
+    // ---- L1, one M-block at a time, -> H1 (bf16 relu), keyed by hidden unit (ones rows h, h + 1 included) ----
+    for (int b = 0; b < n_mb; ++b) {
+      mma_phase([&] {
+        for (int s = 0; s < kK1 / 16; ++s)
+          if (leader) mma_bf16(scratch, smem_desc(w1_addr + (uint32_t)(b * 16 * 16 * kK1 + 256 * s), 128u, 16 * kK1),
+                               smem_desc(x_addr + 256u * s, 128u, 16 * kK1), id_rows, s > 0);
+      });
+      const int u = unit_of_row(128 * b + 32 * q + lane);
+      uint32_t v[32];
+      tmem_ld32(scratch + lane_addr + (uint32_t)(32 * ch), v);
+      tmem_ld_wait(v);
+      if (u >= 0) relu_to_h1(v, h1buf + (uint32_t)((u & 7) * 16 + (u >> 3) * (16 * kBwdRows)), ch, u < KP);
+      phase_end();
+    }
+    // ---- L2, one M-block at a time, -> dH2 keyed by W2 image row ----
+    for (int b = 0; b < n_mb; ++b) {
+      mma_phase([&] {
+        for (int s = 0; s < KP / 16; ++s)
+          if (leader) mma_bf16(scratch, smem_desc(w2_addr + (uint32_t)(b * 16 * 16 * KP + 256 * s), 128u, 16 * KP),
+                               smem_desc(h1_addr + (uint32_t)(2 * 16 * kBwdRows * s), 16 * kBwdRows, 128u), id_l2, s > 0);
+      });
+      const int r = 128 * b + 32 * q + lane, u = unit_of_row(r);
+      uint32_t v[32];
+      tmem_ld32(scratch + lane_addr + (uint32_t)(32 * ch), v);
+      tmem_ld_wait(v);
+      if (u >= 0) {
+        // this thread's 32 rows are the slots of 32 / S envs
+        const int e0 = tile * (kBwdRows >> sh) + ((32 * ch) >> sh);
+        float d[4];
+#pragma unroll
+        for (int i = 0; i < 4; ++i) {
+          const int e = e0 + i;
+          const float gv = (i < (32 >> sh) && u < a.h && e < a.B) ? __ldg(a.g + (size_t)e * a.h + u) : 0.f;
+          d[i] = __bfloat162float(__float2bfloat16_rn(__fmul_rn(gv, inv_n)));
+        }
+        uint8_t* row = dh2buf + (uint32_t)((r & 7) * 16 + (r >> 3) * (16 * kBwdRows));
+#pragma unroll
+        for (int qq = 0; qq < 4; ++qq) {
+          float w[8];
+#pragma unroll
+          for (int i = 0; i < 8; ++i) {
+            const int mi = 8 * qq + i, ei = mi >> sh;
+            const float dv = ei == 0 ? d[0] : (ei == 1 ? d[1] : (ei == 2 ? d[2] : d[3]));
+            w[i] = __uint_as_float(v[mi]) > 0.f ? dv : 0.f;
+          }
+          *reinterpret_cast<uint4*>(row + (uint32_t)((ch * 4 + qq) * 128)) =
+              make_uint4(pack_bf16(w[0], w[1]), pack_bf16(w[2], w[3]), pack_bf16(w[4], w[5]), pack_bf16(w[6], w[7]));
+        }
+      }
+      phase_end();
+    }
+    // ---- dW2 += dH2^T H1 (both M-blocks), and dH1^T = W2^T dH2^T one M-block at a time -> dH1 over H1 ----
+    for (int b = 0; b < n_mb; ++b) {
+      mma_phase([&] {
+        if (b == 0)
+          for (int bb = 0; bb < n_mb; ++bb)
+            for (int s = 0; s < kBwdRows / 16; ++s)
+              if (leader) mma_bf16(tmem_base + kBwdW2Col + (uint32_t)bb * kBwdW2Stride,
+                                   smem_desc(dh2_addr + (uint32_t)(bb * 16 * 16 * kBwdRows + 256 * s), 128u, 16 * kBwdRows),
+                                   smem_desc(h1_addr + 256u * s, 128u, 16 * kBwdRows), id_dw2, (k > 0 || s > 0) ? 1u : 0u);
+        bool first = true;
+        for (int s = 0; s < MP / 16; ++s) {
+          if (s >= 8 && s < 12) continue;                    // image rows 128 .. 191: zero rows of W2
+          if (leader) mma_bf16(scratch, smem_desc(w2_addr + (uint32_t)(b * 16 * 128 + 2 * 16 * KP * s), 16 * KP, 128u),
+                               smem_desc(dh2_addr + (uint32_t)(2 * 16 * kBwdRows * s), 16 * kBwdRows, 128u), id_dh1, first ? 0u : 1u);
+          first = false;
+        }
+      });
+      const int j = 128 * b + 32 * q + lane;
+      uint32_t v[32];
+      tmem_ld32(scratch + lane_addr + (uint32_t)(32 * ch), v);
+      tmem_ld_wait(v);
+      if (j < a.h) {
+        uint8_t* row = h1buf + (uint32_t)((j & 7) * 16 + (j >> 3) * (16 * kBwdRows));
+#pragma unroll
+        for (int qq = 0; qq < 4; ++qq) {
+          uint4* p = reinterpret_cast<uint4*>(row + (uint32_t)((ch * 4 + qq) * 128));
+          const uint4 hv = *p;
+          const uint32_t hw[4] = {hv.x, hv.y, hv.z, hv.w};
+          float w[8];
+#pragma unroll
+          for (int i = 0; i < 4; ++i) {
+            w[2 * i] = bf16_bits_to_float(hw[i] & 0xffffu) > 0.f ? __uint_as_float(v[8 * qq + 2 * i]) : 0.f;
+            w[2 * i + 1] = bf16_bits_to_float(hw[i] >> 16) > 0.f ? __uint_as_float(v[8 * qq + 2 * i + 1]) : 0.f;
+          }
+          *p = make_uint4(pack_bf16(w[0], w[1]), pack_bf16(w[2], w[3]), pack_bf16(w[4], w[5]), pack_bf16(w[6], w[7]));
+        }
+      }
+      phase_end();
+    }
+    // ---- dW1 += dH1^T X: completion is awaited by the next tile's first phase (before H1 / this X buffer are reused) ----
+    if (warp == 0) {
+      tc_fence_after();
+      for (int b = 0; b < n_mb; ++b)
+        for (int s = 0; s < kBwdRows / 16; ++s)
+          if (leader) mma_bf16(tmem_base + kBwdW1Col + (uint32_t)(32 * b),
+                               smem_desc(h1_addr + (uint32_t)(b * 16 * 16 * kBwdRows + 256 * s), 128u, 16 * kBwdRows),
+                               smem_desc(x_addr + (uint32_t)(2 * 16 * kK1 * s), 16 * kK1, 128u), id_dw1, (k > 0 || s > 0) ? 1u : 0u);
+      __syncwarp();
+    }
+  }
+  // ---- the CTA's partial: TMEM -> workspace (transposed: consecutive lanes = consecutive hidden units, coalesced) ----
+  mma_phase([&] {});                                           // every MMA issued so far has completed
+  float* part = a.part + (size_t)blockIdx.x * (size_t)bwd_partial_floats(a.h, in_dim);
+  for (int b = 0; b < n_mb; ++b) {
+    const int u = unit_of_row(128 * b + 32 * q + lane);
+    for (int c = ch; c * 32 <= a.h; c += 2) {                 // columns 0 .. h (h: the ones row -> db2)
+      uint32_t v[32];
+      tmem_ld32(tmem_base + lane_addr + kBwdW2Col + (uint32_t)b * kBwdW2Stride + (uint32_t)(32 * c), v);
+      tmem_ld_wait(v);
+      if (u >= 0 && u < a.h)
+#pragma unroll
+        for (int i = 0; i < 32; ++i)
+          if (32 * c + i <= a.h) part[(size_t)(32 * c + i) * a.h + u] = __uint_as_float(v[i]);
+    }
+    if (ch == 0) {                                             // columns 0 .. in_dim (in_dim: the ones column -> db1)
+      const int j = 128 * b + 32 * q + lane;
+      uint32_t v[32];
+      tmem_ld32(tmem_base + lane_addr + kBwdW1Col + (uint32_t)(32 * b), v);
+      tmem_ld_wait(v);
+      float* p1 = part + (size_t)(a.h + 1) * a.h;
+      if (j < a.h)
+#pragma unroll
+        for (int i = 0; i < 32; ++i)
+          if (i <= in_dim) p1[(size_t)i * a.h + j] = __uint_as_float(v[i]);
+    }
+  }
+  if (!healthy && a.status) atomicExch(a.status, 1);
+  tc_fence_before();
+  __syncthreads();
+  if (t < 32) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" :: "r"(tmem_base), "r"(kTmemCols) : "memory");
+}
+
+// element i of the partials, summed over the n_part CTAs in index order in fp64 -> torch-layout fp32 outputs
+struct BwdReduceArgs { const float* part; float *dw1, *db1, *dw2, *db2; int n_part, h, in_dim; };
+__global__ void encoder_bwd_reduce_kernel(const BwdReduceArgs a) {
+  const int64_t n = bwd_partial_floats(a.h, a.in_dim), e2 = (int64_t)(a.h + 1) * a.h;
+  for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+    double s = 0.0;
+    for (int p = 0; p < a.n_part; ++p) s += (double)__ldg(a.part + (size_t)p * n + i);
+    const float v = (float)s;
+    if (i < e2) {
+      const int col = (int)(i / a.h), u = (int)(i % a.h);
+      if (col < a.h) a.dw2[(size_t)u * a.h + col] = v;
+      else a.db2[u] = v;
+    } else {
+      const int col = (int)((i - e2) / a.h), u = (int)((i - e2) % a.h);
+      if (col < a.in_dim) a.dw1[(size_t)u * a.in_dim + col] = v;
+      else a.db1[u] = v;
+    }
+  }
+}
+
 static int check_shape(const CrlEncoderShape* s) {
   if (!s) return CRL_ERR_NULL;
   if (s->obs_dim <= 0 || s->zone_dim <= 0 || s->obs_dim + s->zone_dim + 1 > 32) return CRL_ERR_CONFIG;   // + a ones column
@@ -1574,6 +1871,65 @@ int crl_zone_encode_precise(const CrlEncoderShape* s, int32_t num_envs, const fl
   const int want = a.n_tiles * nb, cap = sms / nb * nb;       // CTA c owns M-block c % nb of tiles c / nb, c / nb + grid / nb, ..
   const int grid = want < cap ? want : cap;
   zone_encode_precise_kernel<<<grid, kGroupThreads, o.s_end, static_cast<cudaStream_t>(stream)>>>(a);
+  return cudaGetLastError() == cudaSuccess ? CRL_OK : CRL_ERR_LAUNCH;
+}
+
+// ---- backward ----
+// the launch rule: one partial per CTA, grid = min(tiles of kBwdRows rows, SMs of the current device)
+static int bwd_grid(const CrlEncoderShape* s, int32_t num_envs, int* grid, int* n_tiles) {
+  int dev = 0, sms = 148;
+  if (cudaGetDevice(&dev) != cudaSuccess) return CRL_ERR_DEVICE;
+  if (cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess) return CRL_ERR_DEVICE;
+  const int per_tile = kBwdRows / slots_per_env(s->num_zones);
+  *n_tiles = (int)(((int64_t)num_envs + per_tile - 1) / per_tile);
+  *grid = *n_tiles < sms ? *n_tiles : sms;
+  return CRL_OK;
+}
+
+int crl_encoder_backward_workspace_bytes(const CrlEncoderShape* s, int32_t num_envs, int64_t* bytes) {
+  const int rc = check_shape(s);
+  if (rc) return rc;
+  if (!bytes) return CRL_ERR_NULL;
+  if (num_envs <= 0) return CRL_ERR_CONFIG;
+  int grid = 0, n_tiles = 0;
+  const int rg = bwd_grid(s, num_envs, &grid, &n_tiles);
+  if (rg) return rg;
+  *bytes = (int64_t)grid * bwd_partial_floats(s->hidden, s->obs_dim + s->zone_dim) * 4;
+  return CRL_OK;
+}
+
+int crl_zone_encode_backward(const CrlEncoderShape* s, int32_t num_envs, const float* obs, const float* zone_obs,
+                             const void* packed, const float* grad_pooled, void* workspace, float* dw1, float* db1,
+                             float* dw2, float* db2, int32_t* status, void* stream) {
+  const int rc = check_shape(s);
+  if (rc) return rc;
+  if (!obs || !zone_obs || !packed || !grad_pooled || !workspace || !dw1 || !db1 || !dw2 || !db2) return CRL_ERR_NULL;
+  if (num_envs <= 0) return CRL_ERR_CONFIG;
+  if ((reinterpret_cast<uintptr_t>(packed) | reinterpret_cast<uintptr_t>(workspace)) & 15u) return CRL_ERR_ALIGN;
+  const BwdOffsets o = bwd_offsets(s->hidden, s->obs_dim + s->zone_dim);
+  if (o.smem_end > 227u * 1024u) return CRL_ERR_UNSUPPORTED;
+  int grid = 0, n_tiles = 0;
+  const int rg = bwd_grid(s, num_envs, &grid, &n_tiles);
+  if (rg) return rg;
+  int dev = 0;
+  if (cudaGetDevice(&dev) != cudaSuccess) return CRL_ERR_DEVICE;
+  static bool attr_set[64] = {false};
+  if (dev < 0 || dev >= 64 || !attr_set[dev]) {
+    if (cudaFuncSetAttribute(zone_encode_backward_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024) != cudaSuccess)
+      return CRL_ERR_DEVICE;
+    if (dev >= 0 && dev < 64) attr_set[dev] = true;
+  }
+  BwdArgs a{};
+  a.obs = obs; a.zone_obs = zone_obs; a.g = grad_pooled; a.packed = static_cast<const uint8_t*>(packed);
+  a.part = static_cast<float*>(workspace); a.status = status;
+  a.B = num_envs; a.N = s->num_zones; a.Z = s->zone_dim; a.obs_dim = s->obs_dim; a.h = s->hidden;
+  a.S = slots_per_env(s->num_zones); a.n_tiles = n_tiles;
+  const cudaStream_t cs = static_cast<cudaStream_t>(stream);
+  zone_encode_backward_kernel<<<grid, kBwdThreads, o.smem_end, cs>>>(a);
+  if (cudaGetLastError() != cudaSuccess) return CRL_ERR_LAUNCH;
+  const BwdReduceArgs r{static_cast<const float*>(workspace), dw1, db1, dw2, db2, grid, s->hidden, s->obs_dim + s->zone_dim};
+  const int64_t n = bwd_partial_floats(s->hidden, s->obs_dim + s->zone_dim);
+  encoder_bwd_reduce_kernel<<<(int)((n + 255) / 256), 256, 0, cs>>>(r);
   return cudaGetLastError() == cudaSuccess ? CRL_OK : CRL_ERR_LAUNCH;
 }
 

@@ -12,12 +12,24 @@ operand image directly (no fp32 ``pooled`` in between), the second fetches it wi
     emb = enc(env.obs, env.zone_obs)                        # == model(DictList(obs=..., zone_obs=...))
 
 All GEMMs run with bf16 operands and fp32 accumulation (the reference: fp32; biases ride in the GEMMs as bf16
-hi + lo pairs).  Inference only -- no autograd graph is built.  There is no CPU path: the constructor raises
-without CUDA.
+hi + lo pairs).  ``ZoneEncoder`` is inference only -- no autograd graph is built.  There is no CPU path: the
+constructors raise without CUDA.
+
+Training: ``FusedZoneEnvModel`` is a drop-in ``nn.Module`` for the reference's ``ZoneEnvModel`` (same parameter names,
+so ``state_dict`` loads strictly either way) whose ``pooled`` runs forward AND backward on the tensor cores
+(crl_zone_encode / crl_zone_encode_backward: H1 and the layer-2 pre-activation are recomputed per tile, the (B N, h)
+activations and their gradients never reach memory, dW1 / db1 / dW2 / db2 are summed per CTA and reduced in a fixed
+order in fp64).  The B-row rest -- ``zone_net_[4]`` and ``combine_net_`` -- is ordinary fp32 torch autograd on
+``pooled``.  Gradients reach the first two Linears only; ``obs`` / ``zone_obs`` that require grad are refused.
+
+    model = FusedZoneEnvModel(obs_dim=8, zone_dim=6, num_zones=15, hidden=185).cuda()
+    model.load_state_dict(reference_model.state_dict())     # strict: the reference's keys
+    loss = f(model(obs_dict)); loss.backward(); opt.step()
 """
 import ctypes
 
 import torch
+import torch.nn as nn
 
 from . import _lib
 
@@ -231,3 +243,108 @@ class ZoneEncoder:
         if zone_obs is None:
             obs, zone_obs = obs['obs'], obs['zone_obs']
         return self._forward(obs, zone_obs)
+
+
+class _FusedCore:
+    """The library calls behind FusedZoneEnvModel for one (obs_dim, zone_dim, hidden, num_zones): the packed weight
+    image (one buffer, re-packed by every forward and backward from the weights they were given) and the backward's
+    workspace (one batch size at a time)."""
+
+    def __init__(self, obs_dim, zone_dim, hidden, num_zones, device):
+        self.lib = _lib.load()
+        self.device = device
+        self.shape = _lib.CrlEncoderShape(obs_dim=obs_dim, zone_dim=zone_dim, hidden=hidden, num_zones=num_zones)
+        n = ctypes.c_int64()
+        _lib.check(self.lib.crl_encoder_packed_bytes(self.shape, ctypes.byref(n)))
+        self.packed = torch.zeros(n.value, dtype=torch.uint8, device=device)
+        self.status = torch.zeros(1, dtype=torch.int32, device=device)
+        self._ws = (None, None)
+
+    def _stream(self):
+        return ctypes.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
+
+    def pack(self, w1, b1, w2, b2):
+        with torch.cuda.device(self.device):
+            _lib.check(self.lib.crl_encoder_pack(self.shape, w1.data_ptr(), b1.data_ptr(), w2.data_ptr(), b2.data_ptr(),
+                                                 self.packed.data_ptr(), self._stream()))
+
+    def pooled(self, obs, zone_obs):
+        out = torch.empty(obs.shape[0], self.shape.hidden, dtype=torch.float32, device=self.device)
+        with torch.cuda.device(self.device):
+            _lib.check(self.lib.crl_zone_encode(self.shape, obs.shape[0], obs.data_ptr(), zone_obs.data_ptr(),
+                                                self.packed.data_ptr(), out.data_ptr(), self.status.data_ptr(),
+                                                self._stream()))
+        return out
+
+    def backward(self, obs, zone_obs, grad_pooled):
+        B, h, in_dim = obs.shape[0], self.shape.hidden, self.shape.obs_dim + self.shape.zone_dim
+        if self._ws[0] != B:
+            n = ctypes.c_int64()
+            with torch.cuda.device(self.device):
+                _lib.check(self.lib.crl_encoder_backward_workspace_bytes(self.shape, B, ctypes.byref(n)))
+            self._ws = (B, torch.empty(n.value, dtype=torch.uint8, device=self.device))
+        f = lambda *s: torch.empty(*s, dtype=torch.float32, device=self.device)
+        dw1, db1, dw2, db2 = f(h, in_dim), f(h), f(h, h), f(h)
+        with torch.cuda.device(self.device):
+            _lib.check(self.lib.crl_zone_encode_backward(
+                self.shape, B, obs.data_ptr(), zone_obs.data_ptr(), self.packed.data_ptr(), grad_pooled.data_ptr(),
+                self._ws[1].data_ptr(), dw1.data_ptr(), db1.data_ptr(), dw2.data_ptr(), db2.data_ptr(),
+                self.status.data_ptr(), self._stream()))
+        return dw1, db1, dw2, db2
+
+
+class _FusedPooled(torch.autograd.Function):
+    """pooled = mean_z relu(W2 relu(W1 [obs, zone_obs[:, z]] + b1) + b2) with gradients for W1, b1, W2, b2."""
+
+    @staticmethod
+    def forward(ctx, core, obs, zone_obs, w1, b1, w2, b2):
+        if obs.requires_grad or zone_obs.requires_grad:
+            raise RuntimeError('FusedZoneEnvModel: gradients with respect to obs / zone_obs are not computed; '
+                               'detach the inputs')
+        core.pack(w1, b1, w2, b2)
+        ctx.core = core
+        ctx.save_for_backward(obs, zone_obs, w1, b1, w2, b2)    # the version counters catch an in-place update
+        return core.pooled(obs, zone_obs)
+
+    @staticmethod
+    def backward(ctx, grad_pooled):
+        obs, zone_obs, w1, b1, w2, b2 = ctx.saved_tensors
+        ctx.core.pack(w1, b1, w2, b2)                             # the image of exactly the weights the forward used
+        dw1, db1, dw2, db2 = ctx.core.backward(obs, zone_obs, grad_pooled.contiguous())
+        return None, None, None, dw1, db1, dw2, db2
+
+
+class FusedZoneEnvModel(nn.Module):
+    """The reference's ZoneEnvModel (env_model.py:48-79) with its (B N)-row part forward and backward on the tensor
+    cores.  ``forward(obs)`` takes the env's obs dict or an object with ``.obs`` / ``.zone_obs`` (the reference's DictList)
+    and returns ``combine_net_([obs, zone_net_[4](pooled)])``."""
+
+    def __init__(self, obs_dim, zone_dim, num_zones, hidden=185, device='cuda:0'):
+        super().__init__()
+        if not torch.cuda.is_available():
+            raise RuntimeError('FusedZoneEnvModel needs a CUDA device (sm_100a); there is no CPU fallback')
+        self.obs_dim, self.zone_dim, self.num_zones, self.hidden = int(obs_dim), int(zone_dim), int(num_zones), int(hidden)
+        self.zone_net_ = nn.Sequential(nn.Linear(obs_dim + zone_dim, hidden), nn.ReLU(), nn.Linear(hidden, hidden),
+                                       nn.ReLU(), nn.Linear(hidden, hidden))
+        self.combine_net_ = nn.Linear(obs_dim + hidden, hidden)
+        self.to(device)
+        self._core = _FusedCore(self.obs_dim, self.zone_dim, self.hidden, self.num_zones, torch.device(device))
+
+    def pooled(self, obs, zone_obs):
+        B = obs.shape[0]
+        assert obs.shape == (B, self.obs_dim) and zone_obs.shape == (B, self.num_zones, self.zone_dim)
+        assert obs.dtype == zone_obs.dtype == torch.float32
+        l1, l2 = self.zone_net_[0], self.zone_net_[2]
+        return _FusedPooled.apply(self._core, obs.contiguous(), zone_obs.contiguous(),
+                                  l1.weight.contiguous(), l1.bias.contiguous(), l2.weight.contiguous(), l2.bias.contiguous())
+
+    def forward(self, obs):
+        if isinstance(obs, dict):
+            o, z = obs['obs'], obs['zone_obs']
+        else:
+            o, z = obs.obs, obs.zone_obs
+        return self.combine_net_(torch.cat([o, self.zone_net_[4](self.pooled(o, z))], dim=-1))
+
+    def healthy(self):
+        """False if a tensor-core completion wait ever expired (synchronises)."""
+        return int(self._core.status.item()) == 0

@@ -2,10 +2,12 @@
 BaseAlgo.collect_experiences (main/src/torch_ac/algos/base.py:110-249) with a small policy of the
 reference's shape (per-zone MLP, mean over zones: main/src/env_model.py:48-79), everything on the GPU.
 
-    python examples/collect_ppo.py --env PointTSP-v0 --envs 65536 --frames 64 --updates 3 [--fused-encoder]
+    python examples/collect_ppo.py --env PointTSP-v0 --envs 65536 --frames 64 --updates 3 [--fused-encoder | --fused-train]
 
 --fused-encoder: the collection forward runs the embedding on crl.ZoneEncoder (the tcgen05 kernel, bf16 operands);
 the update keeps the torch module, whose weights are re-packed after every optimiser step.
+--fused-train: the policy embeds through crl.FusedZoneEnvModel in collection AND update: the (B N)-row part of the
+embedding runs forward and backward on the tensor cores, the rest is torch autograd.
 
 The env writes each frame straight into the rollout (no per-frame copies), crl_gae computes the
 advantages; what is left for torch is the policy itself.
@@ -49,6 +51,22 @@ class ZonePolicy(nn.Module):
         return sd
 
 
+class FusedZonePolicy(nn.Module):
+    """ZonePolicy with the embedding as crl.FusedZoneEnvModel (the reference's parameter names: env_model.zone_net_.*,
+    env_model.combine_net_.*)."""
+
+    def __init__(self, zone_dim, num_zones, h=64):
+        super().__init__()
+        self.env_model = crl.FusedZoneEnvModel(8, zone_dim, num_zones, h)
+        self.actor, self.critic = nn.Linear(h, 2), nn.Linear(h, 1)
+        self.log_std = nn.Parameter(torch.zeros(2))
+
+    def forward(self, obs):
+        return self.heads(torch.relu(self.env_model(obs)))
+
+    heads = ZonePolicy.heads
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument('--env', default='PointTSP-v0')
@@ -56,9 +74,15 @@ def main():
     ap.add_argument('--frames', type=int, default=64)
     ap.add_argument('--updates', type=int, default=3)
     ap.add_argument('--fused-encoder', action='store_true')
+    ap.add_argument('--fused-train', action='store_true')
     args = ap.parse_args()
+    if args.fused_encoder and args.fused_train:
+        ap.error('--fused-encoder and --fused-train are alternatives')
     env = crl.ZoneVecEnv(args.env, args.envs, seed_mode='fixed_range', min_seed=1, max_seed=100)   # make_train_env
-    policy = ZonePolicy(env.spec.zone_dim).cuda()
+    if args.fused_train:
+        policy = FusedZonePolicy(env.spec.zone_dim, env.spec.num_zones).cuda()
+    else:
+        policy = ZonePolicy(env.spec.zone_dim).cuda()
     opt = torch.optim.Adam(policy.parameters(), lr=3e-4)
     ro = Rollout(env, args.frames, discount=0.998, gae_lambda=0.95)
     enc = crl.ZoneEncoder(policy.encoder_state_dict(), num_zones=env.spec.num_zones) if args.fused_encoder else None

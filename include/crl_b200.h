@@ -415,8 +415,8 @@ int crl_check_state(const CrlConfig* cfg, const CrlState* st, uint64_t* violatio
  * crl_zone_encode computes `pooled` in one fused kernel on the tensor cores (tcgen05, bf16 operands,
  * fp32 accumulation in TMEM; csrc/crl_encode.cu): the (B N, h) activations the reference materialises
  * never leave the SM, and the third Linear shrinks from B N to B rows -- it and combine_net_ stay
- * fp32 library GEMMs on the caller's side.  Inference only (the rollout-time forward of
- * BaseAlgo.collect_experiences, base.py:133-140).  hidden <= 190 (the default is 185,
+ * fp32 library GEMMs on the caller's side.  The rollout-time forward of BaseAlgo.collect_experiences
+ * (base.py:133-140); crl_zone_encode_backward (below) is the training half.  hidden <= 190 (the default is 185,
  * scripts/train_ppo.py:66), obs_dim + zone_dim <= 31 (one K step up to 15, two beyond: ZoneEnvGoalModel /
  * ZoneEnvSkillModel, whose per-env goal / one-hot skill the caller concatenates to obs), num_zones <= 16. */
 typedef struct CrlEncoderShape {
@@ -479,6 +479,27 @@ int crl_encoder_pack_precise(const CrlEncoderShape* shape, const float* w1, cons
                              const float* b2, void* packed, void* stream);
 int crl_zone_encode_precise(const CrlEncoderShape* shape, int32_t num_envs, const float* obs, const float* zone_obs,
                             const void* packed_precise, float* pooled, int32_t* status, void* stream);
+
+/* BACKWARD of `pooled` (the B N-row part of ZoneEnvModel; training through the fused kernel): given
+ * grad_pooled g = dL/dpooled float[B][h], the gradients of the first two Linears in torch layout, fp32:
+ * dw1 float[h][obs_dim + zone_dim], db1 float[h], dw2 float[h][h], db2 float[h] (all overwritten, device).  The third
+ * Linear and combine_net_ act on B rows and stay with the caller (torch autograd on `pooled`).  No input gradients.
+ * `packed` is crl_encoder_pack's image of the weights the forward used; obs / zone_obs as for crl_zone_encode.
+ * Numerics: H1 and the layer-2 pre-activation are recomputed exactly as crl_zone_encode computes them (bf16 operands,
+ * fp32 accumulation, bf16 hi + lo biases); then, per row m of env e,
+ *     dH2[m][i] = acc2[m][i] > 0 ? bf16_rn(fp32(g[e][i] * fp32(1/N))) : 0     (select: a masked-off NaN g gives 0)
+ *     dH1[m][j] = H1[m][j] > 0 ? bf16_rn(sum_i W2[i][j] dH2[m][i]) : 0          (bf16 W2, fp32 accumulation)
+ *     dW2 = sum_m dH2[m]^T H1[m],  db2 = sum_m dH2[m],  dW1 = sum_m dH1[m]^T x[m],  db1 = sum_m dH1[m]
+ * with bf16 operands; padding slots contribute exact zeros.  Launch rule: the rows are cut into tiles of 64 (4 envs of 16
+ * slots, or 8 of 8 when N <= 8); grid = min(tiles, SMs of the current device); CTA c sums tiles c, c + grid, ... in fp32
+ * (at most 64 ceil(tiles / grid) rows per partial) into its own fp32 partial in `workspace`
+ * (crl_encoder_backward_workspace_bytes; contents are scratch), and a second kernel adds the partials in CTA order in
+ * fp64 and rounds once to fp32.  No float atomics: the result is bit-identical from run to run for the same B on the
+ * same device.  Same shapes as crl_zone_encode; packed and workspace 16-byte aligned.  status as for crl_zone_encode. */
+int crl_encoder_backward_workspace_bytes(const CrlEncoderShape* shape, int32_t num_envs, int64_t* bytes);
+int crl_zone_encode_backward(const CrlEncoderShape* shape, int32_t num_envs, const float* obs, const float* zone_obs,
+                             const void* packed, const float* grad_pooled, void* workspace,
+                             float* dw1, float* db1, float* dw2, float* db2, int32_t* status, void* stream);
 
 /* Copies the eight counters to the host (synchronises `stream`).  The first four (sum of
  * returns, episodes, successes, sum of lengths) are what ranks all-reduce. */
