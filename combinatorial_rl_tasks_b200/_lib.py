@@ -28,7 +28,9 @@ SYMBOLS = ['crl_abi_version', 'crl_strerror', 'crl_plane_bytes', 'crl_step_bytes
            'crl_encoder_head_packed_bytes', 'crl_encoder_pack_head', 'crl_encoder_head',
            'crl_encoder_workspace_bytes', 'crl_encoder_forward',
            'crl_encoder_precise_packed_bytes', 'crl_encoder_pack_precise', 'crl_zone_encode_precise',
-           'crl_encoder_backward_workspace_bytes', 'crl_zone_encode_backward']
+           'crl_encoder_backward_workspace_bytes', 'crl_zone_encode_backward',
+           'crl_frame_capture', 'crl_zone_encode_frames', 'crl_zone_encode_backward_frames', 'crl_frames_zone_obs']
+FRAME_NO_LAYOUT = 0xffffffff
 
 
 class CrlConfig(ctypes.Structure):
@@ -120,6 +122,11 @@ def load():
     lib.crl_encoder_forward.argtypes = [P(CrlEncoderShape), P(CrlConfig), P(CrlState), c_int32] + [c_void_p] * 8
     lib.crl_encoder_backward_workspace_bytes.argtypes = [P(CrlEncoderShape), c_int32, P(c_int64)]
     lib.crl_zone_encode_backward.argtypes = [P(CrlEncoderShape), c_int32] + [c_void_p] * 11
+    lib.crl_frame_capture.argtypes = [P(CrlConfig), P(CrlState), c_void_p, c_int32, c_void_p, c_void_p, c_void_p, c_uint32,
+                                      c_void_p, c_void_p]
+    lib.crl_zone_encode_frames.argtypes = [P(CrlEncoderShape), P(CrlConfig), c_int32] + [c_void_p] * 8
+    lib.crl_zone_encode_backward_frames.argtypes = [P(CrlEncoderShape), P(CrlConfig), c_int32] + [c_void_p] * 13
+    lib.crl_frames_zone_obs.argtypes = [P(CrlConfig), c_int32] + [c_void_p] * 5
     for name in SYMBOLS:
         getattr(lib, name)
     if lib.crl_abi_version() != ABI_VERSION:

@@ -226,40 +226,72 @@ struct EncArgs {
   const uint2* cooldown;       // uint2[B] (ColourMatch)
   int task, num_steps;
   crl::DivConst div_steps, div_cd;
+  // crl_zone_encode_frames / crl_frames_zone_obs: the zone part is built from a CrlFrame per row and the layout table
+  const uint4* frames;         // CrlFrame[B]: bits, layout, cooldown
+  const float2* layout_xy;     // float2[capacity][N]
+  const uint32_t* layout_tmax; // uint32[capacity][ceil(N/2)] (TimedTSP)
 };
 
-// Feature f of zone `slot` of env e from the state planes: EXACTLY what step_kernel's zone_row writes to
-// zone_obs[e][slot][f] (crl_kernels.cu; tests/test_gpu_encode.py compares the two paths bit for bit):
-// x/3, y/3, r, g, b, 0.25 [, time left | cooldown / max_cooldown]
-__device__ __forceinline__ void zone_features_from_state(const EncArgs& a, int e, int slot, float (&z)[7]) {
-  const float2 c = __ldg(a.zone_xy + (size_t)slot * a.B + e);
-  const uint32_t bits = (uint32_t)__float_as_int(__ldg(reinterpret_cast<const float*>(a.aux + e) + 3));
+// where the zone part of a layer-1 input row comes from
+enum RowSrc : int { kSrcZoneObs = 0, kSrcState = 1, kSrcFrames = 2 };
+
+// The features of zone `slot`: EXACTLY what step_kernel's zone_row writes to zone_obs[e][slot] (crl_kernels.cu;
+// tests/test_gpu_encode.py and tests/test_gpu_rollout_frames.py compare bit for bit): x/3, y/3, r, g, b, 0.25
+// [, time left | cooldown / max_cooldown], from the zone centre c, the state word aux.w and -- loaded only by the task
+// that needs it -- the TimedTSP timeout word (tmax_word()) or the ColourMatch cooldown bytes (cooldown()).
+template <class TmaxWord, class Cooldown>
+__device__ __forceinline__ void zone_features(int task, const crl::DivConst& div_steps, const crl::DivConst& div_cd,
+                                              float2 c, uint32_t bits, int slot, TmaxWord tmax_word, Cooldown cooldown,
+                                              float (&z)[7]) {
   const int steps = (int)(bits & 0xffffu);
   const uint32_t hi = bits >> 16;
   const float third = 1.0f / 3.0f;
   z[0] = c.x * third; z[1] = c.y * third; z[5] = 0.25f; z[6] = 0.f;
-  if (a.task == CRL_TASK_CM) {
+  if (task == CRL_TASK_CM) {
     const uint32_t col = (hi >> (2 * slot)) & 3u;               // 0 B, 1 G, 2 R
     z[2] = col == 2u ? 1.f : 0.f; z[3] = col == 1u ? 1.f : 0.f; z[4] = col == 0u ? 1.f : 0.f;
-    const uint2 cd = __ldg(a.cooldown + e);
+    const uint2 cd = cooldown();
     const uint32_t w = slot < 4 ? cd.x : cd.y;
-    z[6] = crl::div_const((float)((w >> (8 * (slot & 3))) & 0xffu), a.div_cd);
+    z[6] = crl::div_const((float)((w >> (8 * (slot & 3))) & 0xffu), div_cd);
   } else {
     const bool v = (hi >> slot) & 1u;                          // Yellow (1,1,0) visited / Cyan (0,1,1)
     z[2] = v ? 1.f : 0.f; z[3] = 1.f; z[4] = v ? 0.f : 1.f;
-    if (a.task == CRL_TASK_TTSP) {
-      const uint32_t w = __ldg(a.zone_tmax + (size_t)(slot >> 1) * a.B + e);
+    if (task == CRL_TASK_TTSP) {
+      const uint32_t w = tmax_word();
       const int tm = (int)((w >> (16 * (slot & 1))) & 0xffffu);
-      z[6] = v ? 1.0f : crl::div_const((float)(tm - steps), a.div_steps);
+      z[6] = v ? 1.0f : crl::div_const((float)(tm - steps), div_steps);
     }
   }
 }
 
+// ... of env e, from the state planes
+__device__ __forceinline__ void zone_features_from_state(const EncArgs& a, int e, int slot, float (&z)[7]) {
+  const float2 c = __ldg(a.zone_xy + (size_t)slot * a.B + e);
+  const uint32_t bits = (uint32_t)__float_as_int(__ldg(reinterpret_cast<const float*>(a.aux + e) + 3));
+  zone_features(a.task, a.div_steps, a.div_cd, c, bits, slot,
+                [&] { return __ldg(a.zone_tmax + (size_t)(slot >> 1) * a.B + e); }, [&] { return __ldg(a.cooldown + e); }, z);
+}
+
+// ... of row e, from its CrlFrame and the layout table; a record without a layout entry (the table overflowed) gives NaN
+__device__ __forceinline__ void zone_features_from_frame(const EncArgs& a, int e, int slot, float (&z)[7]) {
+  const uint4 f = __ldg(a.frames + e);                         // bits, layout, cooldown.x, cooldown.y
+  if (f.y == CRL_FRAME_NO_LAYOUT) {
+#pragma unroll
+    for (int j = 0; j < 7; ++j) z[j] = __int_as_float(0x7fc00000);
+    return;
+  }
+  const float2 c = __ldg(a.layout_xy + (size_t)f.y * a.N + slot);
+  zone_features(a.task, a.div_steps, a.div_cd, c, f.x, slot,
+                [&] { return __ldg(a.layout_tmax + (size_t)f.y * ((a.N + 1) >> 1) + (slot >> 1)); },
+                [&] { return make_uint2(f.z, f.w); }, z);
+}
+
 // eight consecutive values (k = 8 kc .. 8 kc + 7) of row (e, slot) of the layer-1 input
 // [obs[e], zone_obs[e][slot], 1, 1, 0...]; all zeros -- the ones included -- for a padding row.
-// STATE: the zone part comes from the state planes (obs_dim == 8, so chunk 1 is exactly the zone features + ones);
-// a template parameter so that the materialised path compiles exactly as it did without the feature.
-template <bool STATE>
+// SRC (RowSrc): kSrcState / kSrcFrames build the zone part from the state planes / from a CrlFrame (obs_dim == 8, so
+// chunk 1 is exactly the zone features + ones); a template parameter so that the materialised path compiles exactly as
+// it did without them.
+template <int SRC>
 __device__ __forceinline__ void load_half_row(const EncArgs& a, int tile, int m, int kc, float (&x)[8]) {
 #pragma unroll
   for (int j = 0; j < 8; ++j) x[j] = 0.f;
@@ -267,13 +299,14 @@ __device__ __forceinline__ void load_half_row(const EncArgs& a, int tile, int m,
   const int e = (tile << (7 - sh)) + (m >> sh), slot = m & (a.S - 1);
   if (tile < a.n_tiles && e < a.B && slot < a.N) {
     const float* ob = a.obs + (size_t)e * a.obs_dim;
-    if (STATE) {
+    if (SRC != kSrcZoneObs) {
       if (kc == 0) {
 #pragma unroll
         for (int j = 0; j < 8; ++j) x[j] = __ldg(ob + j);
       } else {
         float z[7];
-        zone_features_from_state(a, e, slot, z);
+        if (SRC == kSrcState) zone_features_from_state(a, e, slot, z);
+        else zone_features_from_frame(a, e, slot, z);
 #pragma unroll
         for (int j = 0; j < 8; ++j) x[j] = j < 7 && j < a.Z ? z[j < 7 ? j : 0] : (j <= a.Z + 1 ? 1.f : 0.f);
       }
@@ -459,7 +492,7 @@ __device__ long long g_timeline[148 * 2 * 64 * 16];
 // parameter so that the plain kernels carry none of it (with a run-time test they lost 8 % to register pressure)
 // WIDE: the layer-1 input takes two K steps (obs_dim + zone_dim + 1 > 16: ZoneEnvGoalModel / ZoneEnvSkillModel); a template
 // parameter because the second prefetched chunk costs the one-step kernels eight registers they do not have (96 per thread)
-template <bool STATE, bool XHEAD, bool WIDE = false>
+template <int SRC, bool XHEAD, bool WIDE = false>
 __global__ void __launch_bounds__(kEncThreads, 1) zone_encode_kernel(const EncArgs a) {
   extern __shared__ __align__(128) uint8_t smem[];
   const Offsets o = offsets(a.h, a.obs_dim + a.Z);
@@ -647,11 +680,11 @@ __global__ void __launch_bounds__(kEncThreads, 1) zone_encode_kernel(const EncAr
       fence_async_smem();
     };
     auto fetch_x = [&](int tl) {
-      load_half_row<STATE>(a, tl, m, half, x);
-      if (WIDE) load_half_row<STATE>(a, tl, m, half + 2, x2);
+      load_half_row<SRC>(a, tl, m, half, x);
+      if (WIDE) load_half_row<SRC>(a, tl, m, half + 2, x2);
       if (dual) {
-        load_half_row<STATE>(a, tl, md, half, y);
-        if (WIDE) load_half_row<STATE>(a, tl, md, half + 2, y2);
+        load_half_row<SRC>(a, tl, md, half, y);
+        if (WIDE) load_half_row<SRC>(a, tl, md, half + 2, y2);
       }
     };
     fetch_x(tile);
@@ -1193,7 +1226,7 @@ __global__ void __launch_bounds__(kGroupThreads, 1) zone_encode_precise_kernel(c
   uint32_t parity = 0u;
   bool healthy = true, weights_in = false;
   float x[8];
-  load_half_row<false>(a, (int)blockIdx.x / n_mblocks, m, half, x);
+  load_half_row<kSrcZoneObs>(a, (int)blockIdx.x / n_mblocks, m, half, x);
   for (int tile = (int)blockIdx.x / n_mblocks; tile < a.n_tiles; tile += (int)gridDim.x / n_mblocks) {
     // ---- the tile's input rows (prefetched a tile ago), split ----
     float xh[8], xl[8];
@@ -1207,7 +1240,7 @@ __global__ void __launch_bounds__(kGroupThreads, 1) zone_encode_precise_kernel(c
     fence_async_smem();
     tc_fence_before();
     __syncthreads();
-    load_half_row<false>(a, tile + (int)gridDim.x / n_mblocks, m, half, x);   // the next tile's rows travel under this tile
+    load_half_row<kSrcZoneObs>(a, tile + (int)gridDim.x / n_mblocks, m, half, x);   // the next tile's rows travel under this tile
     // MMAs are issued by warp 0 with all its lanes CONVERGED (uniform descriptors; one elected lane executes the
     // tcgen05 instructions): from a single-thread branch every MMA costs ~300 cycles of issue (see zone_encode_kernel)
     if (warp == 0) {
@@ -1353,9 +1386,14 @@ struct BwdArgs {
   int* status;
   int B, N, Z, obs_dim, h, n_tiles, S;
 };
+// kSrcFrames: plus the frames source of the forward (frames, layout table, task, divisors); a type of its own so that the
+// kernel of materialised rows keeps its parameter block
+struct BwdFramesArgs : BwdArgs { EncArgs rows; };
 
-// eight consecutive values (k = 8 kc ..) of row m of a backward tile; zeros for padding rows and rows beyond the batch
-__device__ __forceinline__ void bwd_load_chunk(const BwdArgs& a, int tile, int m, int kc, float (&x)[8]) {
+// eight consecutive values (k = 8 kc ..) of row m of a backward tile; zeros for padding rows and rows beyond the batch.
+// SRC: where the zone part comes from, as for load_half_row (kSrcFrames: obs_dim == 8, chunk 1 = zone features + ones)
+template <int SRC, class Args>
+__device__ __forceinline__ void bwd_load_chunk(const Args& a, int tile, int m, int kc, float (&x)[8]) {
 #pragma unroll
   for (int j = 0; j < 8; ++j) x[j] = 0.f;
   const int sh = a.S == 16 ? 4 : 3;
@@ -1363,6 +1401,18 @@ __device__ __forceinline__ void bwd_load_chunk(const BwdArgs& a, int tile, int m
   const int in_dim = a.obs_dim + a.Z;
   if (tile < a.n_tiles && e < a.B && slot < a.N && 8 * kc < padded_k1(in_dim)) {
     const float* ob = a.obs + (size_t)e * a.obs_dim;
+    if constexpr (SRC == kSrcFrames) {
+      if (kc == 0) {
+#pragma unroll
+        for (int j = 0; j < 8; ++j) x[j] = __ldg(ob + j);
+      } else {
+        float z[7];
+        zone_features_from_frame(a.rows, e, slot, z);
+#pragma unroll
+        for (int j = 0; j < 8; ++j) x[j] = j < 7 && j < a.Z ? z[j < 7 ? j : 0] : (j <= a.Z + 1 ? 1.f : 0.f);
+      }
+      return;
+    }
     const float* zo = a.zone_obs + ((size_t)e * a.N + slot) * a.Z;
 #pragma unroll
     for (int j = 0; j < 8; ++j) {
@@ -1376,7 +1426,8 @@ __device__ __forceinline__ void bwd_load_chunk(const BwdArgs& a, int tile, int m
 
 __device__ __forceinline__ float bf16_bits_to_float(uint32_t b) { return __uint_as_float(b << 16); }
 
-__global__ void __launch_bounds__(kBwdThreads, 1) zone_encode_backward_kernel(const BwdArgs a) {
+template <int SRC, class Args>
+__global__ void __launch_bounds__(kBwdThreads, 1) zone_encode_backward_kernel(const Args a) {
   extern __shared__ __align__(128) uint8_t smem[];
   const int in_dim = a.obs_dim + a.Z;
   const Offsets fo = offsets(a.h, in_dim);
@@ -1443,14 +1494,14 @@ __global__ void __launch_bounds__(kBwdThreads, 1) zone_encode_backward_kernel(co
   const uint32_t x_off = (uint32_t)((m_st & 7) * 16 + (m_st >> 3) * (16 * kK1) + kc_st * 128);
   float x[8];
   int tile = (int)blockIdx.x;
-  bwd_load_chunk(a, tile, m_st, kc_st, x);
+  bwd_load_chunk<SRC>(a, tile, m_st, kc_st, x);
   for (int k = 0; tile < a.n_tiles; tile += (int)gridDim.x, ++k) {
     const uint32_t xb = o.x + (uint32_t)(k & 1) * o.x_bytes;
     if (kc_st < kK1 / 8)
       *reinterpret_cast<uint4*>(smem + xb + x_off) =
           make_uint4(pack_bf16(x[0], x[1]), pack_bf16(x[2], x[3]), pack_bf16(x[4], x[5]), pack_bf16(x[6], x[7]));
     phase_end();
-    bwd_load_chunk(a, tile + (int)gridDim.x, m_st, kc_st, x);  // the next tile's rows travel under this one
+    bwd_load_chunk<SRC>(a, tile + (int)gridDim.x, m_st, kc_st, x);  // the next tile's rows travel under this one
     const uint32_t x_addr = smem_u32(smem + xb);
     if (k == 0 && warp == 0) { healthy = mbar_wait(wbar, 0u) && healthy; __syncwarp(); }
     // ---- L1, one M-block at a time, -> H1 (bf16 relu), keyed by hidden unit (ones rows h, h + 1 included) ----
@@ -1646,24 +1697,71 @@ int crl_encoder_pack(const CrlEncoderShape* s, const float* w1, const float* b1,
   return cudaGetLastError() == cudaSuccess ? CRL_OK : CRL_ERR_LAUNCH;
 }
 
+// The frames source of crl_zone_encode_frames / crl_zone_encode_backward_frames / crl_frames_zone_obs
+struct FrameRows { const CrlFrame* frames; const float* layout_xy; const uint32_t* layout_tmax; };
+
+// the exact-division constants the step kernel uses (proven on the host once per divisor)
+static crl::DivConst enc_div_const(int d, int lo, int hi) {
+  static struct { int d, lo, hi; crl::DivConst k; } cache[8];
+  static int used = 0;
+  for (int i = 0; i < used; ++i)
+    if (cache[i].d == d && cache[i].lo == lo && cache[i].hi == hi) return cache[i].k;
+  const crl::DivConst k = crl::make_div_const(d, lo, hi);
+  if (used < 8) { cache[used].d = d; cache[used].lo = lo; cache[used].hi = hi; cache[used].k = k; ++used; }
+  return k;
+}
+
+// Rows built from frames: the env configuration (task, N, num_steps, max_cooldown; CRL_ERR_CONFIG for one no step
+// accepts), the encoder shape (obs_dim 8: CRL_ERR_UNSUPPORTED otherwise; the task's zone_dim and num_zones:
+// CRL_ERR_CONFIG otherwise) and the record / table pointers -> the frames fields of `a`.
+static int frame_row_params(const CrlEncoderShape* s, const CrlConfig* cfg, const FrameRows& fr, EncArgs& a) {
+  if (!cfg) return CRL_ERR_NULL;
+  if (cfg->task < 0 || cfg->task > 2 || cfg->num_zones <= 0 || cfg->num_zones > (cfg->task == CRL_TASK_CM ? 7 : 15) ||
+      cfg->num_steps <= 0 || cfg->num_steps > 65534 || cfg->max_cooldown < 0 || cfg->max_cooldown > 255)
+    return CRL_ERR_CONFIG;
+  if (s) {
+    if (s->obs_dim != 8) return CRL_ERR_UNSUPPORTED;
+    if (cfg->num_zones != s->num_zones || s->zone_dim != (cfg->task == CRL_TASK_TSP ? 6 : 7)) return CRL_ERR_CONFIG;
+  }
+  if (!fr.frames || !fr.layout_xy || (cfg->task == CRL_TASK_TTSP && !fr.layout_tmax)) return CRL_ERR_NULL;
+  if ((reinterpret_cast<uintptr_t>(fr.frames) & 15u) || (reinterpret_cast<uintptr_t>(fr.layout_xy) & 7u) ||
+      (reinterpret_cast<uintptr_t>(fr.layout_tmax) & 3u))
+    return CRL_ERR_ALIGN;
+  a.task = cfg->task; a.num_steps = cfg->num_steps; a.N = cfg->num_zones; a.Z = cfg->task == CRL_TASK_TSP ? 6 : 7;
+  a.div_steps = enc_div_const(cfg->num_steps, -65535, 65535);
+  a.div_cd = enc_div_const(cfg->max_cooldown > 0 ? cfg->max_cooldown : 1, 0, 255);
+  if (!a.div_steps.exact || !a.div_cd.exact) return CRL_ERR_CONFIG;
+  a.frames = reinterpret_cast<const uint4*>(fr.frames);
+  a.layout_xy = reinterpret_cast<const float2*>(fr.layout_xy);
+  a.layout_tmax = fr.layout_tmax;
+  return CRL_OK;
+}
+
 static int zone_encode_launch(const CrlEncoderShape* s, int32_t num_envs, const float* obs, const float* zone_obs,
                               const CrlConfig* cfg, const CrlState* st, const void* packed, float* pooled, int32_t* status,
-                              void* stream, void* xhead = nullptr) {
+                              void* stream, void* xhead = nullptr, const FrameRows* fr = nullptr) {
   const int rc = check_shape(s);
   if (rc) return rc;
-  if (!obs || (!zone_obs && !st) || !packed || (!pooled && !xhead)) return CRL_ERR_NULL;
+  if (!obs || (!zone_obs && !st && !fr) || !packed || (!pooled && !xhead)) return CRL_ERR_NULL;
   if (num_envs <= 0) return CRL_ERR_CONFIG;
   if (reinterpret_cast<uintptr_t>(packed) & 15u) return CRL_ERR_ALIGN;
+  if (fr) {                                                  // checked before any CUDA call
+    if (xhead) return CRL_ERR_UNSUPPORTED;
+    EncArgs probe{};
+    const int rf = frame_row_params(s, cfg, *fr, probe);
+    if (rf) return rf;
+  }
   const Offsets o = offsets(s->hidden, s->obs_dim + s->zone_dim);
   int dev = 0, sms = 148;
   if (cudaGetDevice(&dev) != cudaSuccess) return CRL_ERR_DEVICE;
   static bool attr_set[64] = {false};                       // per device: opt in to > 48 KB of dynamic shared memory
   if (dev < 0 || dev >= 64 || !attr_set[dev]) {
-    if (cudaFuncSetAttribute(zone_encode_kernel<false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024) != cudaSuccess ||
-        cudaFuncSetAttribute(zone_encode_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024) != cudaSuccess ||
-        cudaFuncSetAttribute(zone_encode_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024) != cudaSuccess ||
-        cudaFuncSetAttribute(zone_encode_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024) != cudaSuccess ||
-        cudaFuncSetAttribute(zone_encode_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024) != cudaSuccess)
+    if (cudaFuncSetAttribute(zone_encode_kernel<kSrcZoneObs, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024) != cudaSuccess ||
+        cudaFuncSetAttribute(zone_encode_kernel<kSrcZoneObs, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024) != cudaSuccess ||
+        cudaFuncSetAttribute(zone_encode_kernel<kSrcState, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024) != cudaSuccess ||
+        cudaFuncSetAttribute(zone_encode_kernel<kSrcZoneObs, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024) != cudaSuccess ||
+        cudaFuncSetAttribute(zone_encode_kernel<kSrcState, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024) != cudaSuccess ||
+        cudaFuncSetAttribute(zone_encode_kernel<kSrcFrames, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024) != cudaSuccess)
       return CRL_ERR_DEVICE;
     if (dev >= 0 && dev < 64) attr_set[dev] = true;
   }
@@ -1687,29 +1785,23 @@ static int zone_encode_launch(const CrlEncoderShape* s, int32_t num_envs, const 
     a.zone_tmax = st->zone_tmax;
     a.cooldown = reinterpret_cast<const uint2*>(st->cooldown);
     a.task = cfg->task; a.num_steps = cfg->num_steps;
-    // the same exact-division constants the step kernel uses (proven on the host once per divisor)
-    static struct { int d, lo, hi; crl::DivConst k; } cache[8];
-    static int used = 0;
-    auto div_for = [&](int d, int lo, int hi) {
-      for (int i = 0; i < used; ++i)
-        if (cache[i].d == d && cache[i].lo == lo && cache[i].hi == hi) return cache[i].k;
-      const crl::DivConst k = crl::make_div_const(d, lo, hi);
-      if (used < 8) { cache[used].d = d; cache[used].lo = lo; cache[used].hi = hi; cache[used].k = k; ++used; }
-      return k;
-    };
-    a.div_steps = div_for(cfg->num_steps, -65535, 65535);
-    a.div_cd = div_for(cfg->max_cooldown > 0 ? cfg->max_cooldown : 1, 0, 255);
+    a.div_steps = enc_div_const(cfg->num_steps, -65535, 65535);
+    a.div_cd = enc_div_const(cfg->max_cooldown > 0 ? cfg->max_cooldown : 1, 0, 255);
     if (!a.div_steps.exact || !a.div_cd.exact) return CRL_ERR_CONFIG;
+  } else if (fr) {
+    const int rf = frame_row_params(s, cfg, *fr, a);
+    if (rf) return rf;
   }
   cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
   const int want = (a.n_tiles + kGroups - 1) / kGroups;
   const int grid = want < sms ? want : sms;                   // persistent: one CTA per SM, weights loaded once
   const cudaStream_t cs = static_cast<cudaStream_t>(stream);
-  if (st && xhead) zone_encode_kernel<true, true><<<grid, kEncThreads, o.smem_end, cs>>>(a);
-  else if (st) zone_encode_kernel<true, false><<<grid, kEncThreads, o.smem_end, cs>>>(a);
-  else if (xhead) zone_encode_kernel<false, true><<<grid, kEncThreads, o.smem_end, cs>>>(a);
-  else if (padded_k1(s->obs_dim + s->zone_dim) == 32) zone_encode_kernel<false, false, true><<<grid, kEncThreads, o.smem_end, cs>>>(a);
-  else zone_encode_kernel<false, false><<<grid, kEncThreads, o.smem_end, cs>>>(a);
+  if (st && xhead) zone_encode_kernel<kSrcState, true><<<grid, kEncThreads, o.smem_end, cs>>>(a);
+  else if (st) zone_encode_kernel<kSrcState, false><<<grid, kEncThreads, o.smem_end, cs>>>(a);
+  else if (fr) zone_encode_kernel<kSrcFrames, false><<<grid, kEncThreads, o.smem_end, cs>>>(a);
+  else if (xhead) zone_encode_kernel<kSrcZoneObs, true><<<grid, kEncThreads, o.smem_end, cs>>>(a);
+  else if (padded_k1(s->obs_dim + s->zone_dim) == 32) zone_encode_kernel<kSrcZoneObs, false, true><<<grid, kEncThreads, o.smem_end, cs>>>(a);
+  else zone_encode_kernel<kSrcZoneObs, false><<<grid, kEncThreads, o.smem_end, cs>>>(a);
   return cudaGetLastError() == cudaSuccess ? CRL_OK : CRL_ERR_LAUNCH;
 }
 
@@ -1723,6 +1815,40 @@ int crl_zone_encode_state(const CrlEncoderShape* s, const CrlConfig* cfg, const 
                           const void* packed, float* pooled, int32_t* status, void* stream) {
   if (!cfg || !st) return CRL_ERR_NULL;
   return zone_encode_launch(s, cfg->num_envs, obs, nullptr, cfg, st, packed, pooled, status, stream);
+}
+
+int crl_zone_encode_frames(const CrlEncoderShape* s, const CrlConfig* cfg, int32_t num_rows, const float* obs,
+                           const CrlFrame* frames, const float* layout_xy, const uint32_t* layout_tmax, const void* packed,
+                           float* pooled, int32_t* status, void* stream) {
+  if (!cfg) return CRL_ERR_NULL;
+  const FrameRows fr{frames, layout_xy, layout_tmax};
+  return zone_encode_launch(s, num_rows, obs, nullptr, cfg, nullptr, packed, pooled, status, stream, nullptr, &fr);
+}
+
+// one thread per (row, zone): the Z features of zone_features_from_frame
+__global__ void frames_zone_obs_kernel(const EncArgs a, float* zone_obs) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= (int64_t)a.B * a.N) return;
+  const int e = (int)(i / a.N), slot = (int)(i % a.N);
+  float z[7];
+  zone_features_from_frame(a, e, slot, z);
+  float* row = zone_obs + i * a.Z;
+#pragma unroll
+  for (int j = 0; j < 7; ++j)
+    if (j < a.Z) row[j] = z[j];
+}
+
+int crl_frames_zone_obs(const CrlConfig* cfg, int32_t num_rows, const CrlFrame* frames, const float* layout_xy,
+                        const uint32_t* layout_tmax, float* zone_obs, void* stream) {
+  if (!cfg || !zone_obs) return CRL_ERR_NULL;
+  if (num_rows <= 0) return CRL_ERR_CONFIG;
+  EncArgs a{};
+  const int rc = frame_row_params(nullptr, cfg, FrameRows{frames, layout_xy, layout_tmax}, a);
+  if (rc) return rc;
+  a.B = num_rows;
+  const int64_t n = (int64_t)num_rows * a.N;
+  frames_zone_obs_kernel<<<(unsigned)((n + 255) / 256), 256, 0, static_cast<cudaStream_t>(stream)>>>(a, zone_obs);
+  return cudaGetLastError() == cudaSuccess ? CRL_OK : CRL_ERR_LAUNCH;
 }
 
 int crl_encoder_head_packed_bytes(const CrlEncoderShape* s, int64_t* bytes) {
@@ -1898,12 +2024,18 @@ int crl_encoder_backward_workspace_bytes(const CrlEncoderShape* s, int32_t num_e
   return CRL_OK;
 }
 
-int crl_zone_encode_backward(const CrlEncoderShape* s, int32_t num_envs, const float* obs, const float* zone_obs,
-                             const void* packed, const float* grad_pooled, void* workspace, float* dw1, float* db1,
-                             float* dw2, float* db2, int32_t* status, void* stream) {
+static int zone_encode_backward_launch(const CrlEncoderShape* s, int32_t num_envs, const float* obs, const float* zone_obs,
+                                       const CrlConfig* cfg, const FrameRows* fr, const void* packed,
+                                       const float* grad_pooled, void* workspace, float* dw1, float* db1, float* dw2,
+                                       float* db2, int32_t* status, void* stream) {
   const int rc = check_shape(s);
   if (rc) return rc;
-  if (!obs || !zone_obs || !packed || !grad_pooled || !workspace || !dw1 || !db1 || !dw2 || !db2) return CRL_ERR_NULL;
+  if (!obs || (!zone_obs && !fr) || !packed || !grad_pooled || !workspace || !dw1 || !db1 || !dw2 || !db2) return CRL_ERR_NULL;
+  BwdFramesArgs a{};
+  if (fr) {
+    const int rf = frame_row_params(s, cfg, *fr, a.rows);
+    if (rf) return rf;
+  }
   if (num_envs <= 0) return CRL_ERR_CONFIG;
   if ((reinterpret_cast<uintptr_t>(packed) | reinterpret_cast<uintptr_t>(workspace)) & 15u) return CRL_ERR_ALIGN;
   const BwdOffsets o = bwd_offsets(s->hidden, s->obs_dim + s->zone_dim);
@@ -1915,22 +2047,41 @@ int crl_zone_encode_backward(const CrlEncoderShape* s, int32_t num_envs, const f
   if (cudaGetDevice(&dev) != cudaSuccess) return CRL_ERR_DEVICE;
   static bool attr_set[64] = {false};
   if (dev < 0 || dev >= 64 || !attr_set[dev]) {
-    if (cudaFuncSetAttribute(zone_encode_backward_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024) != cudaSuccess)
+    if (cudaFuncSetAttribute(zone_encode_backward_kernel<kSrcZoneObs, BwdArgs>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024) != cudaSuccess ||
+        cudaFuncSetAttribute(zone_encode_backward_kernel<kSrcFrames, BwdFramesArgs>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024) != cudaSuccess)
       return CRL_ERR_DEVICE;
     if (dev >= 0 && dev < 64) attr_set[dev] = true;
   }
-  BwdArgs a{};
   a.obs = obs; a.zone_obs = zone_obs; a.g = grad_pooled; a.packed = static_cast<const uint8_t*>(packed);
   a.part = static_cast<float*>(workspace); a.status = status;
   a.B = num_envs; a.N = s->num_zones; a.Z = s->zone_dim; a.obs_dim = s->obs_dim; a.h = s->hidden;
   a.S = slots_per_env(s->num_zones); a.n_tiles = n_tiles;
   const cudaStream_t cs = static_cast<cudaStream_t>(stream);
-  zone_encode_backward_kernel<<<grid, kBwdThreads, o.smem_end, cs>>>(a);
+  if (fr) zone_encode_backward_kernel<kSrcFrames, BwdFramesArgs><<<grid, kBwdThreads, o.smem_end, cs>>>(a);
+  else zone_encode_backward_kernel<kSrcZoneObs, BwdArgs><<<grid, kBwdThreads, o.smem_end, cs>>>(static_cast<const BwdArgs&>(a));
   if (cudaGetLastError() != cudaSuccess) return CRL_ERR_LAUNCH;
   const BwdReduceArgs r{static_cast<const float*>(workspace), dw1, db1, dw2, db2, grid, s->hidden, s->obs_dim + s->zone_dim};
   const int64_t n = bwd_partial_floats(s->hidden, s->obs_dim + s->zone_dim);
   encoder_bwd_reduce_kernel<<<(int)((n + 255) / 256), 256, 0, cs>>>(r);
   return cudaGetLastError() == cudaSuccess ? CRL_OK : CRL_ERR_LAUNCH;
+}
+
+int crl_zone_encode_backward(const CrlEncoderShape* s, int32_t num_envs, const float* obs, const float* zone_obs,
+                             const void* packed, const float* grad_pooled, void* workspace, float* dw1, float* db1,
+                             float* dw2, float* db2, int32_t* status, void* stream) {
+  if (!zone_obs) return CRL_ERR_NULL;
+  return zone_encode_backward_launch(s, num_envs, obs, zone_obs, nullptr, nullptr, packed, grad_pooled, workspace, dw1, db1,
+                                     dw2, db2, status, stream);
+}
+
+int crl_zone_encode_backward_frames(const CrlEncoderShape* s, const CrlConfig* cfg, int32_t num_rows, const float* obs,
+                                    const CrlFrame* frames, const float* layout_xy, const uint32_t* layout_tmax,
+                                    const void* packed, const float* grad_pooled, void* workspace, float* dw1, float* db1,
+                                    float* dw2, float* db2, int32_t* status, void* stream) {
+  if (!cfg) return CRL_ERR_NULL;
+  const FrameRows fr{frames, layout_xy, layout_tmax};
+  return zone_encode_backward_launch(s, num_rows, obs, nullptr, cfg, &fr, packed, grad_pooled, workspace, dw1, db1, dw2,
+                                     db2, status, stream);
 }
 
 }  // extern "C"

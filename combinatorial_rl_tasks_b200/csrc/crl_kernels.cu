@@ -1628,6 +1628,54 @@ __global__ void check_state_kernel(const KParams p, int task, int N, unsigned lo
   }
 }
 
+// Rollout frames (crl_frame_capture): one thread per env writes the env's CrlFrame; the envs that start an episode (or
+// all, `initial`) take a layout-table entry -- one atomic per warp -- and copy their zone centres (and timeouts) there.
+struct CaptureParams {
+  const float4* aux;
+  const float2* zone_xy;
+  const uint32_t* zone_tmax;
+  const uint2* cooldown;
+  const unsigned long long* result;   // CrlResult[B] of the step; NULL with `initial`
+  uint4* frames;                      // CrlFrame[B] of this slot; frames - B: the previous slot
+  float2* layout_xy;
+  uint32_t* layout_tmax;
+  uint32_t* fill;                     // entries handed out, entries requested
+  uint32_t capacity;
+  int B, N, initial;
+};
+
+__global__ void __launch_bounds__(256) frame_capture_kernel(const CaptureParams c) {
+  const int e = blockIdx.x * blockDim.x + threadIdx.x, lane = threadIdx.x & 31;
+  const bool live = e < c.B;
+  const bool need = live && (c.initial || ((c.result[e] >> 32) & 0xffu) != 0ull);   // done
+  const uint32_t ballot = __ballot_sync(kFull, need);
+  uint32_t layout = CRL_FRAME_NO_LAYOUT;
+  if (ballot) {
+    const int leader = __ffs(ballot) - 1;
+    uint32_t base = 0u;
+    if (lane == leader) {
+      base = atomicAdd(c.fill + 1, (uint32_t)__popc(ballot));
+      const uint32_t end = base + (uint32_t)__popc(ballot);
+      atomicMax(c.fill, end < c.capacity ? end : c.capacity);
+    }
+    base = __shfl_sync(kFull, base, leader);
+    const uint32_t k = base + (uint32_t)__popc(ballot & ((1u << lane) - 1u));
+    if (need && k < c.capacity) layout = k;
+  }
+  if (!live) return;
+  if (!need) {
+    layout = c.frames[e - (ptrdiff_t)c.B].y;                   // the episode goes on: the entry of the previous frame
+  } else if (layout != CRL_FRAME_NO_LAYOUT) {
+    for (int i = 0; i < c.N; ++i) c.layout_xy[(size_t)layout * c.N + i] = c.zone_xy[(size_t)i * c.B + e];
+    if (c.layout_tmax) {
+      const int nh = (c.N + 1) >> 1;
+      for (int j = 0; j < nh; ++j) c.layout_tmax[(size_t)layout * nh + j] = c.zone_tmax[(size_t)j * c.B + e];
+    }
+  }
+  const uint2 cd = c.cooldown ? c.cooldown[e] : make_uint2(0u, 0u);
+  c.frames[e] = make_uint4((uint32_t)__float_as_int(c.aux[e].w), layout, cd.x, cd.y);
+}
+
 // ---- host side ---------------------------------------------------------------------
 static int zone_dim(int task) { return task == CRL_TASK_TSP ? 6 : 7; }
 
@@ -2196,6 +2244,32 @@ int crl_gae(const CrlResult* results, const float* reward_override, const float*
   gae_kernel<<<(num_envs + 127) / 128, 128, 0, static_cast<cudaStream_t>(stream)>>>(
       reinterpret_cast<const unsigned long long*>(results), reward_override, values, next_value, g, gl, num_frames,
       num_envs, advantages, returns);
+  return launch_status();
+}
+
+int crl_frame_capture(const CrlConfig* c, const CrlState* st, const CrlResult* result, int32_t initial, CrlFrame* frames_t,
+                      float* layout_xy, uint32_t* layout_tmax, uint32_t capacity, uint32_t* fill, void* stream) {
+  const int rc = check_config(c);
+  if (rc) return rc;
+  if (!st || !st->aux || !st->zone_xy || !frames_t || !layout_xy || !fill || (!initial && !result)) return CRL_ERR_NULL;
+  if (c->task == CRL_TASK_TTSP && (!st->zone_tmax || !layout_tmax)) return CRL_ERR_NULL;
+  if (c->task == CRL_TASK_CM && !st->cooldown) return CRL_ERR_NULL;
+  if (capacity == 0u) return CRL_ERR_CONFIG;
+  if (!aligned16(st->aux) || !aligned16(frames_t) || (reinterpret_cast<uintptr_t>(layout_xy) & 7u) ||
+      (reinterpret_cast<uintptr_t>(result) & 7u) || (reinterpret_cast<uintptr_t>(fill) & 3u))
+    return CRL_ERR_ALIGN;
+  CaptureParams p;
+  p.aux = reinterpret_cast<const float4*>(st->aux);
+  p.zone_xy = reinterpret_cast<const float2*>(st->zone_xy);
+  p.zone_tmax = c->task == CRL_TASK_TTSP ? st->zone_tmax : nullptr;
+  p.cooldown = c->task == CRL_TASK_CM ? reinterpret_cast<const uint2*>(st->cooldown) : nullptr;
+  p.result = reinterpret_cast<const unsigned long long*>(result);
+  p.frames = reinterpret_cast<uint4*>(frames_t);
+  p.layout_xy = reinterpret_cast<float2*>(layout_xy);
+  p.layout_tmax = c->task == CRL_TASK_TTSP ? layout_tmax : nullptr;
+  p.fill = fill; p.capacity = capacity;
+  p.B = c->num_envs; p.N = c->num_zones; p.initial = initial != 0;
+  frame_capture_kernel<<<(p.B + 255) / 256, 256, 0, static_cast<cudaStream_t>(stream)>>>(p);
   return launch_status();
 }
 

@@ -25,6 +25,10 @@ order in fp64).  The B-row rest -- ``zone_net_[4]`` and ``combine_net_`` -- is o
     model = FusedZoneEnvModel(obs_dim=8, zone_dim=6, num_zones=15, hidden=185).cuda()
     model.load_state_dict(reference_model.state_dict())     # strict: the reference's keys
     loss = f(model(obs_dict)); loss.backward(); opt.step()
+
+Both take the observations of a ``Rollout(store='frames')`` too -- ``{'obs', 'zone_frames'}``, or a minibatch gathered
+from them: the kernels then build each row from its 16-byte frame record and the rollout's layout table
+(crl_zone_encode_frames / crl_zone_encode_backward_frames), with the same results as on the materialised rows.
 """
 import ctypes
 
@@ -113,6 +117,25 @@ class ZoneEncoder:
             _lib.check(self.lib.crl_zone_encode_state(self.shape, env.cfg, env.state, env.obs.data_ptr(),
                                                       self.packed.data_ptr(), out.data_ptr(), self._status.data_ptr(),
                                                       self._stream()))
+        return out
+
+    def pooled_from_frames(self, obs, frames, out=None):
+        """``pooled`` with the zone part of the rows built from a rollout's stored frames (``ZoneFrames``, any leading
+        shape; obs of the same leading shape and 8 columns) by crl_zone_encode_frames: bit-identical to
+        ``pooled(obs, frames.zone_obs())``."""
+        assert frames.num_zones == self.num_zones and frames.zone_dim == self.zone_dim and self.obs_dim == 8
+        rec = frames.flat_records()
+        M = rec.shape[0]
+        obs = obs.reshape(M, self.obs_dim)
+        assert obs.dtype == torch.float32 and obs.is_contiguous()
+        if out is None:
+            out = torch.empty(M, self.hidden, dtype=torch.float32, device=self.device)
+        assert out.shape == (M, self.hidden) and out.dtype == torch.float32 and out.is_contiguous()
+        xy, tm = frames.ptrs()
+        with torch.cuda.device(self.device):
+            _lib.check(self.lib.crl_zone_encode_frames(self.shape, frames.cfg, M, obs.data_ptr(), rec.data_ptr(), xy, tm,
+                                                       self.packed.data_ptr(), out.data_ptr(), self._status.data_ptr(),
+                                                       self._stream()))
         return out
 
     def _workspace(self, B):
@@ -239,8 +262,12 @@ class ZoneEncoder:
         return int(self._status.item()) == 0
 
     def __call__(self, obs, zone_obs=None):
-        """ZoneEnvModel.forward: accepts the env's obs dict or the two tensors."""
+        """ZoneEnvModel.forward: accepts the env's obs dict or the two tensors.  A dict that carries ``zone_frames``
+        (Rollout(store='frames')) instead of ``zone_obs`` runs ``pooled_from_frames`` and the head kernel."""
         if zone_obs is None:
+            if 'zone_frames' in obs:
+                o = obs['obs'].reshape(-1, self.obs_dim)
+                return self._head(self.packed_head, o, self.pooled_from_frames(o, obs['zone_frames']))
             obs, zone_obs = obs['obs'], obs['zone_obs']
         return self._forward(obs, zone_obs)
 
@@ -276,19 +303,49 @@ class _FusedCore:
                                                 self._stream()))
         return out
 
-    def backward(self, obs, zone_obs, grad_pooled):
-        B, h, in_dim = obs.shape[0], self.shape.hidden, self.shape.obs_dim + self.shape.zone_dim
+    def _workspace(self, B):
         if self._ws[0] != B:
             n = ctypes.c_int64()
             with torch.cuda.device(self.device):
                 _lib.check(self.lib.crl_encoder_backward_workspace_bytes(self.shape, B, ctypes.byref(n)))
             self._ws = (B, torch.empty(n.value, dtype=torch.uint8, device=self.device))
+        return self._ws[1]
+
+    def _grads(self):
+        h, in_dim = self.shape.hidden, self.shape.obs_dim + self.shape.zone_dim
         f = lambda *s: torch.empty(*s, dtype=torch.float32, device=self.device)
-        dw1, db1, dw2, db2 = f(h, in_dim), f(h), f(h, h), f(h)
+        return f(h, in_dim), f(h), f(h, h), f(h)
+
+    def backward(self, obs, zone_obs, grad_pooled):
+        B = obs.shape[0]
+        ws = self._workspace(B)
+        dw1, db1, dw2, db2 = self._grads()
         with torch.cuda.device(self.device):
             _lib.check(self.lib.crl_zone_encode_backward(
                 self.shape, B, obs.data_ptr(), zone_obs.data_ptr(), self.packed.data_ptr(), grad_pooled.data_ptr(),
-                self._ws[1].data_ptr(), dw1.data_ptr(), db1.data_ptr(), dw2.data_ptr(), db2.data_ptr(),
+                ws.data_ptr(), dw1.data_ptr(), db1.data_ptr(), dw2.data_ptr(), db2.data_ptr(),
+                self.status.data_ptr(), self._stream()))
+        return dw1, db1, dw2, db2
+
+    # the same from stored frames (records (M, 4) int32 and the rollout's layout table)
+    def pooled_frames(self, obs, records, frames):
+        out = torch.empty(obs.shape[0], self.shape.hidden, dtype=torch.float32, device=self.device)
+        xy, tm = frames.ptrs()
+        with torch.cuda.device(self.device):
+            _lib.check(self.lib.crl_zone_encode_frames(self.shape, frames.cfg, obs.shape[0], obs.data_ptr(),
+                                                       records.data_ptr(), xy, tm, self.packed.data_ptr(), out.data_ptr(),
+                                                       self.status.data_ptr(), self._stream()))
+        return out
+
+    def backward_frames(self, obs, records, frames, grad_pooled):
+        B = obs.shape[0]
+        ws = self._workspace(B)
+        dw1, db1, dw2, db2 = self._grads()
+        xy, tm = frames.ptrs()
+        with torch.cuda.device(self.device):
+            _lib.check(self.lib.crl_zone_encode_backward_frames(
+                self.shape, frames.cfg, B, obs.data_ptr(), records.data_ptr(), xy, tm, self.packed.data_ptr(),
+                grad_pooled.data_ptr(), ws.data_ptr(), dw1.data_ptr(), db1.data_ptr(), dw2.data_ptr(), db2.data_ptr(),
                 self.status.data_ptr(), self._stream()))
         return dw1, db1, dw2, db2
 
@@ -312,6 +369,26 @@ class _FusedPooled(torch.autograd.Function):
         ctx.core.pack(w1, b1, w2, b2)                             # the image of exactly the weights the forward used
         dw1, db1, dw2, db2 = ctx.core.backward(obs, zone_obs, grad_pooled.contiguous())
         return None, None, None, dw1, db1, dw2, db2
+
+
+class _FusedPooledFrames(torch.autograd.Function):
+    """_FusedPooled with the zone rows built from stored frames (crl_zone_encode_frames / _backward_frames)."""
+
+    @staticmethod
+    def forward(ctx, core, frames, obs, records, w1, b1, w2, b2):
+        if obs.requires_grad:
+            raise RuntimeError('FusedZoneEnvModel: gradients with respect to obs are not computed; detach the inputs')
+        core.pack(w1, b1, w2, b2)
+        ctx.core, ctx.frames = core, frames
+        ctx.save_for_backward(obs, records, w1, b1, w2, b2)
+        return core.pooled_frames(obs, records, frames)
+
+    @staticmethod
+    def backward(ctx, grad_pooled):
+        obs, records, w1, b1, w2, b2 = ctx.saved_tensors
+        ctx.core.pack(w1, b1, w2, b2)
+        dw1, db1, dw2, db2 = ctx.core.backward_frames(obs, records, ctx.frames, grad_pooled.contiguous())
+        return None, None, None, None, dw1, db1, dw2, db2
 
 
 class FusedZoneEnvModel(nn.Module):
@@ -338,12 +415,28 @@ class FusedZoneEnvModel(nn.Module):
         return _FusedPooled.apply(self._core, obs.contiguous(), zone_obs.contiguous(),
                                   l1.weight.contiguous(), l1.bias.contiguous(), l2.weight.contiguous(), l2.bias.contiguous())
 
+    def pooled_from_frames(self, obs, frames):
+        """``pooled`` of rows built from stored frames (``ZoneFrames``; Rollout(store='frames')), forward and backward:
+        the same numbers as ``pooled(obs, frames.zone_obs())`` without the rows ever being materialised.  The frames stay
+        valid until the rollout's next ``begin()``: run the backward before that."""
+        assert frames.num_zones == self.num_zones and frames.zone_dim == self.zone_dim and self.obs_dim == 8
+        records = frames.flat_records()
+        obs = obs.reshape(records.shape[0], self.obs_dim)
+        assert obs.dtype == torch.float32
+        l1, l2 = self.zone_net_[0], self.zone_net_[2]
+        return _FusedPooledFrames.apply(self._core, frames, obs.contiguous(), records, l1.weight.contiguous(),
+                                        l1.bias.contiguous(), l2.weight.contiguous(), l2.bias.contiguous())
+
     def forward(self, obs):
-        if isinstance(obs, dict):
-            o, z = obs['obs'], obs['zone_obs']
+        """``obs``: a dict / DictList with ``obs`` and either ``zone_obs`` or ``zone_frames`` (Rollout(store='frames'))."""
+        get = (lambda k: obs.get(k)) if isinstance(obs, dict) else (lambda k: getattr(obs, k, None))
+        o, z, fr = get('obs'), get('zone_obs'), get('zone_frames')
+        if z is None and fr is not None:
+            o = o.reshape(-1, self.obs_dim)
+            pooled = self.pooled_from_frames(o, fr)
         else:
-            o, z = obs.obs, obs.zone_obs
-        return self.combine_net_(torch.cat([o, self.zone_net_[4](self.pooled(o, z))], dim=-1))
+            pooled = self.pooled(o, z)
+        return self.combine_net_(torch.cat([o, self.zone_net_[4](pooled)], dim=-1))
 
     def healthy(self):
         """False if a tensor-core completion wait ever expired (synchronises)."""

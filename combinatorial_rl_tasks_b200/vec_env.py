@@ -215,16 +215,20 @@ class ZoneVecEnv:
     def prepare_outputs(self, obs, zone_obs, result, shaped_reward=None):
         """Validate a set of caller-owned output tensors once and return a binding that
         ``bind_outputs(binding=...)`` installs with a few attribute stores (rollout.py prepares
-        one per slot)."""
+        one per slot).  ``zone_obs=None``: for steps that write no zone_obs (``write_zone_obs = False``); a reset or a
+        step that would write it then fails."""
         B, N, Z = self.num_envs, self.spec.num_zones, self.spec.zone_dim
-        assert obs.shape == (B, 8) and zone_obs.shape == (B, N, Z) and result.shape == (B, 8)
-        assert obs.dtype == zone_obs.dtype == torch.float32 and result.dtype == torch.uint8
-        assert obs.is_contiguous() and zone_obs.is_contiguous() and result.is_contiguous()
+        assert obs.shape == (B, 8) and result.shape == (B, 8)
+        assert obs.dtype == torch.float32 and result.dtype == torch.uint8
+        assert obs.is_contiguous() and result.is_contiguous()
+        if zone_obs is not None:
+            assert zone_obs.shape == (B, N, Z) and zone_obs.dtype == torch.float32 and zone_obs.is_contiguous()
         if shaped_reward is None:
             shaped_reward = getattr(self, 'shaped_reward', None)
             if shaped_reward is None:
                 shaped_reward = torch.zeros(B, dtype=torch.float32, device=self.device)
-        out = _lib.CrlOut(obs=obs.data_ptr(), zone_obs=zone_obs.data_ptr(), result=result.data_ptr(),
+        out = _lib.CrlOut(obs=obs.data_ptr(), zone_obs=None if zone_obs is None else zone_obs.data_ptr(),
+                          result=result.data_ptr(),
                           shaped_reward=shaped_reward.data_ptr())
         return (obs, zone_obs, result, shaped_reward, result.view(torch.float32)[:, 0], result[:, 4].view(torch.bool),
                 result[:, 5].view(torch.bool), result[:, 6].view(torch.int8), result[:, 7].view(torch.bool), out)

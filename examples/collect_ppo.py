@@ -8,6 +8,8 @@ reference's shape (per-zone MLP, mean over zones: main/src/env_model.py:48-79), 
 the update keeps the torch module, whose weights are re-packed after every optimiser step.
 --fused-train: the policy embeds through crl.FusedZoneEnvModel in collection AND update: the (B N)-row part of the
 embedding runs forward and backward on the tensor cores, the rest is torch autograd.
+--store frames: the rollout keeps a 16-byte record per env and frame plus one layout per episode instead of zone_obs
+(Rollout(store='frames')); the fused paths build the rows inside their kernels, the torch policy calls .zone_obs().
 
 The env writes each frame straight into the rollout (no per-frame copies), crl_gae computes the
 advantages; what is left for torch is the policy itself.
@@ -36,7 +38,8 @@ class ZonePolicy(nn.Module):
         self.log_std = nn.Parameter(torch.zeros(2))
 
     def forward(self, obs):
-        o, z = obs['obs'], obs['zone_obs']
+        o = obs['obs']
+        z = obs['zone_obs'] if 'zone_obs' in obs else obs['zone_frames'].zone_obs()    # Rollout(store='frames')
         x = torch.cat([o[:, None, :].expand(-1, z.shape[1], -1), z], dim=-1)
         emb = torch.relu(self.combine(torch.cat([o, self.zone_net(x).mean(dim=1)], dim=-1)))
         return self.heads(emb)
@@ -75,6 +78,7 @@ def main():
     ap.add_argument('--updates', type=int, default=3)
     ap.add_argument('--fused-encoder', action='store_true')
     ap.add_argument('--fused-train', action='store_true')
+    ap.add_argument('--store', choices=('zone_obs', 'frames'), default='zone_obs')
     args = ap.parse_args()
     if args.fused_encoder and args.fused_train:
         ap.error('--fused-encoder and --fused-train are alternatives')
@@ -84,7 +88,10 @@ def main():
     else:
         policy = ZonePolicy(env.spec.zone_dim).cuda()
     opt = torch.optim.Adam(policy.parameters(), lr=3e-4)
-    ro = Rollout(env, args.frames, discount=0.998, gae_lambda=0.95)
+    ro = Rollout(env, args.frames, discount=0.998, gae_lambda=0.95, store=args.store)
+    sb = ro.storage_bytes()
+    zone = sum(v for k, v in sb.items() if k in ('zone_obs', 'frames', 'layout_xy', 'layout_tmax'))
+    print(f'rollout storage ({args.store}): {sum(sb.values()) / 1e6:.1f} MB, of which zone state {zone / 1e6:.1f} MB')
     enc = crl.ZoneEncoder(policy.encoder_state_dict(), num_zones=env.spec.num_zones) if args.fused_encoder else None
     act = (lambda o: policy.heads(torch.relu(enc(o)))) if enc else policy
     for it in range(args.updates):

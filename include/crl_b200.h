@@ -501,6 +501,50 @@ int crl_zone_encode_backward(const CrlEncoderShape* shape, int32_t num_envs, con
                              const void* packed, const float* grad_pooled, void* workspace,
                              float* dw1, float* db1, float* dw2, float* db2, int32_t* status, void* stream);
 
+/* ---- rollout frames: the zone rows of a stored frame as a 16-byte record plus a per-episode layout ----
+ * A zone row (x/3, y/3, r, g, b, 0.25 [, time left | cooldown / max_cooldown]) depends on the zone centres (and TimedTSP
+ * timeouts), which change only at a reset, on the state word aux.w and on the ColourMatch cooldown bytes -- not on the
+ * robot.  So a rollout can store, per env and frame, one CrlFrame instead of the N Z floats of zone_obs (360 / 420 / 168
+ * bytes for PointTSP / TimedTSP / ColourMatch), and each episode's layout once, in a LAYOUT TABLE of `capacity` entries:
+ *   layout_xy   float2[capacity][N]            zone centres of entry k, row-major per entry
+ *   layout_tmax uint32[capacity][ceil(N/2)]    TimedTSP timeouts packed like CrlState.zone_tmax; NULL for the other tasks
+ *   fill        uint32[2]                      entries handed out (<= capacity), entries requested
+ * The same format serves every task.  CrlFrame.layout == CRL_FRAME_NO_LAYOUT: the capture that should have taken an entry
+ * found the table full; every row built from such a record is NaN in all its features (the rows of other records are not
+ * affected), and fill[1] > capacity tells the caller how many entries it would have needed. */
+typedef struct CrlFrame {
+  uint32_t bits;         /* aux.w verbatim: steps, visited mask / colour codes, episode parity */
+  uint32_t layout;       /* entry of the layout table, or CRL_FRAME_NO_LAYOUT */
+  uint32_t cooldown[2];  /* ColourMatch: CrlState.cooldown of the env (one byte per zone); 0 for the other tasks */
+} CrlFrame;
+#define CRL_FRAME_NO_LAYOUT 0xffffffffu
+
+/* Record frame t of every env after a step (a kernel of its own, launched behind crl_step): frames_t[e] = {aux.w, layout,
+ * cooldown}.  An env whose `result[e].done` is set -- or every env when `initial` != 0 -- takes a new table entry (one
+ * atomic per warp on fill[1]) and copies its zone_xy (and zone_tmax) into it; any other env keeps the entry of its
+ * previous record, which must lie at frames_t - num_envs (slot t - 1 of a [T + 1][B] array; not read when `initial`).
+ * The order in which entries are handed out is not deterministic; the rows built from the records are.  `result` may be
+ * NULL when `initial` != 0.  frames_t 16-byte aligned, capacity >= 1. */
+int crl_frame_capture(const CrlConfig* cfg, const CrlState* st, const CrlResult* result, int32_t initial,
+                      CrlFrame* frames_t, float* layout_xy, uint32_t* layout_tmax, uint32_t capacity, uint32_t* fill,
+                      void* stream);
+/* crl_zone_encode with the zone part of each of the M input rows built from frames[m] and the layout table (any flat or
+ * gathered set of records, with their obs rows float[M][8]): bit-identical to crl_zone_encode on the rows
+ * crl_frames_zone_obs materialises.  `cfg` is the env's (task, num_zones, num_steps, max_cooldown).  Needs obs_dim == 8
+ * (CRL_ERR_UNSUPPORTED otherwise) and the task's zone_dim and num_zones (CRL_ERR_CONFIG otherwise). */
+int crl_zone_encode_frames(const CrlEncoderShape* shape, const CrlConfig* cfg, int32_t num_rows, const float* obs,
+                           const CrlFrame* frames, const float* layout_xy, const uint32_t* layout_tmax, const void* packed,
+                           float* pooled, int32_t* status, void* stream);
+/* crl_zone_encode_backward on the same rows: same workspace (crl_encoder_backward_workspace_bytes for num_rows), same
+ * launch rule and fixed-order fp64 reduction, bit-identical to crl_zone_encode_backward on the materialised rows. */
+int crl_zone_encode_backward_frames(const CrlEncoderShape* shape, const CrlConfig* cfg, int32_t num_rows, const float* obs,
+                                    const CrlFrame* frames, const float* layout_xy, const uint32_t* layout_tmax,
+                                    const void* packed, const float* grad_pooled, void* workspace, float* dw1, float* db1,
+                                    float* dw2, float* db2, int32_t* status, void* stream);
+/* The rows themselves: zone_obs float[num_rows][N][Z], bit for bit what the step wrote for those frames. */
+int crl_frames_zone_obs(const CrlConfig* cfg, int32_t num_rows, const CrlFrame* frames, const float* layout_xy,
+                        const uint32_t* layout_tmax, float* zone_obs, void* stream);
+
 /* Copies the eight counters to the host (synchronises `stream`).  The first four (sum of
  * returns, episodes, successes, sum of lengths) are what ranks all-reduce. */
 int crl_counters_read(const CrlState* st, double out[8], void* stream);
