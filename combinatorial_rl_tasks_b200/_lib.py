@@ -13,14 +13,14 @@ c_void_p, c_int32, c_int64, c_uint32, c_uint64, c_double = (
 TASK_TSP, TASK_TTSP, TASK_CM = 0, 1, 2
 SEED_INCREMENT, SEED_FIXED_RANGE = 0, 1
 STEP_AUTO_RESET, STEP_PHYSICS_ONLY, STEP_CHAINED, STEP_CHAIN_START, STEP_TRACK_ROWS = 1, 2, 4, 8, 16
-STEP_GOALS, STEP_WAIT, STEP_ACTION_COUNTER, STEP_HOST_ZERO_COPY, STEP_NO_ZONE_OBS, STEP_HOST_PLANES = 32, 64, 128, 256, 512, 1024
+STEP_GOALS, STEP_WAIT, STEP_ACTION_COUNTER, STEP_NO_ZONE_OBS, STEP_HOST_PLANES = 32, 64, 128, 512, 1024
 STEP_ZONE_OBS_DELTA = 2048
-ABI_VERSION = 8
+ABI_VERSION = 9
 NUM_PLANES = 23
 
 # every symbol include/crl_b200.h declares
 SYMBOLS = ['crl_abi_version', 'crl_strerror', 'crl_plane_bytes', 'crl_step_bytes', 'crl_reset',
-           'crl_prefetch_layouts', 'crl_prefetch_publish', 'crl_reset_from_layout', 'crl_step', 'crl_step_host', 'crl_step_host_delta',
+           'crl_prefetch_layouts', 'crl_prefetch_publish', 'crl_reset_from_layout', 'crl_step', 'crl_step_host',
            'crl_host_call_create', 'crl_host_call_step', 'crl_host_call_destroy',
            'crl_set_goal', 'crl_goal_query', 'crl_set_qpos_qvel',
            'crl_get_qpos_qvel', 'crl_gae', 'crl_check_state', 'crl_counters_read',
@@ -89,8 +89,6 @@ def load():
                              c_void_p]
     lib.crl_step_host.argtypes = [P(CrlConfig), P(CrlState), c_void_p, c_void_p, P(CrlOut), P(CrlOut),
                                   c_uint32, c_void_p]
-    lib.crl_step_host_delta.argtypes = [P(CrlConfig), P(CrlState), c_void_p, c_void_p, P(CrlOut), P(CrlOut),
-                                        c_void_p, c_int64, c_uint32, P(c_int32), c_void_p]
     lib.crl_host_call_create.argtypes = [P(CrlConfig), P(CrlState), P(CrlOut), P(CrlOut), c_uint32, P(c_void_p)]
     lib.crl_host_call_step.argtypes = [c_void_p, c_void_p, c_void_p]
     lib.crl_host_call_destroy.argtypes = [c_void_p]

@@ -19,7 +19,7 @@
 //   7. writes state and the 8-float obs row.
 // Episode statistics go through warp ballots and one atomic per warp.  Also here: the
 // goal-conditioned / WaitWrapper variant of the step (EXT), the host-facing steps
-// (crl_step_host, crl_step_host_delta + gather_rows_kernel), goal RPC kernels and crl_gae.
+// (crl_step_host, crl_host_call_*), goal RPC kernels and crl_gae.
 #include <cuda_runtime.h>
 
 #include <atomic>
@@ -70,8 +70,8 @@ struct KParams {
   const uint32_t* epoch;        // CrlState.prefetch_epoch: last sampler round whose slots the step may trust
   uint32_t round;               // crl_prefetch_layouts: the round being run
   uint32_t* row_list;
-  float* zone_obs_host;         // CRL_STEP_HOST_ZERO_COPY: the caller's host zone_obs (device-mapped); changed rows go there
-  unsigned long long* result_dev;   // CRL_STEP_HOST_ZERO_COPY: the DEVICE copy of the result records (`result` is then the host's)
+  float* zone_obs_host;         // host-direct step: the caller's host zone_obs (device-mapped); changed rows go there
+  unsigned long long* result_dev;   // host-direct step: the DEVICE copy of the result records (`result` is then the host's)
   int32_t* goal;
   const float2* bank_zone_xy;
   const float4* bank_origin;
@@ -837,9 +837,9 @@ __device__ __forceinline__ void zone_obs_send(const KParams& p, const Env<N>& en
 }
 
 // The rows of `mask`'s lanes (the envs whose zone_obs row this step changed) from the warp's stage into `out`, each
-// row by the whole warp with coalesced stores.  A handful of rows per launch.  CRL_STEP_HOST_ZERO_COPY: `out` is the
-// caller's host mirror of zone_obs (pinned, device-mapped), which so stays a byte-exact copy of the device one with no
-// list, no gather kernel and no host-side scatter.  CRL_STEP_ZONE_OBS_DELTA: `out` is the device zone_obs itself.
+// row by the whole warp with coalesced stores.  A handful of rows per launch.  Host-direct step (crl_host_call_step):
+// `out` is the caller's host mirror of zone_obs (pinned, device-mapped), which so stays a byte-exact copy of the device
+// one.  CRL_STEP_ZONE_OBS_DELTA: `out` is the device zone_obs itself.
 // CRL_STEP_HOST_PLANES (TimedTSP, host mirror only): the host mirror is PLANE-major, float[Z][B][N] (the caller views
 // it as (B, N, Z) through strides), so that the one column that moves every step -- time left, plane 6 -- is a
 // contiguous [B][N] array: the warp writes its 32 x N values of it with fully coalesced stores, every step; a changed
@@ -931,7 +931,7 @@ __device__ __forceinline__ void store_state_obs_host(const KParams& p, const Env
                 warp_env0);
 }
 
-// CRL_STEP_HOST_ZERO_COPY: p.obs is host memory.  The warp's 32 obs rows (1 KB, contiguous) leave as ONE bulk
+// Host-direct step: p.obs is host memory.  The warp's 32 obs rows (1 KB, contiguous) leave as ONE bulk
 // copy through the zone_obs stage (long drained by now) instead of 64 half-line stores: full-size PCIe writes.
 // Takes the row by value: a reference to the caller's Env would put the whole Env into local memory.
 __device__ __noinline__ void obs_rows_bulk(float4* obs, int B, float4 row0, float4 row1, bool valid, float* stage, int lane,
@@ -1219,14 +1219,7 @@ __global__ void __maxnreg__(MaxRegs<N>::v) step_kernel(const __grid_constant__ K
       const unsigned cm = __ballot_sync(kFull, ch);
       // the rows themselves are written below: to the host mirror, or only these rows of the device zone_obs
       if (some_rows && lane == 0) s_rows_mask[warp] = cm;
-      if ((p.flags & CRL_STEP_TRACK_ROWS) && cm) {
-        uint32_t base = 0u;
-        if (lane == 0) base = atomicAdd(p.row_list, (uint32_t)__popc(cm));
-        if (!p.zone_obs_host) {
-          base = __shfl_sync(kFull, base, 0);
-          if (ch) p.row_list[4u + base + (uint32_t)__popc(cm & ((1u << lane) - 1u))] = (uint32_t)e;
-        }
-      }
+      if ((p.flags & CRL_STEP_TRACK_ROWS) && cm && lane == 0) atomicAdd(p.row_list, __popc(cm));
     }
     // (4) result word and episode statistics
     bool res_moved = false;
@@ -1318,7 +1311,7 @@ __global__ void __maxnreg__(MaxRegs<N>::v) step_kernel(const __grid_constant__ K
       env.b.phi = wrap_pi(env.b.phi);
     }
     if (p.zone_obs_host) {
-      // CRL_STEP_HOST_ZERO_COPY: p.obs is host memory; the warp's 32 obs rows leave as one bulk copy
+      // host-direct step: p.obs is host memory; the warp's 32 obs rows leave as one bulk copy
       store_state_obs_host<TASK, N>(p, env, valid, e, c, s, stage, lane, warp_env0);
     } else if (valid) {
       store_state_obs<TASK, N>(p, env, e, c, s);
@@ -1479,24 +1472,6 @@ __global__ void get_qpos_qvel_kernel(const KParams p, double* qpos, double* qvel
   qvel[3 * i] = c0 * (double)ps.w + s0 * (double)ax.x;
   qvel[3 * i + 1] = -s0 * (double)ps.w + c0 * (double)ax.x;
   qvel[3 * i + 2] = (double)ax.y;
-}
-
-// crl_step_host_delta: the rows the step listed, packed, written straight into the caller's
-// device-mapped pinned host memory.  One warp per row; `dst_rows` row i belongs to env
-// list[4 + i].  The header and the ids are mirrored to the host in front of the rows.
-__global__ void __launch_bounds__(256) gather_rows_kernel(const uint32_t* __restrict__ list, const float* __restrict__ zone_obs,
-                                                          uint32_t* host_list, float* host_rows, int row_floats, int B) {
-  const uint32_t count = min(list[0], (uint32_t)B);
-  const int lane = threadIdx.x & 31;
-  const uint32_t warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, n_warps = (gridDim.x * blockDim.x) >> 5;
-  if (warp == 0 && lane == 0) host_list[0] = count;
-  for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < count; i += gridDim.x * blockDim.x)
-    host_list[4u + i] = list[4u + i];
-  for (uint32_t i = warp; i < count; i += n_warps) {
-    const float* src = zone_obs + (size_t)list[4u + i] * row_floats;
-    float* dst = host_rows + (size_t)i * row_floats;
-    for (int k = lane; k < row_floats; k += 32) dst[k] = src[k];
-  }
 }
 
 // Goal RPCs of the goal-conditioned variants, batched (zone-goals penv.py:18-25, 75-99).
@@ -1853,7 +1828,7 @@ int crl_plane_bytes(const CrlConfig* c, int64_t* out_bytes, int32_t n) {
   o[14] = 32 * B; o[15] = 4 * N * Z * B; o[16] = 8 * B;
   o[17] = 3 * 4 * ((B + 31) / 32);
   o[18] = 16 * (1 + 2 * B);
-  o[19] = 4 * (4 + B);
+  o[19] = 16;      /* row_list */
   o[20] = 4 * B;   /* goal */
   o[21] = 4 * B;   /* shaped_reward */
   o[22] = 16;      /* prefetch_epoch */
@@ -2124,7 +2099,6 @@ int crl_host_call_create(const CrlConfig* c, const CrlState* st, const CrlOut* o
     return CRL_ERR_NULL;
   int rc = check_config(c);
   if (rc) return rc;
-  flags &= ~CRL_STEP_HOST_ZERO_COPY;
   CrlHostCall h{};
   if (!out->result) return CRL_ERR_NULL;
   h.cfg = c; h.st = st; h.direct = *out; h.flags = flags | CRL_STEP_TRACK_ROWS; h.result_dev = out->result;
@@ -2156,81 +2130,6 @@ int crl_host_call_step(CrlHostCall* h, const float* actions_host, void* stream) 
 }
 
 void crl_host_call_destroy(CrlHostCall* h) { delete h; }
-
-int crl_step_host_delta(const CrlConfig* c, const CrlState* st, const float* actions_host, float* actions_dev,
-                        const CrlOut* out, const CrlOut* host_out, void* host_delta, int64_t host_delta_bytes,
-                        uint32_t flags, int32_t* delta_rows, void* stream) {
-  if (!c || !st || !actions_host || !out || !host_out || !host_out->obs || !host_out->zone_obs ||
-      !host_out->result || !st->row_list)
-    return CRL_ERR_NULL;
-  int rc = check_config(c);
-  if (rc) return rc;
-  cudaStream_t s = static_cast<cudaStream_t>(stream);
-  const bool zero_copy = (flags & CRL_STEP_HOST_ZERO_COPY) != 0u;
-  flags &= ~CRL_STEP_HOST_ZERO_COPY;
-  if (zero_copy) {
-    // ONE kernel and a stream synchronisation.  The step kernel itself reads the actions from, and writes
-    // obs / result (/ shaped_reward) and every zone_obs row it changed to, the caller's pinned device-mapped
-    // host buffers: no copy-engine transfers, no staging, no row list, no gather, no host-side scatter
-    // (host_delta and actions_dev are not used).  row_list[0] counts the rows (cumulative).
-    auto mapped = [](const void* h) { return mapped_alias(h); };
-    CrlOut direct = *out;
-    direct.obs = static_cast<float*>(mapped(host_out->obs));
-    direct.result = static_cast<CrlResult*>(mapped(host_out->result));
-    const float* act = static_cast<const float*>(mapped(actions_host));
-    float* zhost = static_cast<float*>(mapped(host_out->zone_obs));
-    if ((flags & CRL_STEP_GOALS) && host_out->shaped_reward)
-      direct.shaped_reward = static_cast<float*>(mapped(host_out->shaped_reward));
-    if (!direct.obs || !direct.result || !act || !zhost || ((flags & CRL_STEP_GOALS) && !direct.shaped_reward)) return CRL_ERR_CONFIG;
-    if (!out->result) return CRL_ERR_NULL;
-    rc = step_launch(c, st, act, &direct, flags | CRL_STEP_TRACK_ROWS, 0, 0, zhost, stream, out->result);
-    if (rc) return rc;
-    if (cudaStreamSynchronize(s) != cudaSuccess) return CRL_ERR_DEVICE;
-    if (delta_rows) *delta_rows = -1;              // not known to the host: row_list[0] counts them on the device
-    return CRL_OK;
-  }
-  if (!host_delta || !actions_dev) return CRL_ERR_NULL;
-  const size_t B = c->num_envs, N = c->num_zones, Z = zone_dim(c->task), row = N * Z;
-  const size_t rows_off = (16 + 4 * B + 15) & ~(size_t)15;
-  if (!aligned16(host_delta) || (size_t)host_delta_bytes < rows_off + B * row * 4) return CRL_ERR_CONFIG;
-  // the gather kernel writes into host memory: it must be page-locked and device-mapped
-  cudaPointerAttributes pa;
-  if (cudaPointerGetAttributes(&pa, host_delta) != cudaSuccess || pa.type != cudaMemoryTypeHost || !pa.devicePointer) {
-    (void)cudaGetLastError();
-    return CRL_ERR_CONFIG;
-  }
-  uint32_t* host_list = static_cast<uint32_t*>(host_delta);
-  float* host_rows = reinterpret_cast<float*>(static_cast<char*>(host_delta) + rows_off);
-  uint32_t* dev_host_list = static_cast<uint32_t*>(pa.devicePointer);
-  float* dev_host_rows = reinterpret_cast<float*>(static_cast<char*>(pa.devicePointer) + rows_off);
-  {
-    if (cudaMemsetAsync(st->row_list, 0, 16, s) != cudaSuccess) return CRL_ERR_DEVICE;
-    if (cudaMemcpyAsync(actions_dev, actions_host, B * 8, cudaMemcpyHostToDevice, s) != cudaSuccess) return CRL_ERR_DEVICE;
-    rc = crl_step(c, st, actions_dev, out, flags | CRL_STEP_TRACK_ROWS, 0, 0, stream);
-    if (rc) return rc;
-    // plain launch: ordered after the whole step kernel
-    gather_rows_kernel<<<148, 256, 0, s>>>(st->row_list, out->zone_obs, dev_host_list, dev_host_rows, (int)row, (int)B);
-    rc = launch_status();
-    if (rc) return rc;
-    if (cudaMemcpyAsync(host_out->obs, out->obs, B * 32, cudaMemcpyDeviceToHost, s) != cudaSuccess) return CRL_ERR_DEVICE;
-    if (cudaMemcpyAsync(host_out->result, out->result, B * 8, cudaMemcpyDeviceToHost, s) != cudaSuccess)
-      return CRL_ERR_DEVICE;
-    if ((flags & CRL_STEP_GOALS) && host_out->shaped_reward &&
-        cudaMemcpyAsync(host_out->shaped_reward, out->shaped_reward, B * 4, cudaMemcpyDeviceToHost, s) != cudaSuccess)
-      return CRL_ERR_DEVICE;
-  }
-  if (cudaStreamSynchronize(s) != cudaSuccess) return CRL_ERR_DEVICE;
-  const uint32_t count = host_list[0];
-  if (count > B) return CRL_ERR_DEVICE;
-  float* hz = host_out->zone_obs;
-  for (uint32_t i = 0; i < count; ++i) {
-    const uint32_t e = host_list[4 + i];
-    if (e >= B) return CRL_ERR_DEVICE;
-    memcpy(hz + (size_t)e * row, host_rows + (size_t)i * row, row * 4);
-  }
-  if (delta_rows) *delta_rows = (int32_t)count;
-  return CRL_OK;
-}
 
 int crl_gae(const CrlResult* results, const float* reward_override, const float* values, const float* next_value,
             double discount, double gae_lambda, int32_t num_frames, int32_t num_envs, float* advantages,

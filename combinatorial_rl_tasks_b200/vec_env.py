@@ -135,8 +135,8 @@ class ZoneVecEnv:
         # per-warp completion stamps of crl_step (CRL_STEP_CHAINED)
         self.stamp = z(3, (B + 31) // 32, dtype=torch.int32)
         self._chain_ok = False                    # True: the last kernel enqueued for this state was a ticketed step
-        # envs whose zone_obs row changed in the last step (CRL_STEP_TRACK_ROWS, step_host)
-        self._row_list = z(4 + B, dtype=torch.int32)
+        # zone_obs rows and result records the host-direct step_host calls moved (CRL_STEP_TRACK_ROWS, cumulative)
+        self._row_list = z(4, dtype=torch.int32)
         self._mirror_ok = False                   # True: the host zone_obs buffer equals the device one
         # True: the bound zone_obs tensor holds the rows of the current state, so a step may write only the rows that
         # change (CRL_STEP_ZONE_OBS_DELTA).  Set by a full reset and by every step that writes zone_obs
@@ -509,27 +509,25 @@ class ZoneVecEnv:
         flags = (_lib.STEP_AUTO_RESET if auto_reset else 0) | (_lib.STEP_ACTION_COUNTER if replayable else 0)
         return self._step(None, flags, action_seed, chained=chained)
 
-    def step_host(self, actions, auto_reset=True, delta=True, wait=False, zero_copy=True, prepared=True):
+    def step_host(self, actions, auto_reset=True, delta=True, wait=False):
         """The reference-facing call with HOST buffers: numpy actions in, numpy obs /
         reward / done out (pinned staging; host<->device copies inside the call).  The returned
         arrays are persistent host buffers overwritten by the next call, as the device ones are --
-        READ-ONLY for the caller: on the delta paths a zone_obs row or a result record is rewritten only
+        READ-ONLY for the caller: on the delta path a zone_obs row or a result record is rewritten only
         when it changes, so an in-place edit (``reward *= scale``) would stay there; copy first.
 
-        ``delta=True``: once the host zone_obs buffer mirrors the device one, later calls move only
-        the rows that changed; the arrays returned are byte-identical to a full copy.  TimedTSP's
-        time-left column moves every step: its host mirror is plane-major (``zone_obs`` is then a
-        (B, N, Z) strided view of a [Z][B][N] buffer) and that column crosses as one contiguous plane.
-        ``zero_copy=True`` (with the delta path): ONE kernel and a stream synchronisation -- the step
-        kernel reads the actions from, and writes obs / result / shaped_reward and the changed zone_obs
-        rows to, the pinned host buffers itself; a result record (reward, done, goal_met, event, need_next_goal: all
-        zeros except on an event) crosses only when it differs from the one the host array already holds.  The DEVICE
-        tensor ``env.obs`` is then not updated by the call (``env.zone_obs`` and ``env.result`` are).  ``env.delta_rows`` =
-        rows the call moved (B = all; -1 = counted on the device only, see ``host_rows_moved()`` / ``host_results_moved()``).  ``prepared=True``: the zero-copy call goes through
-        a prepared call object (``crl_host_call_step``: three arguments per frame, buffers and flags resolved once) instead
-        of ``crl_step_host_delta`` with its eleven; same kernel, same bytes."""
+        ``delta=True``: once the host buffers mirror the device ones (after the first call), a call is ONE kernel and a
+        stream synchronisation -- the step kernel reads the actions from, and writes obs / result / shaped_reward and the
+        changed zone_obs rows to, the pinned host buffers itself, through a prepared call object (``crl_host_call_step``:
+        three arguments per frame, buffers and flags resolved once).  A result record (reward, done, goal_met, event,
+        need_next_goal: all zeros except on an event) crosses only when it differs from the one the host array already
+        holds.  The arrays returned are byte-identical to a full copy.  The DEVICE tensor ``env.obs`` is then not updated
+        by the call (``env.zone_obs`` and ``env.result`` are).  TimedTSP's time-left column moves every step: its host
+        mirror is plane-major (``zone_obs`` is then a (B, N, Z) strided view of a [Z][B][N] buffer) and that column
+        crosses as one contiguous plane.  ``env.delta_rows`` = rows the call moved (B = all; -1 = counted on the device
+        only, see ``host_rows_moved()`` / ``host_results_moved()``)."""
         h = self._host or self._host_buffers()
-        if prepared and delta and zero_copy and self._mirror_ok:
+        if delta and self._mirror_ok:
             # the prepared call (crl_host_call_*): buffers and flags resolved once, three arguments per frame
             call = self._host_calls.get((auto_reset, wait))
             if call is None:
@@ -567,28 +565,8 @@ class ZoneVecEnv:
         flags = (_lib.STEP_AUTO_RESET if auto_reset else 0) | self._mode_flags
         if wait:
             flags |= _lib.STEP_WAIT
-        ttsp = self.spec.task == _lib.TASK_TTSP
-        use_delta = delta and self._mirror_ok and (zero_copy or not ttsp)
         with self._guard():
-            if use_delta and zero_copy:
-                # TimedTSP: the host mirror is plane-major (see _host_buffers), the time-left plane crosses every step
-                zc = _lib.STEP_HOST_ZERO_COPY | (_lib.STEP_HOST_PLANES if ttsp else 0)
-                _lib.check(self.lib.crl_step_host_delta(self.cfg, self.state, aptr, None, self.out, h['out'],
-                                                        None, 0, flags | zc, None, self._stream()))
-                self.delta_rows = -1
-            elif use_delta:
-                if h['delta'] is None:
-                    B, N, Z = self.num_envs, self.spec.num_zones, self.spec.zone_dim
-                    nbytes = ((16 + 4 * B + 15) & ~15) + 4 * B * N * Z
-                    h['delta'] = torch.zeros(nbytes, dtype=torch.uint8).pin_memory()
-                n = ctypes.c_int32(0)
-                _lib.check(self.lib.crl_step_host_delta(self.cfg, self.state, aptr,
-                                                        self._actions_dev.data_ptr(), self.out, h['out'],
-                                                        h['delta'].data_ptr(), h['delta'].numel(), flags,
-                                                        ctypes.byref(n), self._stream()))
-                self.delta_rows = n.value
-                self.gpu_launches += 1                # the gather kernel
-            elif ttsp:
+            if self.spec.task == _lib.TASK_TTSP:
                 # full copy into the plane-major mirror: step on the device, then everything crosses (the device
                 # transposes zone_obs to [Z][B][N] first)
                 src = h['actions'] if aptr == h['actions_ptr'] else self._pinned[id(actions)][0]
@@ -601,12 +579,11 @@ class ZoneVecEnv:
                 if self.spec.goals:
                     h['shaped'].copy_(self.shaped_reward, non_blocking=True)
                 torch.cuda.current_stream(self.device).synchronize()
-                self.delta_rows = self.num_envs
             else:
                 _lib.check(self.lib.crl_step_host(self.cfg, self.state, aptr,
                                                   self._actions_dev.data_ptr(), self.out, h['out'],
                                                   flags, self._stream()))
-                self.delta_rows = self.num_envs
+        self.delta_rows = self.num_envs
         self._step_index += 1
         self.gpu_launches += 1
         self._chain_ok = False                    # memcpys follow the step kernel on the stream
@@ -641,7 +618,7 @@ class ZoneVecEnv:
             pass
 
     def host_rows_moved(self, reset=False):
-        """zone_obs rows the zero-copy step_host calls have written to the host mirror since the count was last
+        """zone_obs rows the host-direct step_host calls have written to the host mirror since the count was last
         reset (the kernel counts them in CrlState.row_list[0])."""
         n = int(self._row_list[0].item())
         if reset:
@@ -649,7 +626,7 @@ class ZoneVecEnv:
         return n
 
     def host_results_moved(self, reset=False):
-        """Result records the zero-copy step_host calls have written to the host array since the count was last reset
+        """Result records the host-direct step_host calls have written to the host array since the count was last reset
         (CrlState.row_list[1]); the others were equal to what the host already held."""
         n = int(self._row_list[1].item())
         if reset:
@@ -671,7 +648,6 @@ class ZoneVecEnv:
             h['np'] = {k: h[k].numpy() for k in ('actions', 'obs', 'zone_obs', 'result', 'shaped')}
             if self.spec.task == _lib.TASK_TTSP:
                 h['np']['zone_obs'] = h['np']['zone_obs'].transpose(1, 2, 0)
-            h['delta'] = None
             h['actions_ptr'] = h['actions'].data_ptr()
             # what every step_host call returns: views of the persistent host buffers, built once
             res = h['np']['result']

@@ -53,8 +53,8 @@
  *    sampler round r)
  *  optional stamp uint32[2][ceil(B/32)]: steps started / finished per group of 32 envs,
  *  see CRL_STEP_CHAINED
- *  optional row_list uint32[4 + B] (CRL_STEP_TRACK_ROWS, crl_step_host_delta; header word 0 = zone_obs rows listed or
- *  moved, word 1 = result records moved by the host-direct step, words 2-3 unused, then the env ids) and goal int32[B]
+ *  optional row_list uint32[4] (CRL_STEP_TRACK_ROWS, crl_host_call_*; word 0 = zone_obs rows moved or counted,
+ *  word 1 = result records moved by the host-direct step, words 2-3 unused) and goal int32[B]
  *  (goal-conditioned variants, CRL_STEP_GOALS): see CrlState
  *  outputs, the layout the reference's consumer builds (main/src/utils/format.py:27-28):
  *    obs       float[B][8]      remaining, pos/3 (2), dir (2), vel/1.5 (2), yaw rate/3
@@ -71,7 +71,7 @@
 extern "C" {
 #endif
 
-#define CRL_ABI_VERSION 8
+#define CRL_ABI_VERSION 9
 #define CRL_MAX_ZONES 16
 
 /* task ids; reference classes: main/envs/TSP_env.py:11, TTSP_env.py:12, colour_match_env.py:11 */
@@ -103,10 +103,11 @@ enum CrlError {
  * flag never touch the stamps. */
 #define CRL_STEP_CHAINED 4u
 #define CRL_STEP_CHAIN_START 8u
-/* Needs CrlState.row_list.  The step appends to it the index of every env whose zone_obs row
+/* Needs CrlState.row_list.  The step adds to row_list[0] the number of envs whose zone_obs row
  * differs from the row the previous step left there (a zone fired, the env was reset, a
  * ColourMatch cooldown ticked; every TimedTSP env, whose time-left column moves each step).
- * Used by crl_step_host_delta; the caller zeroes the list header before the step. */
+ * The count is cumulative: the caller zeroes it when it wants a new one.  Implied by the
+ * host-direct step (crl_host_call_*). */
 #define CRL_STEP_TRACK_ROWS 16u
 /* Goal-conditioned variants PointTSP-v3 / PointTTSP-v3 / ColourMatch-v3
  * (zone-goals/envs/TSP_next_city_env.py:52-75, TTSP_next_city_env.py:45-56,
@@ -125,35 +126,24 @@ enum CrlError {
  * iid U(-1,1)^2 actions per (env, step) at every replay -- action_space.sample() of a random-action
  * rollout -- with nothing coming from the host.  Needs CrlState.stamp. */
 #define CRL_STEP_ACTION_COUNTER 128u
-/* crl_step_host_delta only: ONE kernel and a stream synchronisation per call.  No staging, no
- * copy-engine transfers, no row list, no gather kernel, no host-side scatter -- the step kernel reads
- * the actions from, and writes obs / result / shaped_reward AND every zone_obs row it changed straight
- * to, the caller's host buffers (actions_host and all of host_out), which must be page-locked and
- * device-mapped (cudaHostAlloc; CRL_ERR_CONFIG otherwise).  host_delta and actions_dev are not used
- * (may be NULL); *delta_rows is set to -1 and CrlState.row_list[0] counts the rows moved, cumulatively.
- * Result records are treated like zone_obs rows: a record (all zeros except on an event, a done or a goal change) is
- * written to host_out->result only when it differs from the one there, which the kernel knows from the device copy
- * out->result (updated by every step) -- PRECONDITION: host_out->result holds out->result as of the previous step, as
- * crl_step_host leaves it.  CrlState.row_list[1] counts the records moved.
- * The device copies CrlOut.obs / shaped_reward are NOT updated by such a call (zone_obs and result are). */
-#define CRL_STEP_HOST_ZERO_COPY 256u
 /* The step does not build or write zone_obs (CrlOut.zone_obs may be NULL): for a consumer that derives the zone
  * rows from the state planes itself -- crl_zone_encode_state, the fused ZoneEnvModel encoder -- a rollout that only
  * needs the embedding never materialises 360 / 420 / 168 of the 584 / 676 / 336 bytes an env-step moves.  Not with
- * CRL_STEP_TRACK_ROWS / CRL_STEP_HOST_ZERO_COPY (they ship zone_obs rows). */
+ * CRL_STEP_TRACK_ROWS or the host-direct step, crl_host_call_* (they ship zone_obs rows). */
 #define CRL_STEP_NO_ZONE_OBS 512u
-/* With CRL_STEP_HOST_ZERO_COPY, TimedTSP only: host_out->zone_obs is PLANE-major, float[Z][B][N] (the caller views it
- * as (B, N, Z) through strides).  TimedTSP's time-left column moves every step, so with a row-major mirror every row
- * would cross PCIe every step (420 B per env); plane-major, that column is one contiguous [B][N] plane the step
- * writes with coalesced stores (60 B per env), and only the rows of visits and resets touch the other six planes. */
+/* Host-direct step (crl_host_call_*), TimedTSP only: host_out->zone_obs is PLANE-major, float[Z][B][N] (the caller
+ * views it as (B, N, Z) through strides).  TimedTSP's time-left column moves every step, so with a row-major mirror
+ * every row would cross PCIe every step (420 B per env); plane-major, that column is one contiguous [B][N] plane the
+ * step writes with coalesced stores (60 B per env), and only the rows of visits and resets touch the other six planes. */
 #define CRL_STEP_HOST_PLANES 1024u
-/* The step writes only the zone_obs rows whose bytes change -- the rows CRL_STEP_TRACK_ROWS lists: a zone fired, the env
+/* The step writes only the zone_obs rows whose bytes change -- the rows CRL_STEP_TRACK_ROWS counts: a zone fired, the env
  * was rebuilt by the auto-reset, a ColourMatch cooldown ticked, every TimedTSP row -- and leaves every other row of
  * CrlOut.zone_obs untouched.  PRECONDITION: out->zone_obs holds the rows of the state the step starts from, as a crl_reset
  * of all envs or a step that wrote zone_obs left them.  PointTSP then moves 224 instead of 584 bytes per env-step, plus a
- * row for each zone event and reset.  TimedTSP ignores the flag (its time-left column moves every step).  Not with CRL_STEP_NO_ZONE_OBS, the host-direct steps (crl_step_host_delta with
- * CRL_STEP_HOST_ZERO_COPY, crl_host_call_step) or the goal-conditioned / WaitWrapper / walled kernels (CRL_STEP_GOALS,
- * CRL_STEP_WAIT, CrlConfig.walled): CRL_ERR_CONFIG.  A library that ignores the bit writes every row: the same bytes. */
+ * row for each zone event and reset.  TimedTSP ignores the flag (its time-left column moves every step).  Not with
+ * CRL_STEP_NO_ZONE_OBS, the host-direct step (crl_host_call_step) or the goal-conditioned / WaitWrapper / walled kernels
+ * (CRL_STEP_GOALS, CRL_STEP_WAIT, CrlConfig.walled): CRL_ERR_CONFIG.  A library that ignores the bit writes every row:
+ * the same bytes. */
 #define CRL_STEP_ZONE_OBS_DELTA 2048u
 
 /* how a reset chooses the episode's seed; wrappers.py:10-23 and Engine.seed/reset */
@@ -212,8 +202,9 @@ typedef struct CrlState {
                            in-kernel-action steps taken (CRL_STEP_ACTION_COUNTER) */
   uint32_t* prefetch_work; /* 16 (1 + 2 B) bytes, 16-byte aligned: work list of crl_prefetch_layouts
                               (needed with next_*) */
-  uint32_t* row_list;   /* uint32[4 + B]; optional (CRL_STEP_TRACK_ROWS): word 0 = number of envs
-                           whose zone_obs row changed in the step, words 4.. = their indices */
+  uint32_t* row_list;   /* uint32[4]; optional (CRL_STEP_TRACK_ROWS, crl_host_call_*): word 0 = number
+                           of envs whose zone_obs row changed (or, host-direct, moved), word 1 = result
+                           records the host-direct step moved, both cumulative; words 2-3 unused */
   int32_t* goal;        /* int32[B]; optional (CRL_STEP_GOALS): goal_zone of each env, -1 = None.
                            Every reset clears it */
   /* optional LAYOUT BANK (all three NULL = none): the maps of the K = max_seed - min_seed + 1
@@ -330,33 +321,29 @@ int crl_step_host(const CrlConfig* cfg, const CrlState* st, const float* actions
                   float* actions_dev, const CrlOut* out, const CrlOut* host_out,
                   uint32_t flags, void* stream);
 
-/* crl_step_host for a caller that keeps its host observation buffers between calls (as
- * ParallelEnv's consumers do: the obs of step t is only read before step t+1).  zone_obs is
- * 60-90 % of a step's output bytes and almost all of it repeats the previous step (zone
- * centres never move inside an episode; a colour changes only when a zone fires), so only the
- * rows that CHANGED cross PCIe: the step lists them (CRL_STEP_TRACK_ROWS), a gather kernel
- * writes {count, env ids, rows} straight into the caller's pinned host memory
- * (`host_delta`, device-mapped: uint32[4 + B] header and ids, then at byte offset
- * 16 + 4 B rounded up to 16 the rows, float[B][N][Z] worst case), the stream is
- * synchronised and the rows are scattered into `host_out->zone_obs` on the host.  obs and
- * result are copied whole.  PRECONDITION: host_out->zone_obs holds the device zone_obs as of
- * the previous step (e.g. left there by crl_step_host or by a full copy after crl_reset).
- * The result is byte-identical to crl_step_host's.  `delta_rows`, if not NULL, receives the
- * number of rows that crossed.  host_delta must be page-locked (cudaHostAlloc / pinned). */
-int crl_step_host_delta(const CrlConfig* cfg, const CrlState* st, const float* actions_host,
-                        float* actions_dev, const CrlOut* out, const CrlOut* host_out,
-                        void* host_delta, int64_t host_delta_bytes, uint32_t flags,
-                        int32_t* delta_rows, void* stream);
-
-/* The CRL_STEP_HOST_ZERO_COPY call, PREPARED: what ParallelEnv.step (penv.py:52-59) does once per frame with the same
- * envs and the same buffers is resolved once -- the device aliases of the caller's page-locked host buffers, the flags --
- * so that a per-frame call carries three arguments instead of eleven (a ctypes / cgo / JNI binding pays per argument:
- * 3.5 us against 0.9 us through ctypes).  crl_host_call_create: `cfg` and `st` are kept BY POINTER (the caller keeps them
- * alive and may change their fields between steps, as with crl_step_host_delta); `out` and `host_out` are read now; `flags`
- * as for crl_step_host_delta (CRL_STEP_HOST_ZERO_COPY implied).  crl_host_call_step: one step; `actions_host` float[B][2],
- * page-locked and device-mapped (CRL_ERR_CONFIG otherwise); result byte-identical to crl_step_host_delta's; the stream is
- * synchronised before it returns.  Same precondition on host_out->zone_obs.  A call object is used by one thread at a time;
- * the host buffers it was created with (and the action buffers it has seen) stay allocated and page-locked while it lives. */
+/* The HOST-DIRECT step: crl_step_host for a caller that keeps its host observation buffers between calls (as
+ * ParallelEnv's consumers do: the obs of step t is only read before step t+1), in ONE kernel and a stream synchronisation
+ * per call.  No staging and no copy-engine transfers: the step kernel reads the actions from, and writes obs / result /
+ * shaped_reward AND every zone_obs row it changed straight to, the caller's host buffers (actions_host and all of
+ * host_out), which must be page-locked and device-mapped (cudaHostAlloc; CRL_ERR_CONFIG otherwise).  zone_obs is 60-90 %
+ * of a step's output bytes and almost all of it repeats the previous step (zone centres never move inside an episode; a
+ * colour changes only when a zone fires), so only the rows that CHANGED cross PCIe.  PRECONDITION: host_out->zone_obs
+ * holds the device zone_obs as of the previous step (e.g. left there by crl_step_host or by a full copy after crl_reset).
+ * Result records are treated like zone_obs rows: a record (all zeros except on an event, a done or a goal change) is
+ * written to host_out->result only when it differs from the one there, which the kernel knows from the device copy
+ * out->result (updated by every step) -- PRECONDITION: host_out->result holds out->result as of the previous step, as
+ * crl_step_host leaves it.  What the caller sees is byte-identical to crl_step_host's.  Needs CrlState.row_list:
+ * row_list[0] counts the zone_obs rows moved and row_list[1] the result records moved, cumulatively.  The device copies
+ * CrlOut.obs / shaped_reward are NOT updated by such a call (zone_obs and result are).
+ * The call is PREPARED: what ParallelEnv.step (penv.py:52-59) does once per frame with the same envs and the same buffers
+ * is resolved once -- the device aliases of the caller's page-locked host buffers, the flags -- so that a per-frame call
+ * carries three arguments (a ctypes / cgo / JNI binding pays per argument: 3.5 us for eleven against 0.9 us for three
+ * through ctypes).  crl_host_call_create: `cfg` and `st` are kept BY POINTER (the caller keeps them alive and may change
+ * their fields between steps); `out` and `host_out` are read now; `flags` as for crl_step (CRL_STEP_TRACK_ROWS implied;
+ * CRL_STEP_HOST_PLANES for a plane-major TimedTSP mirror).  crl_host_call_step: one step; `actions_host` float[B][2],
+ * page-locked and device-mapped (CRL_ERR_CONFIG otherwise); the stream is synchronised before it returns.  A call object
+ * is used by one thread at a time; the host buffers it was created with (and the action buffers it has seen) stay
+ * allocated and page-locked while it lives. */
 typedef struct CrlHostCall CrlHostCall;
 int crl_host_call_create(const CrlConfig* cfg, const CrlState* st, const CrlOut* out, const CrlOut* host_out,
                          uint32_t flags, CrlHostCall** call);

@@ -83,7 +83,7 @@ def check_obs(task, obs_gpu, zobs_gpu, obs_ref, zobs_ref, where):
 def test_library_is_the_cuda_one(crl):
     from combinatorial_rl_tasks_b200 import _lib
     lib = _lib.load()
-    assert lib.crl_abi_version() == _lib.ABI_VERSION == 8
+    assert lib.crl_abi_version() == _lib.ABI_VERSION == 9
     with open('/proc/self/maps') as f:
         assert 'libcrl_b200.so' in f.read()
 

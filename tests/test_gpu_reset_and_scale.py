@@ -212,21 +212,21 @@ def test_step_host_no_reset_wait_equals_device_step_no_reset(crl):
     assert not env_a._host_calls
 
 
-@pytest.mark.parametrize('zero_copy', [True, 'unprepared', False], ids=['zero_copy', 'zero_copy_unprepared', 'staged'])
+@pytest.mark.parametrize('actions', ['numpy', 'host_actions', 'pinned_actions'])
 @pytest.mark.parametrize('env_id', TASKS + ['PointTTSP-v3', 'ColourMatch-v3'])     # -v3: the EXT kernels (shaped_reward too)
-def test_step_host_delta_is_byte_identical_to_full_copy(crl, env_id, zero_copy):
-    """crl_step_host_delta moves only the zone_obs rows that changed; what the caller sees in its
-    host buffers must be byte for byte what crl_step_host (full copy) delivers -- across zone
-    events, cooldown ticks, timeouts and auto-resets (episodes cut short to force many).  Both flavours:
-    zero-copy (one kernel; the step writes obs / result / changed rows into the pinned host buffers itself)
-    and staged (row list + gather kernel + copy-engine transfers); zero-copy through the prepared call object
-    (crl_host_call_step, the default) and through crl_step_host_delta itself."""
-    prepared, zero_copy = zero_copy is True, bool(zero_copy)
+def test_step_host_delta_is_byte_identical_to_full_copy(crl, env_id, actions):
+    """The host-direct step (crl_host_call_step: one kernel; the step writes obs / result / changed rows into the pinned
+    host buffers itself) moves only the zone_obs rows and result records that changed; what the caller sees in its
+    host buffers must be byte for byte what crl_step_host (full copy) delivers -- across zone events, cooldown ticks,
+    timeouts and auto-resets (episodes cut short to force many).  The actions come from an ordinary numpy array (copied
+    into the env's pinned buffer), from that buffer filled in place (host_actions()) or from a rotation of
+    pinned_actions() arrays that the kernel reads where they lie."""
     B = 1000
     envs = []
     for _ in range(2):
         e = crl.ZoneVecEnv(env_id, B); e.seed(11); e.cfg.num_steps = 40; e.reset(); envs.append(e)
     full, delta = envs
+    pinned = delta.pinned_actions(4)
     rs = np.random.RandomState(5)
     moved = []
     for t in range(130):
@@ -239,7 +239,10 @@ def test_step_host_delta_is_byte_identical_to_full_copy(crl, env_id, zero_copy):
             for e in envs:
                 e.pose[:200, :2] = e.zone_xy[3, :200, :]
         of, rf, df, inf_ = full.step_host(a, delta=False)
-        od, rd, dd, ind = delta.step_host(a, delta=True, zero_copy=zero_copy, prepared=prepared)
+        ad = {'numpy': a, 'host_actions': delta.host_actions(), 'pinned_actions': pinned[t % 4]}[actions]
+        if ad is not a:
+            ad[:] = a
+        od, rd, dd, ind = delta.step_host(ad, delta=True)
         rows = delta.delta_rows if delta.delta_rows >= 0 else delta.host_rows_moved(reset=True)   # -1: counted on the device
         if t == 20:
             assert rows >= 200 and (env_id.startswith('ColourMatch') or int((ind['event'] != 0).sum()) >= 200)
@@ -252,17 +255,14 @@ def test_step_host_delta_is_byte_identical_to_full_copy(crl, env_id, zero_copy):
         assert np.array_equal(od['zone_obs'], delta.zone_obs.cpu().numpy()), t
         moved.append(rows)
     assert moved[0] == B and moved[70] == B           # first call and the call after device-side work: full copy
-    if zero_copy:
-        # result records cross only when they differ from what the host holds: far fewer than one per env and step
-        # (equality with the full copy was checked at every step above)
-        assert 0 < delta.host_results_moved() < 128 * B // 3
-    if env_id.startswith('PointTTSP') and not zero_copy:
-        assert all(m == B for m in moved)             # the time-left column moves every step: staged = full copies
-    else:                                             # (zero-copy TimedTSP: plane-major mirror, that column is its own plane)
-        # between the step-limit resets only a few rows move (TimedTSP: its 40-step episodes also end on timeouts)
-        assert max(moved[1:39]) < (B // 2 if env_id.startswith('PointTTSP') else B // 4)
-        if not env_id.startswith('PointTTSP'):                  # (TimedTSP's episodes are desynchronised by their timeouts long before)
-            assert B in moved[39:42] or max(moved[38:42]) >= B // 2   # the step-limit reset rewrites every row
+    # result records cross only when they differ from what the host holds: far fewer than one per env and step
+    # (equality with the full copy was checked at every step above)
+    assert 0 < delta.host_results_moved() < 128 * B // 3
+    # between the step-limit resets only a few rows move (TimedTSP: its 40-step episodes also end on timeouts; its
+    # time-left column is a plane of its own in the plane-major mirror and is not counted as a row)
+    assert max(moved[1:39]) < (B // 2 if env_id.startswith('PointTTSP') else B // 4)
+    if not env_id.startswith('PointTTSP'):                  # (TimedTSP's episodes are desynchronised by their timeouts long before)
+        assert B in moved[39:42] or max(moved[38:42]) >= B // 2   # the step-limit reset rewrites every row
 
 
 @pytest.mark.parametrize('env_id,B', [('PointTSP-v0', 65536), ('PointTTSP-v0', 262144), ('ColourMatch-v0', 262144)])

@@ -48,7 +48,8 @@ def test_library_exports_every_declared_symbol():
     lib = _lib.load()
     for name in declared:
         assert getattr(lib, name) is not None
-    assert lib.crl_abi_version() == 8
+    assert lib.crl_abi_version() == 9
+    assert not hasattr(lib, 'crl_step_host_delta')
     assert b'NULL' in lib.crl_strerror(-1)
 
 
@@ -60,7 +61,7 @@ def test_argument_errors_are_detected_on_the_host():
     sizes = (ctypes.c_int64 * 23)()
     assert lib.crl_plane_bytes(cfg, sizes, 23) == 0
     assert list(sizes) == [1024, 1024, 7680, 0, 0, 512, 256, 1024, 64, 2 * 7680, 0, 2 * 1024, 2 * 512, 2 * 256,
-                           2048, 64 * 90 * 4, 512, 24, 16 * 129, 4 * 68, 256, 256, 16]
+                           2048, 64 * 90 * 4, 512, 24, 16 * 129, 16, 256, 256, 16]
     rd, wr = ctypes.c_int64(), ctypes.c_int64()
     assert lib.crl_step_bytes(cfg, ctypes.byref(rd), ctypes.byref(wr)) == 0 and (rd.value, wr.value) == (160, 432)
     bad = _lib.CrlConfig(task=7, num_envs=64, num_zones=15, num_steps=2000, zone_size=0.2)
@@ -76,7 +77,6 @@ def test_argument_errors_are_detected_on_the_host():
     assert lib.crl_step(cfg2, st, None, out, 0, 0, 0, None) == -4         # no kernel for N = 9
     assert lib.crl_step(cfg, st, None, out, _lib.STEP_CHAINED, 0, 0, None) == -1   # chained needs CrlState.stamp
     assert lib.crl_step(cfg, st, None, out, _lib.STEP_TRACK_ROWS, 0, 0, None) == -1  # needs CrlState.row_list
-    assert lib.crl_step_host_delta(cfg, st, a16, a16, out, out, a16, 4096, 0, None, None) == -1  # no row_list
     call = ctypes.c_void_p()
     assert lib.crl_host_call_create(cfg, st, out, out, 0, ctypes.byref(call)) == -1   # no row_list
     assert lib.crl_host_call_step(None, a16, None) == -1 and not call.value

@@ -14,8 +14,6 @@ def t(f, n=200):
     for _ in range(n): f()
     torch.cuda.synchronize(); return (time.perf_counter() - t0) / n * 1e6
 h = env._host_buffers()
-print('step_host(delta, staged) total %.1f us' % t(lambda: env.step_host(a, zero_copy=False)))
-print('step_host(delta, staged), pinned in %.1f us' % t(lambda: env.step_host(h['np']['actions'], zero_copy=False)))
 print('step_host(full)             %.1f us' % t(lambda: env.step_host(a, delta=False), 50))
 env.step_host(a)
 print('np.copyto actions           %.1f us' % t(lambda: np.copyto(h['np']['actions'], a)))
@@ -32,19 +30,16 @@ def kern(): env.step(env._actions_dev); s.synchronize()
 print('device step + sync          %.1f us' % t(kern))
 print('empty sync                  %.1f us' % t(lambda: s.synchronize()))
 env.step_host(a)
-print('step_host(delta, zero-copy)           %.1f us' % t(lambda: env.step_host(a, zero_copy=True)))
-print('step_host(delta, zero-copy, pinned in)%.1f us' % t(lambda: env.step_host(h['np']['actions'], zero_copy=True)))
-print('  ... unprepared (crl_step_host_delta)%.1f us' % t(lambda: env.step_host(h['np']['actions'], zero_copy=True, prepared=False)))
+print('step_host(delta, zero-copy)           %.1f us' % t(lambda: env.step_host(a)))
+print('step_host(delta, zero-copy, pinned in)%.1f us' % t(lambda: env.step_host(h['np']['actions'])))
 pa = env.pinned_actions(1)[0]; np.copyto(pa, a)
-print('  ... prepared, pinned_actions() array %.1f us' % t(lambda: env.step_host(pa)))
-print('  ... unprepared, same array           %.1f us' % t(lambda: env.step_host(pa, prepared=False)))
-print('  ... prepared again                   %.1f us' % t(lambda: env.step_host(pa)))
+print('  ... pinned_actions() array           %.1f us' % t(lambda: env.step_host(pa)))
 ref = crl.ZoneVecEnv('PointTSP-v0', B); ref.seed(1); ref.reset()
 env2 = crl.ZoneVecEnv('PointTSP-v0', B); env2.seed(1); env2.reset()
 rs = np.random.RandomState(3)
 for k in range(60):
     aa = rs.uniform(-1, 1, (B, 2)).astype(np.float32)
     o1, r1, d1, i1 = ref.step_host(aa, delta=False)
-    o2, r2, d2, i2 = env2.step_host(aa, zero_copy=True)
+    o2, r2, d2, i2 = env2.step_host(aa)
     assert np.array_equal(o1['obs'], o2['obs']) and np.array_equal(o1['zone_obs'], o2['zone_obs']) and np.array_equal(r1, r2) and np.array_equal(d1, d2), k
 print('zero-copy host buffers identical to full copy over 60 steps')

@@ -1,7 +1,7 @@
 """Diagnostic (not a bench line): how does a step_host call scale when k of the N ranks of one box run it at once?
 torchrun --nproc-per-node N tools/probe_e2e_multi.py   -> one JSON line per (mode, active ranks) from rank 0.
-Modes: zero_copy (one kernel, posted writes to pinned memory), staged (delta path through the copy engine), d2h (the
-copy engine alone moving the same 2.6 MB), d2h_big (26 MB per call)."""
+Modes: zero_copy (one kernel, posted writes to pinned memory), d2h (the copy engine alone moving the same 2.6 MB),
+d2h_big (26 MB per call)."""
 import os, sys, time, json
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch, torch.distributed as dist
@@ -25,9 +25,7 @@ big_dst = torch.empty(26 * 1024 * 1024, dtype=torch.uint8).pin_memory()
 s = torch.cuda.current_stream()
 n_call = [0]
 def zero_copy():
-    env.step_host(acts[n_call[0] % 4], zero_copy=True); n_call[0] += 1
-def staged():
-    env.step_host(acts[n_call[0] % 4], zero_copy=False); n_call[0] += 1
+    env.step_host(acts[n_call[0] % 4]); n_call[0] += 1
 def d2h():
     h['obs'].copy_(env.obs, non_blocking=True); h['result'].copy_(env.result, non_blocking=True); s.synchronize()
 def d2h_big():
@@ -65,7 +63,7 @@ sets = {'all': list(range(world)), 'rank0': [0]}
 if world >= 2: sets['0,1'] = [0, 1]
 if world >= 4: sets['0,2'] = [0, 2]; sets['0-3'] = [0, 1, 2, 3]; sets['even'] = list(range(0, world, 2))
 if world >= 8: sets['0,4'] = [0, 4]; sets['0,1,4,5'] = [0, 1, 4, 5]
-for mode, fn in (('zero_copy', zero_copy), ('staged', staged), ('d2h', d2h), ('d2h_big', d2h_big), ('dev_step', dev_step)):
+for mode, fn in (('zero_copy', zero_copy), ('d2h', d2h), ('d2h_big', d2h_big), ('dev_step', dev_step)):
     for name, ranks in sets.items():
         if mode in ('d2h_big', 'dev_step') and name not in ('all', 'rank0', '0,1', '0,4'):
             continue

@@ -27,7 +27,7 @@ def count(env_id, B, steps):
     env._row_list[:4].zero_()
     for _ in range(steps):
         _lib.check(env.lib.crl_step(env.cfg, env.state, None, env.out, flags, 1234, 0, env._stream()))
-        rows += env._row_list[0]                     # the header counts this step's rows; the list holds B at most
+        rows += env._row_list[0]                     # word 0 counts this step's rows
         env._row_list[:1].zero_()
         env.tick()
     per = int(rows.item()) / (steps * B)

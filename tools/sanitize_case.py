@@ -34,7 +34,6 @@ for env_id in ('PointTSP-v0', 'PointTTSP-v0', 'ColourMatch-v0', 'PointTSP-v1'):
         env.step_random(action_seed=9, chained=True)
     env.step_host(np.zeros((B, 2), np.float32))                       # full copy: the host mirror becomes valid
     env.step_host(np.zeros((B, 2), np.float32))                       # delta rows + zero-copy obs / result
-    env.step_host(np.zeros((B, 2), np.float32), zero_copy=False)      # delta rows, staged copies
     torch.cuda.synchronize()
     print(env_id, 'ok', env.counters())
 
