@@ -29,7 +29,8 @@ SYMBOLS = ['crl_abi_version', 'crl_strerror', 'crl_plane_bytes', 'crl_step_bytes
            'crl_encoder_workspace_bytes', 'crl_encoder_forward',
            'crl_encoder_precise_packed_bytes', 'crl_encoder_pack_precise', 'crl_zone_encode_precise',
            'crl_encoder_backward_workspace_bytes', 'crl_zone_encode_backward',
-           'crl_frame_capture', 'crl_zone_encode_frames', 'crl_zone_encode_backward_frames', 'crl_frames_zone_obs']
+           'crl_frame_capture', 'crl_zone_encode_frames', 'crl_zone_encode_backward_frames', 'crl_frames_zone_obs',
+           'crl_copy_envs']
 FRAME_NO_LAYOUT = 0xffffffff
 
 
@@ -125,6 +126,8 @@ def load():
     lib.crl_zone_encode_frames.argtypes = [P(CrlEncoderShape), P(CrlConfig), c_int32] + [c_void_p] * 8
     lib.crl_zone_encode_backward_frames.argtypes = [P(CrlEncoderShape), P(CrlConfig), c_int32] + [c_void_p] * 13
     lib.crl_frames_zone_obs.argtypes = [P(CrlConfig), c_int32] + [c_void_p] * 5
+    lib.crl_copy_envs.argtypes = [P(CrlConfig), P(CrlState), P(CrlOut), c_void_p, P(CrlConfig), P(CrlState), P(CrlOut),
+                                  c_void_p, c_int32, c_void_p, c_void_p]
     for name in SYMBOLS:
         getattr(lib, name)
     if lib.crl_abi_version() != ABI_VERSION:

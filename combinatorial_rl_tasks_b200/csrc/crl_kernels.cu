@@ -1651,6 +1651,119 @@ __global__ void __launch_bounds__(256) frame_capture_kernel(const CaptureParams 
   c.frames[e] = make_uint4((uint32_t)__float_as_int(c.aux[e].w), layout, cd.x, cd.y);
 }
 
+// Env copies (crl_copy_envs): pair i copies env src ids[i] onto env dst ids[i], plane by plane, bit for bit.  One side
+// of the copy: its planes (NULL = not copied; the host made both sides agree) and its ids.
+struct CopySide {
+  float4* pose;
+  float4* aux;
+  float2* zone_xy;
+  uint32_t* zone_tmax;
+  uint2* cooldown;
+  long long* seed;
+  uint32_t* episode;
+  float4* origin;
+  int32_t* goal;
+  float4* obs;
+  float* zone_obs;
+  unsigned long long* result;
+  float* shaped;
+  const int32_t* ids;   // NULL: pair i is env i
+  int B;
+};
+
+struct CopyParams {
+  CopySide dst, src;
+  uint32_t* next_ready;   // dst's, or NULL
+  uint32_t* rejected;     // pairs with an id out of range, or NULL
+  int n;
+};
+
+// One thread per pair moves the 16-byte vectors, the scalars and the plane-major zone centres: a warp of consecutive
+// dst ids writes whole 128-byte lines of every plane, and the gathered src reads of a branch (each src env read K times in
+// a row) come from L2.  A warp's 32 zone_obs rows (N Z floats each, 4-byte aligned only) are one span of 32 N Z floats
+// that lane j copies at j, j + 32, ...: consecutive dst rows are written at consecutive addresses.  Stores are streaming
+// (st.global.cs): the dst is not read again here, the src may be.
+template <int TASK, int N>
+__global__ void __launch_bounds__(256) copy_envs_kernel(const __grid_constant__ CopyParams c) {
+  constexpr int Z = ZoneDim<TASK>::Z, ROW = N * Z, NH = (N + 1) / 2;
+  const int i = blockIdx.x * blockDim.x + threadIdx.x, lane = threadIdx.x & 31;
+  int s = -1, d = -1;
+  bool bad = false;
+  if (i < c.n) {
+    s = c.src.ids ? c.src.ids[i] : i;
+    d = c.dst.ids ? c.dst.ids[i] : i;
+    if (s < 0 || s >= c.src.B || d < 0 || d >= c.dst.B) { bad = true; s = d = -1; }
+  }
+  if (c.rejected) {
+    const uint32_t b = __ballot_sync(kFull, bad);
+    if (b && lane == __ffs(b) - 1) atomicAdd(c.rejected, (uint32_t)__popc(b));
+  }
+  if (d >= 0) {
+    const size_t Bs = c.src.B, Bd = c.dst.B;
+    const float4 pose = c.src.pose[s], aux = c.src.aux[s], origin = c.src.origin[s];
+    const long long seed = c.src.seed[s];
+    const uint32_t episode = c.src.episode[s];
+    float2 xy[N];
+#pragma unroll
+    for (int z = 0; z < N; ++z) xy[z] = c.src.zone_xy[z * Bs + s];
+    uint32_t tmax[NH];
+    if constexpr (TASK == CRL_TASK_TTSP) {
+#pragma unroll
+      for (int j = 0; j < NH; ++j) tmax[j] = c.src.zone_tmax[j * Bs + s];
+    }
+    uint2 cd;
+    if constexpr (TASK == CRL_TASK_CM) cd = c.src.cooldown[s];
+    const int32_t goal = c.src.goal ? c.src.goal[s] : 0;
+    float4 o0, o1;
+    if (c.src.obs) { o0 = c.src.obs[2 * (size_t)s]; o1 = c.src.obs[2 * (size_t)s + 1]; }
+    const unsigned long long res = c.src.result ? c.src.result[s] : 0ull;
+    const float shaped = c.src.shaped ? c.src.shaped[s] : 0.f;
+
+    __stcs(c.dst.pose + d, pose);
+    __stcs(c.dst.aux + d, aux);
+    __stcs(c.dst.origin + d, origin);
+    __stcs(c.dst.seed + d, seed);
+    __stcs(c.dst.episode + d, episode);
+#pragma unroll
+    for (int z = 0; z < N; ++z) __stcs(c.dst.zone_xy + z * Bd + d, xy[z]);
+    if constexpr (TASK == CRL_TASK_TTSP) {
+#pragma unroll
+      for (int j = 0; j < NH; ++j) __stcs(c.dst.zone_tmax + j * Bd + d, tmax[j]);
+    }
+    if constexpr (TASK == CRL_TASK_CM) __stcs(c.dst.cooldown + d, cd);
+    if (c.dst.goal) __stcs(c.dst.goal + d, goal);
+    if (c.dst.obs) { __stcs(c.dst.obs + 2 * (size_t)d, o0); __stcs(c.dst.obs + 2 * (size_t)d + 1, o1); }
+    if (c.dst.result) __stcs(c.dst.result + d, res);
+    if (c.dst.shaped) __stcs(c.dst.shaped + d, shaped);
+    // the parked layouts were drawn for the old seed and episode: the next reset samples inline until a sampler round
+    // refills the slots
+    if (c.next_ready) { __stcs(c.next_ready + d, 0u); __stcs(c.next_ready + Bd + d, 0u); }
+  }
+  if (c.src.zone_obs) {
+    // loads of U floats in flight per lane before their stores; the guard `f0 + 32 u < 32 ROW` is warp-uniform
+    constexpr int U = 8;
+    for (int f0 = 0; f0 < 32 * ROW; f0 += 32 * U) {
+      float v[U];
+      long long at[U];
+#pragma unroll
+      for (int u = 0; u < U; ++u) {
+        at[u] = -1;
+        if (f0 + 32 * u < 32 * ROW) {
+          const int f = f0 + 32 * u + lane, pr = f / ROW, k = f - pr * ROW;
+          const int sp = __shfl_sync(kFull, s, pr), dp = __shfl_sync(kFull, d, pr);
+          if (dp >= 0) {
+            v[u] = c.src.zone_obs[(size_t)sp * ROW + k];
+            at[u] = (long long)dp * ROW + k;
+          }
+        }
+      }
+#pragma unroll
+      for (int u = 0; u < U; ++u)
+        if (at[u] >= 0) __stcs(c.dst.zone_obs + at[u], v[u]);
+    }
+  }
+}
+
 // ---- host side ---------------------------------------------------------------------
 static int zone_dim(int task) { return task == CRL_TASK_TSP ? 6 : 7; }
 
@@ -2170,6 +2283,72 @@ int crl_frame_capture(const CrlConfig* c, const CrlState* st, const CrlResult* r
   p.B = c->num_envs; p.N = c->num_zones; p.initial = initial != 0;
   frame_capture_kernel<<<(p.B + 255) / 256, 256, 0, static_cast<cudaStream_t>(stream)>>>(p);
   return launch_status();
+}
+
+// crl_copy_envs: the state planes of one side, checked as fill_params checks them (the counters are not copied and
+// not needed).
+static int copy_state_side(const CrlConfig* c, const CrlState* st, const int32_t* ids, CopySide& side) {
+  if (!st || !st->pose || !st->aux || !st->zone_xy || !st->seed || !st->episode || !st->origin) return CRL_ERR_NULL;
+  if (c->task == CRL_TASK_TTSP && !st->zone_tmax) return CRL_ERR_NULL;
+  if (c->task == CRL_TASK_CM && !st->cooldown) return CRL_ERR_NULL;
+  if (!aligned16(st->pose) || !aligned16(st->aux) || !aligned16(st->zone_xy) || !aligned16(st->origin) ||
+      (reinterpret_cast<uintptr_t>(st->seed) & 7u) || (reinterpret_cast<uintptr_t>(st->cooldown) & 7u))
+    return CRL_ERR_ALIGN;
+  side.pose = reinterpret_cast<float4*>(st->pose); side.aux = reinterpret_cast<float4*>(st->aux);
+  side.zone_xy = reinterpret_cast<float2*>(st->zone_xy);
+  side.zone_tmax = c->task == CRL_TASK_TTSP ? st->zone_tmax : nullptr;
+  side.cooldown = c->task == CRL_TASK_CM ? reinterpret_cast<uint2*>(st->cooldown) : nullptr;
+  side.seed = reinterpret_cast<long long*>(st->seed); side.episode = st->episode;
+  side.origin = reinterpret_cast<float4*>(st->origin);
+  side.ids = ids; side.B = c->num_envs;
+  return CRL_OK;
+}
+
+// the two configs describe the same task instance: every field but the batch's size, place and seed range
+static bool same_task_config(const CrlConfig* a, const CrlConfig* b) {
+  CrlConfig x = *a, y = *b;
+  for (CrlConfig* c : {&x, &y}) { c->num_envs = 0; c->env_offset = 0; c->seed_mode = 0; c->min_seed = 0; c->max_seed = 0; }
+  return memcmp(&x, &y, sizeof(CrlConfig)) == 0;
+}
+
+int crl_copy_envs(const CrlConfig* dst_cfg, const CrlState* dst, const CrlOut* dst_out, const int32_t* dst_ids,
+                  const CrlConfig* src_cfg, const CrlState* src, const CrlOut* src_out, const int32_t* src_ids,
+                  int32_t n, uint32_t* rejected, void* stream) {
+  int rc = check_config(dst_cfg);
+  if (rc) return rc;
+  if ((rc = check_config(src_cfg))) return rc;
+  if (!same_task_config(dst_cfg, src_cfg)) return CRL_ERR_CONFIG;
+  if (n < 0) return CRL_ERR_CONFIG;
+  CopyParams p;
+  memset(&p, 0, sizeof(p));
+  if ((rc = copy_state_side(dst_cfg, dst, dst_ids, p.dst))) return rc;
+  if ((rc = copy_state_side(src_cfg, src, src_ids, p.src))) return rc;
+  if (dst->goal && src->goal) { p.dst.goal = dst->goal; p.src.goal = src->goal; }
+  if (!dst_out != !src_out) return CRL_ERR_NULL;
+  if (dst_out) {
+    if (!dst_out->obs != !src_out->obs || !dst_out->zone_obs != !src_out->zone_obs ||
+        !dst_out->result != !src_out->result || !dst_out->shaped_reward != !src_out->shaped_reward)
+      return CRL_ERR_NULL;
+    if (!aligned16(dst_out->obs) || !aligned16(src_out->obs) || (reinterpret_cast<uintptr_t>(dst_out->result) & 7u) ||
+        (reinterpret_cast<uintptr_t>(src_out->result) & 7u) || (reinterpret_cast<uintptr_t>(dst_out->zone_obs) & 3u) ||
+        (reinterpret_cast<uintptr_t>(src_out->zone_obs) & 3u))
+      return CRL_ERR_ALIGN;
+    p.dst.obs = reinterpret_cast<float4*>(dst_out->obs); p.src.obs = reinterpret_cast<float4*>(src_out->obs);
+    p.dst.zone_obs = dst_out->zone_obs; p.src.zone_obs = src_out->zone_obs;
+    p.dst.result = reinterpret_cast<unsigned long long*>(dst_out->result);
+    p.src.result = reinterpret_cast<unsigned long long*>(src_out->result);
+    p.dst.shaped = dst_out->shaped_reward; p.src.shaped = src_out->shaped_reward;
+  }
+  if ((reinterpret_cast<uintptr_t>(rejected) & 3u) || (reinterpret_cast<uintptr_t>(dst_ids) & 3u) ||
+      (reinterpret_cast<uintptr_t>(src_ids) & 3u))
+    return CRL_ERR_ALIGN;
+  p.next_ready = dst->next_ready;
+  p.rejected = rejected;
+  p.n = n;
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+#define CRL_CALL_COPY(T, NN) { if (n > 0) copy_envs_kernel<T, NN><<<(n + 255) / 256, 256, 0, s>>>(p); }
+  CRL_DISPATCH(dst_cfg->task, dst_cfg->num_zones, CRL_CALL_COPY);
+  return n > 0 ? launch_status() : CRL_OK;
 }
 
 int crl_check_state(const CrlConfig* c, const CrlState* st, uint64_t* violations, void* stream) {

@@ -237,6 +237,7 @@ class Rollout:
         self._fill.zero_()                                    # the table restarts with every rollout
         with env._guard():
             self._capture(0, initial=True)
+        self._copies = env.copy_count
         self._started = True
         return self.obs_at(0)
 
@@ -252,6 +253,11 @@ class Rollout:
         self._bind(t + 1)
         env = self.env
         if self.store == 'frames':
+            if env.copy_count != self._copies:
+                # a copied env keeps the layout-table entry of its previous record: the rows built from its next
+                # records would be another episode's
+                raise RuntimeError("Rollout(store='frames'): envs were copied into the env (copy_envs_from) since the "
+                                   'last frame was captured; start a new rollout with begin()')
             if env._write_zone_obs:
                 env.write_zone_obs = False
             _, reward, done, info = env.step(a)

@@ -67,6 +67,62 @@ _raw_stream = getattr(torch._C, '_cuda_getCurrentRawStream', None) or \
     (lambda index: torch.cuda.current_stream(index).cuda_stream)
 
 
+# CrlConfig fields that may differ between the two sides of crl_copy_envs: the batch's size, place and seed range
+_COPY_FREE_FIELDS = ('num_envs', 'env_offset', 'seed_mode', 'min_seed', 'max_seed')
+
+
+def _task_config(cfg):
+    return tuple(getattr(cfg, f) for f, _ in cfg._fields_ if f not in _COPY_FREE_FIELDS)
+
+
+def _dev_index(device):
+    return device.index if device.index is not None else torch.cuda.current_device()
+
+
+def _copy_out(side, zone_obs):
+    """The CrlOut of one side of a copy; ``zone_obs=False``: the rows are not copied (absent on the other side)."""
+    return _lib.CrlOut(obs=side.obs.data_ptr(), zone_obs=side.zone_obs.data_ptr() if zone_obs else None,
+                       result=side.result.data_ptr(), shaped_reward=side.shaped_reward.data_ptr())
+
+
+class EnvSnapshot:
+    """The complete state of n envs of a ZoneVecEnv, gathered on the env's device by crl_copy_envs
+    (``ZoneVecEnv.snapshot``); ``ZoneVecEnv.copy_envs_from(snapshot, ...)`` restores it onto any envs of any
+    ZoneVecEnv with the same env id and config.  Holds the per-env state planes (sized by crl_plane_bytes for n envs,
+    no next-layout planes, no counters) and the output rows of the n envs -- the ZoneVecEnv attribute names, env i of
+    the snapshot being ``env_ids[i]`` of the source -- and no reference to the source env."""
+
+    _PLANES = (('pose', 0, torch.float32, (4,)), ('aux', 1, torch.float32, (4,)), ('zone_xy', 2, torch.float32, None),
+               ('zone_tmax', 3, torch.int32, None), ('cooldown', 4, torch.int32, (2,)), ('seeds', 5, torch.int64, ()),
+               ('episode', 6, torch.int32, ()), ('origin', 7, torch.float32, (4,)), ('obs', 14, torch.float32, (8,)),
+               ('zone_obs', 15, torch.float32, None), ('result', 16, torch.uint8, (8,)), ('goal', 20, torch.int32, ()),
+               ('shaped_reward', 21, torch.float32, ()))
+
+    def __init__(self, env, n):
+        self.env_id, self.spec, self.num_envs, self.device = env.env_id, env.spec, int(n), env.device
+        self.cfg = _lib.CrlConfig.from_buffer_copy(env.cfg)
+        self.cfg.num_envs = self.num_envs
+        self.zone_obs_ok = False                  # the zone_obs rows are those of the state (set by the gather)
+        sizes = (ctypes.c_int64 * _lib.NUM_PLANES)()
+        _lib.check(env.lib.crl_plane_bytes(self.cfg, sizes, _lib.NUM_PLANES))
+        N, Z = self.spec.num_zones, self.spec.zone_dim
+        shapes = {'zone_xy': (N, n, 2), 'zone_tmax': ((N + 1) // 2, n), 'zone_obs': (n, N, Z)}
+        for name, i, dtype, tail in self._PLANES:
+            t = None
+            if sizes[i]:
+                t = torch.zeros(sizes[i], dtype=torch.uint8, device=self.device).view(dtype)
+                t = t.view(shapes[name] if tail is None else (n,) + tail)
+            setattr(self, name, t)
+        ptr = lambda t: None if t is None else t.data_ptr()
+        self.state = _lib.CrlState(pose=ptr(self.pose), aux=ptr(self.aux), zone_xy=ptr(self.zone_xy),
+                                   zone_tmax=ptr(self.zone_tmax), cooldown=ptr(self.cooldown), seed=ptr(self.seeds),
+                                   episode=ptr(self.episode), origin=ptr(self.origin), goal=ptr(self.goal))
+
+    def nbytes(self):
+        """Device bytes the snapshot holds."""
+        return sum(t.numel() * t.element_size() for t in (getattr(self, k) for k, *_ in self._PLANES) if t is not None)
+
+
 class ZoneVecEnv:
     def __init__(self, env_id, num_envs, device='cuda:0', seed_mode='increment', min_seed=1, max_seed=100,
                  env_offset=0, auto_reset=True, prefetch_every=32, wait=False, prefetch_warps=0, layout_bank=None):
@@ -167,6 +223,10 @@ class ZoneVecEnv:
             self._install_layout_bank(layout_bank, seed_mode, min_seed, max_seed)
         self.bind_outputs(z(B, 8), z(B, N, Z), z(B, 8, dtype=torch.uint8), z(B))
         self._actions_dev = z(B, 2)
+        # copy_envs_from: pairs skipped on the device for an id out of range (device ids; cumulative), and the number of
+        # copies made INTO this env (Rollout(store='frames') refuses to go on across one)
+        self.copy_rejects = z(1, dtype=torch.int32)
+        self.copy_count = 0
         self._host = None
         self._host_calls = {}                     # (auto_reset, wait) -> CrlHostCall*, see step_host
         self._host_call_step = self.lib.crl_host_call_step
@@ -740,6 +800,120 @@ class ZoneVecEnv:
         self._zone_obs_ok = False
         if self.prefetch_every and self.state.bank_zone_xy is None:
             self.prefetch(torch.cuda.current_stream(self.device))
+
+    # -- env copies (crl_copy_envs) ----------------------------------------------------
+    def snapshot(self, env_ids=None):
+        """The state and output rows of envs ``env_ids`` (default: all), gathered into an ``EnvSnapshot`` on this env's
+        device.  ``env_ids``: a host sequence (checked here) or a CUDA int tensor (an id out of range is skipped on the
+        device and counted in ``copy_rejects``; its snapshot env stays zero).  Asynchronous on the current stream."""
+        n, sid, _ = self._copy_ids(self, env_ids, None, check_dst=False)
+        if not n:
+            raise ValueError('snapshot: no envs')
+        return self._snapshot(n, sid)
+
+    def _snapshot(self, n, sid, rejected=True):
+        snap = EnvSnapshot(self, n)
+        both = self.zone_obs is not None
+        with self._guard():
+            _lib.check(self.lib.crl_copy_envs(snap.cfg, snap.state, _copy_out(snap, both), None,
+                                              self.cfg, self.state, _copy_out(self, both),
+                                              None if sid is None else sid.data_ptr(), n,
+                                              self.copy_rejects.data_ptr() if rejected else None, self._stream()))
+        snap.zone_obs_ok = both and self._zone_obs_ok
+        self._chain_ok = False                    # the kernel before this env's next step is not a step
+        self.gpu_launches += 1
+        return snap
+
+    def copy_envs_from(self, src, src_ids=None, dst_ids=None):
+        """Make envs ``dst_ids`` of this env exact copies of envs ``src_ids`` of ``src``: state and output rows, bit
+        for bit (crl_copy_envs).  ``src`` is an ``EnvSnapshot`` (restore: ids index the snapshot) or a ``ZoneVecEnv``
+        (branching; ``src`` may be this env, any permutation of its envs is then copied correctly through a temporary
+        snapshot).  ``None`` ids stand for 0..n-1; ``n`` is the length of the ids given, else ``src.num_envs``.
+
+        Ids are host sequences, checked here (range, distinct dst ids, equal lengths: ``ValueError``), or CUDA int
+        tensors, passed on unsynchronised: a pair with an id out of range is skipped on the device and counted in
+        ``copy_rejects``.  ``src`` must have this env's id, device and config (``num_steps`` included) but may differ in
+        size, offset and seed range (``ValueError`` otherwise).  The copies then take the same actions to the same
+        outputs and states as their sources -- through auto-resets too with ``seed_mode='increment'`` or a layout bank;
+        with ``seed_mode='fixed_range'`` until the episode ends, since the next seed is drawn from the dst's global
+        index, as in-kernel random actions are.  Episode counters are not copied.  Asynchronous on the current stream."""
+        if not isinstance(src, (ZoneVecEnv, EnvSnapshot)):
+            raise TypeError(f'copy_envs_from: src must be a ZoneVecEnv or an EnvSnapshot, not {type(src).__name__}')
+        if src.env_id != self.env_id:
+            raise ValueError(f'copy_envs_from: src is {src.env_id}, this env is {self.env_id}')
+        if _dev_index(src.device) != self._dev_index:
+            raise ValueError(f'copy_envs_from: src lives on {src.device}, this env on {self.device}')
+        if _task_config(src.cfg) != _task_config(self.cfg):
+            raise ValueError('copy_envs_from: src has another config (num_steps, ...) than this env')
+        n, sid, did = self._copy_ids(src, src_ids, dst_ids)
+        if not n:
+            return
+        # a sampler round still running on the side stream writes slot flags the copy clears
+        if not torch.cuda.is_current_stream_capturing():
+            torch.cuda.current_stream(self.device).wait_stream(self._side)
+        if src is self:
+            # through a snapshot of the src envs: the id sets of one crl_copy_envs on one state must be disjoint
+            if sid is not None and did is not None:
+                # a src id rejected by the gather leaves a zero env in the snapshot: not to be copied on
+                did = torch.where((sid >= 0) & (sid < self.num_envs), did, torch.full_like(did, -1))
+            elif sid is not None:
+                ar = torch.arange(n, dtype=torch.int32, device=self.device)
+                did = torch.where((sid >= 0) & (sid < self.num_envs), ar, torch.full_like(ar, -1))
+            src, sid = self._snapshot(n, sid, rejected=False), None
+        both = src.zone_obs is not None and self.zone_obs is not None
+        src_zone_ok = src.zone_obs_ok if isinstance(src, EnvSnapshot) else src._zone_obs_ok
+        with self._guard():
+            _lib.check(self.lib.crl_copy_envs(self.cfg, self.state, _copy_out(self, both),
+                                              None if did is None else did.data_ptr(),
+                                              src.cfg, src.state, _copy_out(src, both),
+                                              None if sid is None else sid.data_ptr(), n,
+                                              self.copy_rejects.data_ptr(), self._stream()))
+        self.gpu_launches += 1
+        self.copy_count += 1
+        self._mirror_ok = False
+        self._chain_ok = False
+        # the untouched rows keep what they held; the copied ones are current only if the source's were
+        self._zone_obs_ok = self._zone_obs_ok and both and src_zone_ok
+        if isinstance(src, ZoneVecEnv):
+            src._chain_ok = False
+
+    def _copy_ids(self, src, src_ids, dst_ids, check_dst=True):
+        """(n, src ids, dst ids) of a copy from ``src`` into this env: each id list None (= 0..n-1) or a device int32
+        tensor.  Host ids are checked here; device ids only for their device and length."""
+        def prep(ids, bound, what, distinct):
+            if ids is None:
+                return None, None
+            if isinstance(ids, torch.Tensor) and ids.is_cuda:
+                if ids.is_floating_point() or ids.is_complex() or ids.dtype == torch.bool:
+                    raise ValueError(f'{what} ids must be integers, not {ids.dtype}')
+                if _dev_index(ids.device) != self._dev_index:
+                    raise ValueError(f'{what} ids live on {ids.device}, the envs on {self.device}')
+                ids = ids.reshape(-1)
+                if ids.dtype != torch.int32:     # an id beyond int32 stays out of range instead of wrapping into it
+                    ids = ids.clamp(-1, 2 ** 31 - 1).to(torch.int32)
+                return ids.numel(), ids.contiguous()
+            a = np.asarray(ids.cpu() if isinstance(ids, torch.Tensor) else ids)
+            if a.dtype.kind not in 'iu' and a.size:
+                raise ValueError(f'{what} ids must be integers, not {a.dtype}')
+            a = a.astype(np.int64).reshape(-1)
+            if a.size and (a.min() < 0 or a.max() >= bound):
+                raise ValueError(f'{what} ids must lie in [0, {bound})')
+            if distinct and np.unique(a).size != a.size:
+                raise ValueError(f'{what} ids must be distinct')
+            return a.size, a.astype(np.int32)
+        ns, sid = prep(src_ids, src.num_envs, 'src', False)
+        nd, did = prep(dst_ids, self.num_envs, 'dst', check_dst)
+        if ns is not None and nd is not None and ns != nd:
+            raise ValueError(f'copy_envs_from: {ns} src ids but {nd} dst ids')
+        n = ns if ns is not None else nd if nd is not None else src.num_envs
+        if sid is None and n > src.num_envs:
+            raise ValueError(f'copy_envs_from: {n} envs from a src of {src.num_envs}')
+        if check_dst and did is None and n > self.num_envs:
+            raise ValueError(f'copy_envs_from: {n} envs into an env of {self.num_envs}')
+        if not n:
+            return 0, None, None
+        up = lambda a: torch.from_numpy(a).to(self.device) if isinstance(a, np.ndarray) else a   # checked host ids
+        return n, up(sid), up(did)
 
     def set_qpos_qvel(self, qpos, qvel, env_ids=None):
         """Overwrite sim.data.qpos / qvel (fp64, reference coordinates) of some envs."""

@@ -532,6 +532,32 @@ int crl_zone_encode_backward_frames(const CrlEncoderShape* shape, const CrlConfi
 int crl_frames_zone_obs(const CrlConfig* cfg, int32_t num_rows, const CrlFrame* frames, const float* layout_xy,
                         const uint32_t* layout_tmax, float* zone_obs, void* stream);
 
+/* ---- env copies: snapshot, restore and branch individual envs ----
+ * Copy env src_ids[i] of (src_cfg, src, src_out) onto env dst_ids[i] of (dst_cfg, dst, dst_out), i < n.  NULL ids: 0..n-1.
+ * Copied bit for bit, per env: pose, aux (steps, visited mask / colour codes, return, episode parity), every zone row of
+ * zone_xy (plane-major on both sides, each with its own B), seed, episode, origin, zone_tmax (TimedTSP), cooldown
+ * (ColourMatch), goal when both states have that plane; and, when src_out and dst_out are both given, the obs row, the
+ * zone_obs row, the result record and shaped_reward -- each output field that is non-NULL on both sides (a field, or an
+ * out struct, given on one side only is CRL_ERR_NULL).  Not copied: counters (a copy is not an episode), stamp, row_list,
+ * prefetch_* and next_*.  Both next_ready slots of every dst env written are cleared (when dst->next_ready is set): their
+ * layouts were drawn for the old seed and episode, and the step samples inline, with the identical result, until a
+ * sampler round refills them.
+ * Host checks, before any launch: the configs must agree in every field but num_envs, env_offset, seed_mode, min_seed and
+ * max_seed (CRL_ERR_CONFIG); NULL and alignment of the planes the task needs; n < 0 is CRL_ERR_CONFIG, n == 0 launches
+ * nothing.  On the device, a pair whose src or dst id is out of range is skipped and counted in *rejected (optional,
+ * device uint32, cumulative).  No host synchronisation: the call can be captured in a CUDA graph.
+ * PRECONDITIONS (not checked): the dst ids are distinct; when src and dst are the same state, the src and dst id sets
+ * are disjoint (copy through a second state to permute envs in place).
+ * WHAT A COPY GUARANTEES: the step is a pure function of the state and the action, so a dst env that then takes the same
+ * actions as its src produces the same outputs and state, bit for bit -- through auto-resets too under
+ * CRL_SEED_INCREMENT and with a layout bank, since the next seed is the copied one and the timeouts, colours and layout are
+ * functions of it.  Under CRL_SEED_FIXED_RANGE the next seed is drawn from the dst's global env index, and in-kernel
+ * actions (actions == NULL) are keyed by it as well: a copy then matches its src until its episode ends, and branches
+ * stepped with in-kernel actions diverge by construction. */
+int crl_copy_envs(const CrlConfig* dst_cfg, const CrlState* dst, const CrlOut* dst_out, const int32_t* dst_ids,
+                  const CrlConfig* src_cfg, const CrlState* src, const CrlOut* src_out, const int32_t* src_ids,
+                  int32_t n, uint32_t* rejected, void* stream);
+
 /* Copies the eight counters to the host (synchronises `stream`).  The first four (sum of
  * returns, episodes, successes, sum of lengths) are what ranks all-reduce. */
 int crl_counters_read(const CrlState* st, double out[8], void* stream);
